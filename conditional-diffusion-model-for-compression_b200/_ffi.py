@@ -19,15 +19,31 @@ SYMBOLS = [
 # ... and include/cdc_b200_tools.h (tests / profiling / A-B; same library)
 TOOLS_SYMBOLS = [
     "cdc_set_plan_option", "cdc_num_step_ops", "cdc_step_op_name", "cdc_step_op_flops", "cdc_step_op_bytes", "cdc_run_step_op",
-    "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn",
+    "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn", "cdc_step_op_describe",
 ]
 OPT_FUSE_APPLY, OPT_KF, OPT_KF_S2, OPT_KF_MIN_PIXELS, OPT_KF_RING = range(5)
+OPK_MEMSET, OPK_CONV, OPK_GN_STATS, OPK_GN_APPLY, OPK_ATTENTION = range(5)  # cdc_op_kind
 
 
 class CdcConfig(C.Structure):
     _fields_ = [("base", C.c_int32), ("mults", C.c_int32 * 4), ("groups", C.c_int32), ("heads", C.c_int32),
                 ("head_dim", C.c_int32), ("temb", C.c_int32), ("T", C.c_int32), ("latent_ch", C.c_int32),
                 ("gn_eps", C.c_float)]
+
+
+class TensorDesc(C.Structure):
+    _fields_ = [("p", C.c_void_p), ("C", C.c_int32), ("Cphys", C.c_int32), ("H", C.c_int32), ("W", C.c_int32)]
+
+
+class StepOpDesc(C.Structure):
+    """include/cdc_b200_tools.h cdc_step_op_desc"""
+    _fields_ = [("kind", C.c_int32), ("weight", C.c_char * 64), ("res_weight", C.c_char * 64), ("in_gn", C.c_char * 64),
+                ("film_off", C.c_int32), ("mode", C.c_int32), ("ksize", C.c_int32), ("epi", C.c_int32), ("silu", C.c_int32),
+                ("kernel", C.c_int32), ("bn", C.c_int32), ("cpg", C.c_int32), ("ch", C.c_int32), ("staged", C.c_int32),
+                ("xk16", C.c_int32), ("tr", C.c_int32), ("res1", C.c_int32), ("apply", C.c_int32),
+                ("src", TensorDesc * 2), ("residual", TensorDesc), ("out", TensorDesc), ("res_out", TensorDesc),
+                ("gn_in_acc", C.c_void_p), ("gn_out_acc", C.c_void_p), ("gn_slots", C.c_int32),
+                ("x", C.c_void_p), ("x0_out", C.c_void_p), ("xpad", C.c_void_p)]
 
 
 _libs = {}
@@ -104,6 +120,7 @@ def _bind(L):
     L.cdc_step_op_bytes.argtypes = [p, i32]
     L.cdc_step_op_bytes.restype = C.c_double
     L.cdc_run_step_op.argtypes = [p, i32, i32, p]
+    L.cdc_step_op_describe.argtypes = [p, i32, C.POINTER(StepOpDesc)]
     L.cdc_profile_step.argtypes = [p, i32, i32, fp, p]
     L.cdc_profile_graph.argtypes = [p, i32, fp, fp, p]
     L.cdc_test_conv.argtypes = [i32, p, i32, p, i32, i32, i32, i32, f32p, f32p, i32, i32, i32, i32, p, p, p, p]

@@ -99,7 +99,19 @@ struct Op {
     double flops = 0, bytes = 0;
     // (stream, sampler step k, timing slot or null): see ptx.cuh stamp_begin / stamp_end
     std::function<cudaError_t(cudaStream_t, int, long long*)> run;
+    cdc_step_op_desc desc{};  // what the op computes and with which kernel (cdc_step_op_describe); never read by run
 };
+
+static cdc_tensor_desc tensor_desc(const Act& a) {
+    cdc_tensor_desc d;
+    d.p = a.p;
+    d.C = a.C;
+    d.Cphys = a.cs();
+    d.H = a.H;
+    d.W = a.W;
+    return d;
+}
+static void set_desc_name(char (&dst)[64], const std::string& s) { snprintf(dst, sizeof dst, "%s", s.c_str()); }
 
 // per-step sampler coefficients (host copies; oracle/sampler.py make_schedule)
 struct SamplerTab {
@@ -163,6 +175,7 @@ struct ConvBuild {
     const float* in_gamma = nullptr;
     const float* in_beta = nullptr;
     int in_film_off = -1;      // offset into the step's FiLM vector, or -1
+    std::string in_gn;         // parameter prefix of that GroupNorm (op description only)
     float in_eps = 1e-5f;
     float* const* film_base = nullptr;  // -> ctx->film: [steps][*film_total] FiLM vectors of the schedule (set later)
     const int* film_total = nullptr;
@@ -360,7 +373,25 @@ static int build_conv(const ConvBuild& cb, int B, int num_sms, const PlanOpts& p
     const int OH = x2 ? 2 * gh : gh, OW = x2 ? 2 * gw : gw;
     if (cb.epi != EPI_DDIM && (cb.out.H != OH || cb.out.W != OW || cb.out.C != w.n_pad))
         return fail("output tensor shape mismatch");
-
+    cdc_step_op_desc& d = op->desc;
+    d = cdc_step_op_desc{};
+    d.kind = CDC_OPK_CONV;
+    d.film_off = -1;
+    d.mode = cb.mode;
+    d.ksize = cb.ksize;
+    d.epi = cb.epi;
+    d.cpg = cb.cpg;
+    d.ch = ctot / 64;
+    for (size_t s = 0; s < cb.srcs.size(); ++s) d.src[s] = tensor_desc(cb.srcs[s]);
+    d.out = tensor_desc(cb.out);
+    if (cb.residual) {
+        d.residual = d.out;
+        d.residual.p = const_cast<act_t*>(cb.residual);
+    }
+    d.gn_out_acc = cb.gn_acc;
+    d.x = cb.x;
+    d.x0_out = cb.x0_out;
+    d.xpad = cb.xpad;
 
     // ---- kh-fused strip variant (conv_kf.cu) ----
     {
@@ -444,6 +475,20 @@ static int build_conv(const ConvBuild& cb, int B, int num_sms, const PlanOpts& p
             float* const* film_base = cb.film_base;
             const int* film_total = cb.film_total;
             const int film_off = cb.in_film_off;
+            d.kernel = 2;
+            d.bn = bn_k;
+            d.ch = CHk;
+            d.staged = kstaged;
+            d.xk16 = xk;
+            d.tr = kg.tr;
+            d.res1 = kres;
+            d.apply = kapply;
+            if (kres) d.res_out = tensor_desc(cb.res_out);
+            if (kapply) {
+                d.gn_in_acc = const_cast<gn_sum_t*>(cb.in_acc);
+                d.film_off = film_off;
+                set_desc_name(d.in_gn, cb.in_gn);
+            }
             op->run = [kp, bn_k, cpg, epi, CHk, xk, kmode, kres, kapply, kstaged, samp, film_base, film_total, film_off](
                           cudaStream_t s, int k, long long* stamp) -> cudaError_t {
                 KfParams q = *kp;
@@ -621,6 +666,8 @@ static int build_conv(const ConvBuild& cb, int B, int num_sms, const PlanOpts& p
     op->bytes = 2.0 * (m_in * w.c_true + M * w.n_true + static_cast<double>(taps) * w.c_true * w.n_true);
     const int epi = cb.epi, cpg = cb.cpg;
     const SamplerTab* samp = cb.samp;
+    d.kernel = 1;
+    d.bn = bn;
     op->run = [cp, bn, cpg, epi, num_sms, samp](cudaStream_t s, int k, long long* stamp) -> cudaError_t {
         if (epi == EPI_DDIM) {
             if (!samp || k < 0 || k >= static_cast<int>(samp->c0.size())) return cudaErrorInvalidValue;
@@ -858,6 +905,10 @@ struct PlanB {
             rc = ctx->fail(r, "%s", e.c_str());
             return;
         }
+        for (const auto& kv : ctx->convs) {  // parameter prefixes, for the op description
+            if (&kv.second == cb.w) set_desc_name(op.desc.weight, kv.first);
+            if (op.desc.res1 && &kv.second == cb.res_w) set_desc_name(op.desc.res_weight, kv.first);
+        }
         ops->push_back(op);
     }
     // Every GroupNorm of the sequence gets its own accumulator slot; one memset (first op of the sequence) clears them.
@@ -879,6 +930,9 @@ struct PlanB {
         z.run = [c, base, used](cudaStream_t s, int, long long*) {
             return cudaMemsetAsync(base, 0, static_cast<size_t>(*used) * c->B * kGnImgStride * sizeof(gn_sum_t), s);
         };
+        z.desc.kind = CDC_OPK_MEMSET;
+        z.desc.film_off = -1;
+        z.desc.gn_out_acc = base;  // (gn_slots: filled in when described, the sequence is complete by then)
         ops->push_back(z);
     }
     // GroupNorm (+FiLM of step k) apply: coefficients come from the accumulator slot inside the kernel
@@ -900,6 +954,18 @@ struct PlanB {
             const float* film = foff >= 0 ? c->film + static_cast<size_t>(k) * c->film_total + foff : nullptr;
             return launch_gn_apply(xp, acc, gamma, beta, film, c->cfg.gn_eps, rp, yp, B, HW, Cc, si, c->num_sms, s, stamp, c->sat_dev);
         };
+        cdc_step_op_desc& d = a.desc;
+        d.kind = CDC_OPK_GN_APPLY;
+        set_desc_name(d.weight, gnp);
+        d.film_off = foff;
+        d.silu = si;
+        d.src[0] = tensor_desc(x);
+        d.out = tensor_desc(y);
+        if (res) {
+            d.residual = d.out;
+            d.residual.p = const_cast<act_t*>(res);
+        }
+        d.gn_in_acc = const_cast<gn_sum_t*>(acc);
         ops->push_back(a);
     }
     // Time-conditioned ResBlock (oracle/unet.py RB).  film_idx < 0: RBn (context net).
@@ -943,6 +1009,7 @@ struct PlanB {
         c2.in_gamma = find_w(ctx, wp + ".gn1.weight")->p;
         c2.in_beta = find_w(ctx, wp + ".gn1.bias")->p;
         c2.in_eps = ctx->cfg.gn_eps;
+        c2.in_gn = wp + ".gn1";
         if (film_idx >= 0) {
             c2.in_film_off = ctx->film_off[film_idx];
             c2.film_base = &ctx->film;
@@ -1043,6 +1110,11 @@ static int build_plans(cdc_ctx* ctx) {
         const act_t* m1p = m1.p;
         gn_sum_t* aslot = pb.new_gn_slot();
         st.run = [aslot, m1p, B, HW, Cm](cudaStream_t s, int, long long* stamp) { return launch_gn_stats(m1p, aslot, B, HW, Cm, s, stamp); };
+        st.desc.kind = CDC_OPK_GN_STATS;
+        set_desc_name(st.desc.weight, "mid.attn.gn");
+        st.desc.film_off = -1;
+        st.desc.src[0] = tensor_desc(m1);
+        st.desc.gn_out_acc = aslot;
         ctx->step_ops.push_back(st);
         pb.gn("mid.attn.gn", "mid.attn.gn", -1, aslot, m1, nullptr, n, false);
         ConvBuild cq;
@@ -1077,6 +1149,10 @@ static int build_plans(cdc_ctx* ctx) {
             q.stamp = stamp;
             return launch_attention_tc(q, B, s);
         };
+        at.desc.kind = CDC_OPK_ATTENTION;
+        at.desc.film_off = -1;
+        at.desc.src[0] = tensor_desc(qkv);
+        at.desc.out = tensor_desc(o);
         ctx->step_ops.push_back(at);
         ConvBuild cpj;
         cpj.name = "mid.attn.proj";
@@ -1882,6 +1958,13 @@ double cdc_step_op_flops(cdc_ctx* ctx, int i) {
 }
 double cdc_step_op_bytes(cdc_ctx* ctx, int i) {
     return (ctx && i >= 0 && i < static_cast<int>(ctx->step_ops.size())) ? ctx->step_ops[i].bytes : 0;
+}
+int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out) {
+    if (!ctx) return CDC_ERR_STATE;
+    if (!out || i < 0 || i >= static_cast<int>(ctx->step_ops.size())) return ctx->fail(CDC_ERR_SHAPE, "bad op index / null output");
+    *out = ctx->step_ops[i].desc;
+    if (out->kind == CDC_OPK_MEMSET) out->gn_slots = ctx->gn_used_step;
+    return CDC_OK;
 }
 int cdc_run_step_op(cdc_ctx* ctx, int i, int k, cdc_stream s) {
     NEED_PLAN();

@@ -260,6 +260,12 @@ class Decoder:
         return [(self.L.cdc_step_op_name(self.ctx, i).decode(), self.L.cdc_step_op_flops(self.ctx, i),
                  self.L.cdc_step_op_bytes(self.ctx, i)) for i in range(n)]
 
+    def step_op_desc(self, i):
+        """_ffi.StepOpDesc of step op i of the bound plan (include/cdc_b200_tools.h cdc_step_op_describe)."""
+        d = _ffi.StepOpDesc()
+        self._ck(self.L.cdc_step_op_describe(self.ctx, i, C.byref(d)), "cdc_step_op_describe")
+        return d
+
     def run_step_op(self, i, k=0):
         with torch.cuda.device(self.device):
             self._ck(self.L.cdc_run_step_op(self.ctx, i, k, _stream_ptr()), "cdc_run_step_op")

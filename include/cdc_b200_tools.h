@@ -32,6 +32,39 @@ const char* cdc_step_op_name(cdc_ctx* ctx, int i);
 double cdc_step_op_flops(cdc_ctx* ctx, int i);
 double cdc_step_op_bytes(cdc_ctx* ctx, int i);
 int cdc_run_step_op(cdc_ctx* ctx, int i, int k, cdc_stream s);
+
+/* Read-only description of step op i of the bound plan: what it computes, from which tensors into which, and which
+ * kernel instantiation runs it.  Metadata recorded when the plan was built; reading it changes nothing. */
+typedef enum {
+    CDC_OPK_MEMSET = 0,     /* clears the step's GroupNorm accumulator slots (gn_out_acc, gn_slots of them) */
+    CDC_OPK_CONV = 1,
+    CDC_OPK_GN_STATS = 2,   /* GroupNorm statistics of src[0] into gn_out_acc */
+    CDC_OPK_GN_APPLY = 3,   /* out = act(GroupNorm(src[0]; gn_in_acc) [* (1 + s) + sh]) [+ residual] */
+    CDC_OPK_ATTENTION = 4   /* out = softmax(q k^T / 8) v per head, src[0] = qkv [B][HW][3C] */
+} cdc_op_kind;
+typedef struct {
+    void* p;  /* NHWC 16-bit activation; NULL: not used */
+    int C, Cphys, H, W;  /* Cphys: channels stored per pixel (the stem's x_t copy stores fewer than its C) */
+} cdc_tensor_desc;
+typedef struct {
+    int kind;            /* cdc_op_kind */
+    char weight[64];     /* parameter prefix of the conv / GroupNorm ("down.0.rb1.conv2", "mid.attn.gn", "final") or "" */
+    char res_weight[64]; /* 1x1 residual conv computed in the same launch ("down.1.rb1.res") or "" */
+    char in_gn[64];      /* GroupNorm + SiLU applied to the conv's input rows ("down.0.rb1.gn1") or "" */
+    int film_off;        /* offset of the (scale | shift) FiLM pair in a step's FiLM vector (cdc_get_film), -1: none */
+    int mode, ksize, epi, silu;  /* conv: mode 0 stride 1, 1 stride 2, 2 nearest-x2 input; epi 0 store, 1 GroupNorm
+                                    statistics, 2 sampler update (final conv); gn_apply: silu */
+    int kernel;          /* conv: 1 = conv_tc.cu (general), 2 = conv_kf.cu (strip); 0 otherwise */
+    int bn, cpg, ch, staged, xk16, tr, res1, apply;  /* the instantiation / walk that runs (ch: 64-channel input chunks) */
+    cdc_tensor_desc src[2], residual, out, res_out;
+    void* gn_in_acc;     /* GroupNorm accumulator slot read ([B][32][4] int64, csrc/gn_sums.cuh) or NULL */
+    void* gn_out_acc;    /* slot accumulated into (memset: first slot cleared) or NULL */
+    int gn_slots;        /* memset: slots cleared */
+    float* x;            /* final conv: sampler state, NHWC fp32 [B][H][W][3], read as x_t and overwritten with x_prev */
+    float* x0_out;       /* final conv: x0 estimate, NHWC fp32 */
+    void* xpad;          /* final conv: the stem's 16-bit x_t copy, rewritten with x_prev */
+} cdc_step_op_desc;
+int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out);
 /* in-stream device time (microseconds) of every op of step k, after `warm` untimed steps; us_out[cdc_num_step_ops] */
 int cdc_profile_step(cdc_ctx* ctx, int k, int warm, float* us_out, cdc_stream s);
 /* In-graph timing: captures the same K-step graph with every kernel writing (earliest CTA start, latest CTA end) in
