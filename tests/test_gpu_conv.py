@@ -146,6 +146,21 @@ def test_conv_matches_torch(case):
     _check(o, _ref_conv(srcs, w, b, ks, mode), name)
 
 
+def test_conv_up2_refuses_non_3x3():
+    """Nearest-x2 convs run on parity weights pre-summed from 3x3 weights: any other kernel size is refused
+    (CDC_ERR_SHAPE) before anything launches."""
+    L = _lib()
+    B, H, W, cin, cout = 1, 16, 16, 64, 64
+    src = _nhwc_act(_mk((B, cin, H, W), 1))
+    w, b = _mk((cout, cin, 1, 1), 2), _mk((cout,), 3)
+    out = torch.zeros(B, 2 * H, 2 * W, cout, device=DEV, dtype=_act_dtype())
+    rc = L.cdc_test_conv(0, _ptr(src), cin, C.c_void_p(0), 0, B, H, W, _ptr(w), _ptr(b), cout, 1, 2, 0, C.c_void_p(0),
+                         _ptr(out), C.c_void_p(0), C.c_void_p(0))
+    assert rc == -1, rc  # CDC_ERR_SHAPE
+    assert "weight layout does not match the sources" in L.cdc_last_error(None).decode()
+    assert not out.any()
+
+
 def test_conv_residual_epilogue():
     srcs = [_mk((1, 256, 16, 16), 1)]
     w = _mk((256, 256, 1, 1), 2, scale=1 / 16.0)
