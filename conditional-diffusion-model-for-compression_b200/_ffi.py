@@ -21,7 +21,7 @@ TOOLS_SYMBOLS = [
     "cdc_set_plan_option", "cdc_num_step_ops", "cdc_step_op_name", "cdc_step_op_flops", "cdc_step_op_bytes", "cdc_run_step_op",
     "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn", "cdc_step_op_describe",
 ]
-OPT_FUSE_APPLY, OPT_KF, OPT_KF_S2, OPT_KF_MIN_PIXELS, OPT_KF_RING = range(5)
+OPT_FUSE_APPLY, OPT_KF = range(2)
 OPK_MEMSET, OPK_CONV, OPK_GN_STATS, OPK_GN_APPLY, OPK_ATTENTION = range(5)  # cdc_op_kind
 
 

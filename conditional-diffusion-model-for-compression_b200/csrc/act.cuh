@@ -21,7 +21,6 @@ namespace cdc {
 typedef __half act_t;
 constexpr uint32_t kUmmaFormat = 0;  // tcgen05 kind::f16 a_format / b_format: 0 = F16
 #define CDC_TMA_DTYPE CU_TENSOR_MAP_DATA_TYPE_FLOAT16
-#define CDC_MMA_SYNC_T "f16"
 constexpr float kActMax = 65504.0f;  // values beyond it are stored saturated (and counted: ConvParams::sat)
 __host__ __device__ __forceinline__ float sat_act(float v) { return fminf(fmaxf(v, -65504.0f), 65504.0f); }
 __device__ __forceinline__ uint32_t pack_act2(float lo, float hi) {  // saturating: never stores inf
@@ -52,7 +51,6 @@ typedef __nv_bfloat16 act_t;
 constexpr uint32_t kUmmaFormat = 1;  // 1 = BF16
 constexpr float kActMax = 3.3895313892515355e38f;  // bf16 maximum
 #define CDC_TMA_DTYPE CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
-#define CDC_MMA_SYNC_T "bf16"
 __device__ __forceinline__ uint32_t pack_act2(float lo, float hi) {
     __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&h);

@@ -1,231 +1,14 @@
 // K-attn: fused flash-style softmax(Q K^T / 8) V for the 1/16-resolution mid block
-// (4 heads x d = 64, N = HW/256 tokens).  Scores never touch HBM.  The product path is the tcgen05 kernel at the end
-// of this file; the mma.sync kernel below is compiled only into the tools build (-DCDC_TOOLS) as its A/B reference.
-// Oracle counterpart: oracle/unet.py Attn.forward.
+// (4 heads x d = 64, N = HW/256 tokens).  Scores never touch HBM.
 #include "kernels.cuh"
-#include "launch.cuh"
 #include "ptx.cuh"
 
 namespace cdc {
 
 constexpr int kAttD = 64;
 
-#ifdef CDC_TOOLS  // the mma.sync kernel is the A/B reference of tools/ builds only (libcdc_b200_tools.so)
-constexpr int kAttBQ = 64, kAttBK = 64, kAttPitch = 72;  // 16-bit elements per smem row
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, bool pred) {
-    const int sz = pred ? 16 : 0;  // src-size 0 => zero fill
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(sz) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-    asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void mma_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k16.row.col.f32." CDC_MMA_SYNC_T "." CDC_MMA_SYNC_T ".f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ void ldmatrix_x2_trans(uint32_t& r0, uint32_t& r1, uint32_t addr) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x2.trans.shared.b16 {%0,%1}, [%2];" : "=r"(r0), "=r"(r1) : "r"(addr));
-}
-
-// 8 warps: two groups of 4.  Group g takes the K/V tiles j = g, g+2, ... (its own double buffers and named barrier),
-// so the serial chain of tiles is half as long (a 64-query CTA at N = 1536 walks 12 tiles instead of 24 -- the kernel
-// is latency-bound at this size); the two partial (O, m, l) states are merged through shared memory at the end.
-constexpr int kAttThreads = 256;
-constexpr int kAttTile = kAttBK * kAttPitch;                                           // elements of one K or V tile
-constexpr int kAttSmemBytes = (kAttBQ * kAttPitch + 2 * 2 * 2 * kAttTile) * 2;         // Q + [group][K|V][buffer]
-
-__global__ void __launch_bounds__(kAttThreads) attention_kernel(const act_t* qkv, act_t* out, int N, int heads) {
-    extern __shared__ __align__(16) uint8_t att_smem[];
-    act_t(*Qs)[kAttPitch] = reinterpret_cast<act_t(*)[kAttPitch]>(att_smem);
-    act_t* kv0 = reinterpret_cast<act_t*>(att_smem) + kAttBQ * kAttPitch;
-    const int C = heads * kAttD, ld = 3 * C;
-    const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kAttBQ;
-    const int tid = threadIdx.x, grp = tid >> 7, gtid = tid & 127, warp = (tid >> 5) & 3, lane = tid & 31, g = lane >> 2, t = lane & 3;
-    act_t(*Ks)[kAttBK][kAttPitch] = reinterpret_cast<act_t(*)[kAttBK][kAttPitch]>(kv0 + (grp * 4 + 0) * kAttTile);  // [buffer]
-    act_t(*Vs)[kAttBK][kAttPitch] = reinterpret_cast<act_t(*)[kAttBK][kAttPitch]>(kv0 + (grp * 4 + 2) * kAttTile);
-    const act_t* base = qkv + static_cast<size_t>(b) * N * ld + h * kAttD;
-    pdl_wait();  // qkv is written by the preceding conv (it is only read through cp.async below)
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
-
-    auto load_tile = [&](act_t (*dst)[kAttPitch], const act_t* src, int row0, int first, int nthr) {
-        for (int i = first; i < 64 * 8; i += nthr) {
-            const int r = i >> 3, c = i & 7;
-            const bool ok = row0 + r < N;
-            const act_t* sp = src + static_cast<size_t>(ok ? row0 + r : 0) * ld + c * 8;
-            cp_async16(smem_u32(&dst[r][c * 8]), sp, ok);
-        }
-    };
-    const int ntiles = (N + kAttBK - 1) / kAttBK;
-    load_tile(Qs, base, q0, tid, kAttThreads);
-    if (grp < ntiles) {
-        load_tile(Ks[0], base + C, grp * kAttBK, gtid, 128);
-        load_tile(Vs[0], base + 2 * C, grp * kAttBK, gtid, 128);
-    }
-    cp_async_commit();
-    cp_async_wait<0>();
-    __syncthreads();  // Q (loaded by both groups) and every group's first tile
-
-    const float sl2 = 0.125f * 1.4426950408889634f;  // 1/sqrt(64) * log2(e)
-    float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-    float o[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
-    uint32_t qf[4][4];
-#pragma unroll
-    for (int kk = 0; kk < 4; ++kk) {
-        const int r = warp * 16 + g, c = kk * 16 + 2 * t;
-        qf[kk][0] = *reinterpret_cast<const uint32_t*>(&Qs[r][c]);
-        qf[kk][1] = *reinterpret_cast<const uint32_t*>(&Qs[r + 8][c]);
-        qf[kk][2] = *reinterpret_cast<const uint32_t*>(&Qs[r][c + 8]);
-        qf[kk][3] = *reinterpret_cast<const uint32_t*>(&Qs[r + 8][c + 8]);
-    }
-
-    int buf = 0;
-    for (int j = grp; j < ntiles; j += 2, buf ^= 1) {
-        if (j + 2 < ntiles) {
-            load_tile(Ks[buf ^ 1], base + C, (j + 2) * kAttBK, gtid, 128);
-            load_tile(Vs[buf ^ 1], base + 2 * C, (j + 2) * kAttBK, gtid, 128);
-            cp_async_commit();
-            cp_async_wait<1>();
-        } else {
-            cp_async_wait<0>();
-        }
-        named_bar_sync(1 + grp, 128);
-        // S = Q K^T  (16 x 64 per warp)
-        float s[8][4];
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-            s[n][0] = s[n][1] = s[n][2] = s[n][3] = 0.f;
-#pragma unroll
-            for (int kk = 0; kk < 4; ++kk) {
-                const uint32_t b0 = *reinterpret_cast<const uint32_t*>(&Ks[buf][n * 8 + g][kk * 16 + 2 * t]);
-                const uint32_t b1 = *reinterpret_cast<const uint32_t*>(&Ks[buf][n * 8 + g][kk * 16 + 8 + 2 * t]);
-                mma_16816(s[n], qf[kk], b0, b1);
-            }
-        }
-        // scale to log2 domain, mask the key tail
-        const int key0 = j * kAttBK;
-        float mx0 = -INFINITY, mx1 = -INFINITY;
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const int key = key0 + n * 8 + 2 * t + (e & 1);
-                s[n][e] = key < N ? s[n][e] * sl2 : -INFINITY;
-            }
-            mx0 = fmaxf(mx0, fmaxf(s[n][0], s[n][1]));
-            mx1 = fmaxf(mx1, fmaxf(s[n][2], s[n][3]));
-        }
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-        const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);
-        const float sc0 = exp2f(m0 - mn0), sc1 = exp2f(m1 - mn1);
-        m0 = mn0;
-        m1 = mn1;
-        float rs0 = 0.f, rs1 = 0.f;
-        uint32_t pf[4][4];
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-            const float p0 = exp2f(s[n][0] - mn0), p1 = exp2f(s[n][1] - mn0);
-            const float p2 = exp2f(s[n][2] - mn1), p3 = exp2f(s[n][3] - mn1);
-            rs0 += p0 + p1;
-            rs1 += p2 + p3;
-            pf[n >> 1][(n & 1) * 2 + 0] = pack_act2(p0, p1);
-            pf[n >> 1][(n & 1) * 2 + 1] = pack_act2(p2, p3);
-        }
-        rs0 += __shfl_xor_sync(0xffffffffu, rs0, 1);
-        rs0 += __shfl_xor_sync(0xffffffffu, rs0, 2);
-        rs1 += __shfl_xor_sync(0xffffffffu, rs1, 1);
-        rs1 += __shfl_xor_sync(0xffffffffu, rs1, 2);
-        l0 = l0 * sc0 + rs0;
-        l1 = l1 * sc1 + rs1;
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-            o[n][0] *= sc0;
-            o[n][1] *= sc0;
-            o[n][2] *= sc1;
-            o[n][3] *= sc1;
-        }
-        // O += P V   (B fragments of V through ldmatrix.trans: rows = keys, cols = d)
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) {
-#pragma unroll
-            for (int n = 0; n < 8; ++n) {
-                uint32_t b0, b1;
-                const int r = kk * 16 + (lane & 15);
-                ldmatrix_x2_trans(b0, b1, smem_u32(&Vs[buf][r][n * 8]));
-                mma_16816(o[n], pf[kk], b0, b1);
-            }
-        }
-        named_bar_sync(1 + grp, 128);
-    }
-    // merge the two groups' online-softmax states: group 1 -> shared memory -> group 0
-    __syncthreads();  // all tiles consumed: the K/V buffers can be reused as scratch
-    float* scratch = reinterpret_cast<float*>(kv0) + gtid * 36;
-    if (grp == 1) {
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-            scratch[n * 4 + 0] = o[n][0];
-            scratch[n * 4 + 1] = o[n][1];
-            scratch[n * 4 + 2] = o[n][2];
-            scratch[n * 4 + 3] = o[n][3];
-        }
-        scratch[32] = m0;
-        scratch[33] = m1;
-        scratch[34] = l0;
-        scratch[35] = l1;
-    }
-    __syncthreads();
-    if (grp == 1) return;
-    {
-        const float mb0 = scratch[32], mb1 = scratch[33];
-        const float mn0 = fmaxf(m0, mb0), mn1 = fmaxf(m1, mb1);  // group 0 always has a tile: finite
-        const float sa0 = exp2f(m0 - mn0), sa1 = exp2f(m1 - mn1), sb0 = exp2f(mb0 - mn0), sb1 = exp2f(mb1 - mn1);
-        l0 = l0 * sa0 + scratch[34] * sb0;
-        l1 = l1 * sa1 + scratch[35] * sb1;
-#pragma unroll
-        for (int n = 0; n < 8; ++n) {
-            o[n][0] = o[n][0] * sa0 + scratch[n * 4 + 0] * sb0;
-            o[n][1] = o[n][1] * sa0 + scratch[n * 4 + 1] * sb0;
-            o[n][2] = o[n][2] * sa1 + scratch[n * 4 + 2] * sb1;
-            o[n][3] = o[n][3] * sa1 + scratch[n * 4 + 3] * sb1;
-        }
-    }
-    const float inv0 = 1.0f / l0, inv1 = 1.0f / l1;
-    const int r0 = q0 + warp * 16 + g, r1 = r0 + 8;
-#pragma unroll
-    for (int n = 0; n < 8; ++n) {
-        const int d = n * 8 + 2 * t;
-        if (r0 < N)
-            *reinterpret_cast<uint32_t*>(out + (static_cast<size_t>(b) * N + r0) * C + h * kAttD + d) =
-                pack_act2(o[n][0] * inv0, o[n][1] * inv0);
-        if (r1 < N)
-            *reinterpret_cast<uint32_t*>(out + (static_cast<size_t>(b) * N + r1) * C + h * kAttD + d) =
-                pack_act2(o[n][2] * inv1, o[n][3] * inv1);
-    }
-}
-
-cudaError_t configure_attention() {
-    return cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttSmemBytes);
-}
-
-cudaError_t launch_attention(const act_t* qkv, act_t* o, int B, int N, int heads, cudaStream_t s) {
-    static const cudaError_t cfg = configure_attention();  // > 48 KB of dynamic shared memory
-    if (cfg != cudaSuccess) return cfg;
-    dim3 grid((N + kAttBQ - 1) / kAttBQ, heads, B);
-    return launch_pdl(attention_kernel, grid, dim3(kAttThreads), kAttSmemBytes, s, qkv, o, N, heads);
-}
-
-#endif  // CDC_TOOLS
-
 // =====================================================================================================================
-// tcgen05 version: S = Q K^T and O_tile = P V run on the 5th-generation tensor cores with TMEM accumulators.
+// S = Q K^T and O_tile = P V run on the 5th-generation tensor cores (tcgen05) with TMEM accumulators.
 //
 //   CTA = 128 queries of one head; K/V tiles of 128 keys stream through a 2-deep TMA ring.
 //   warp 0 : TMA producer (Q once, then K and V tiles; rows past N are zero-filled by the 3-D tensor map)
@@ -299,8 +82,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) attention_tc_kernel(const __gri
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = *tmem_holder;
-    pdl_wait();
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
 
     if (warp == 0) {
         if (lane == 0) {
@@ -483,7 +264,8 @@ cudaError_t launch_attention_tc(const AttnTcParams& p, int B, cudaStream_t s) {
     static const cudaError_t cfg = configure_attention_tc();
     if (cfg != cudaSuccess) return cfg;
     dim3 grid((p.N + 127) / 128, p.heads, B);
-    return launch_pdl(attention_tc_kernel, grid, dim3(kTcThreads), kTcSmemBytes, s, p);
+    attention_tc_kernel<<<grid, kTcThreads, kTcSmemBytes, s>>>(p);
+    return cudaGetLastError();
 }
 
 }  // namespace cdc

@@ -2,7 +2,7 @@
 # Builds the CUDA extension in-tree for sm_100a (nvcc cross-compiles without a GPU).
 #   build.sh            -> libcdc_b200.so        the product (fp16 storage, no environment switches, no tools hooks)
 #   build.sh bf16       -> libcdc_b200_bf16.so   same sources with -DCDC_ACT_FP16=0: the bf16 variant the precision tests measure
-#   build.sh tools      -> libcdc_b200_tools.so  -DCDC_TOOLS: environment A/B switches, graph-skip hook, mma.sync attention
+#   build.sh tools      -> libcdc_b200_tools.so  -DCDC_TOOLS: graph-skip hook (CDC_GRAPH_SKIP), flushed conv timing (CDC_TEST_CONV_REPS), barrier-timeout messages
 #   build.sh all        -> all three
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
@@ -36,7 +36,6 @@ case "${what}" in
   product) build_variant product ;;
   bf16)    build_variant bf16 -DCDC_ACT_FP16=0 ;;
   tools)   build_variant tools -DCDC_TOOLS ;;
-  x2)      build_variant x2 -DCDC_XF_F32X2=1 ;;   # A/B experiment (tools/ab_bench.sh): packed fp32 pairs in the GroupNorm transform
   all)     build_variant product & p1=$!; build_variant bf16 -DCDC_ACT_FP16=0 & p2=$!; build_variant tools -DCDC_TOOLS & p3=$!
            wait $p1; wait $p2; wait $p3 ;;
   *) echo "usage: build.sh [product|bf16|tools|all]" >&2; exit 2 ;;

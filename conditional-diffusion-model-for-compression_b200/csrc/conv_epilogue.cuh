@@ -63,7 +63,7 @@ constexpr int kEpiThreads = kEpiWarps * 32;
 template <int BN, int CPG, int EPI>
 __device__ __forceinline__ void conv_epilogue_tile(const EpiArgs& e, uint32_t taddr, uint32_t bar_tempty,
                                                    const float* bs, float* red, int q, int half, int lane, bool valid,
-                                                   size_t pix, int n0, gn_sum_t* gn_dst, long long* dbg = nullptr, bool arrive = true) {
+                                                   size_t pix, int n0, gn_sum_t* gn_dst, bool arrive = true) {
     if constexpr (EPI == EPI_DDIM) {
         if (half != 0) return;
         uint32_t v[16];
@@ -101,7 +101,6 @@ __device__ __forceinline__ void conv_epilogue_tile(const EpiArgs& e, uint32_t ta
             uint32_t v[32];
             tmem_ld32(taddr + c0 + ch * 32, v);
             tmem_ld_wait();
-            if (dbg && ch == 0) dbg[1] = clock64();
             if (ch == NCH - 1 && arrive) {  // this warp's share of the accumulator (group) is drained
                 tc_fence_before();
                 mbar_arrive(bar_tempty);
@@ -153,7 +152,6 @@ __device__ __forceinline__ void conv_epilogue_tile(const EpiArgs& e, uint32_t ta
                 }
             }
         }
-        if (dbg) dbg[2] = clock64();
         {   // saturation diagnostics: exact from the packed outputs, or (EPI_STATS) conservative from the sums of squares
             // this thread already holds -- see conv_kf.cu
             bool sat = act2_is_sat(amax2);
@@ -175,7 +173,6 @@ __device__ __forceinline__ void conv_epilogue_tile(const EpiArgs& e, uint32_t ta
                 red[((half * 4 + q) * 16 + g) * 2 + 0] = ws;
                 red[((half * 4 + q) * 16 + g) * 2 + 1] = wq;
             }
-            if (dbg) dbg[3] = clock64();
             named_bar_sync(1, kEpiThreads);
             const int t = (half * 4 + q) * 32 + lane;
             if (t < 2 * GH) {

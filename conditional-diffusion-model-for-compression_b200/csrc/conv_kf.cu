@@ -42,7 +42,6 @@
 #include "conv_kf.cuh"
 #include "kernels.cuh"
 #include "gn_apply.cuh"
-#include "launch.cuh"
 #include "ptx.cuh"
 #include "sampler.cuh"
 
@@ -134,30 +133,8 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
     const int nt = blockIdx.x / p.G1, cta = blockIdx.x % p.G1;
     const int py = MODE == 1 ? (nt & 3) >> 1 : 0, px = MODE == 1 ? nt & 1 : 0;  // output parity (UP2)
     const int cot = MODE == 1 ? nt >> 2 : nt;                                     // output-channel tile
-    const bool kdbg = p.dbg != nullptr && blockIdx.x == 0 && warp == 1 && lane == 0;
-    if (kdbg) {
-        p.dbg[500] = clock64();
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        p.dbg[508] = static_cast<long long>(gt);
-    }
-    if (p.dbg != nullptr && warp == 1 && lane == 0 && blockIdx.x < 160) {  // every CTA: lifetime in globaltimer ns, SM id
-        unsigned long long gt;
-        uint32_t smid;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        p.dbg[512 + 3 * blockIdx.x] = static_cast<long long>(gt);
-        p.dbg[514 + 3 * blockIdx.x] = smid;
-    }
     const int units = p.batch * p.nseg * p.S;
     if (threadIdx.x == 0) stamp_begin(p.stamp);
-    // tools only (strip_timeline.py): timing experiments that break the results -- 1: epilogue drains without work, 2: issuer
-    // skips its tcgen05 fences, 4: accumulators are not re-zeroed, 8: producer ignores the accumulator ring
-#ifdef CDC_TOOLS
-    const int dmode = p.dbg != nullptr ? static_cast<int>(p.dbg[511]) : 0;
-#else
-    constexpr int dmode = 0;
-#endif
 
     if (warp == 0 && lane == 0) {
         prefetch_tensormap(&p.amap[0]);
@@ -184,8 +161,8 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
         if (lane == 0) mbar_init(bar_wres, 1);
         fence_mbar_init();
         __syncwarp();
-        // The weight block starts loading right away -- before the TMEM allocation and the CTA-wide sync (its barrier
-        // was initialised by this warp), and before griddepcontrol.wait: weights are constants.
+        // The weight block starts loading right away, before the TMEM allocation and the CTA-wide sync (its barrier
+        // was initialised by this warp).
         // smem block order [kw][chunk][2 - kh]: the kh taps of one (kw, chunk) form one contiguous B operand; the loads
         // are numbered in the order the MMAs consume them (chunk, horizontal tap, kh), load l by lane l % 32.
         // (Letting the issuer start on the first (chunk, kw) group while the rest is still landing was tried in round 2 --
@@ -226,10 +203,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_holder;
-    if (kdbg) p.dbg[501] = clock64();
-
-    pdl_wait();  // everything below touches activations written by the preceding kernels
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
 
     auto decode = [&](int u, int& b, int& seg, int& si, int& h0, int& L) {
         si = u % p.S;
@@ -257,7 +230,7 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                     // input row i opens the accumulator of output row i (stride 2: of row i / 2, i even): drained and re-zeroed?
                     if (MODE == 2 ? ((i & 1) == 0 && (i >> 1) < L) : i < L) {
                         const uint32_t gi = g + (MODE == 2 ? (i >> 1) : i);
-                        if (!(dmode & 8)) mbar_wait(bar_tempty + 8 * (gi % NACC), (gi / NACC) & 1);
+                        mbar_wait(bar_tempty + 8 * (gi % NACC), (gi / NACC) & 1);
                     }
                     // (the fused 1x1 conv's short accumulator ring is NOT waited for here: with only 2 slots that would tie
                     // the load of row i to the epilogue's progress three rows back -- measured 5300 instead of 2750 cycles per
@@ -310,13 +283,7 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
             const uint32_t wlo = wbase >> 4;
             uint32_t rslot = 0, rpar = 0;
             uint32_t g = 0;  // running output-row counter: row j of the current strip uses accumulator (g + j) % NACC
-#ifdef CDC_TOOLS
-            if (kdbg) p.dbg[502] = clock64();
-#endif
             mbar_wait(bar_wres, 0);
-#ifdef CDC_TOOLS
-            if (kdbg) p.dbg[503] = clock64();
-#endif
             // accumulator window of input row i: it feeds output rows j = i - py - e, e = 0 .. NKH-1 (kh = py + e), clipped to
             // the strip (stride 2: even i -> rows i/2 - 1 (kh = 2) and i/2 (kh = 0); odd i -> row i/2 (kh = 1)); a window
             // that wraps around the accumulator ring is issued as two pieces (A, then B)
@@ -363,14 +330,7 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                 uint32_t alo_base = (ring + rslot * kKfRowBytes) >> 4;
                 mbar_wait(bar_afull + 8 * rslot, rpar);  // first chunk of the strip
                 tc_fence_after();
-#ifdef CDC_TOOLS
-                if (kdbg && u == cta) p.dbg[504] = clock64();
-#endif
                 for (int i = 0; i < nrows; ++i) {
-#ifdef CDC_TOOLS
-                    const bool dbg = p.dbg != nullptr && blockIdx.x == 0 && u == cta && i < 40;
-                    if (dbg) p.dbg[i * 4 + 0] = clock64();
-#endif
                     RowP nxt = cur;
 #pragma unroll
                     for (int pc = 0; pc < CH * NSUB; ++pc) {
@@ -423,9 +383,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                         } else {
                             pin(alo_next ^ rempty_bar);
                         }
-#ifdef CDC_TOOLS
-                        if (dbg && pc == 0) p.dbg[i * 4 + 1] = clock64();
-#endif
                         if (cur.cnt != 0) steps(std::integral_constant<int, TH>{}, std::integral_constant<int, TT>{}, cur.dA, cur.bA, cur.iA);
                         if (cur.nB != 0) steps(std::integral_constant<int, 0>{}, std::integral_constant<int, TT>{}, cur.dB, cur.bB, cur.iB);
                         if (RES1 && i >= 1 && i <= L) {  // fused 1x1 residual conv: centre tap, its own accumulator ring
@@ -442,9 +399,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                         }
                         umma_commit(rempty_bar);                          // chunk consumed
                         if (lastpc && cur.tf != 0u) umma_commit(cur.tf);  // an output row is complete
-#ifdef CDC_TOOLS
-                        if (dbg && pc == 0) p.dbg[i * 4 + 2] = clock64();
-#endif
                         if (!ready) mbar_wait(bar_afull + 8 * nslot, npar);
                         if (more) tc_fence_after();
                         rslot = nslot;
@@ -452,15 +406,9 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                         alo_base = alo_next;
                     }
                     cur = nxt;
-#ifdef CDC_TOOLS
-                    if (dbg) p.dbg[i * 4 + 3] = clock64();
-#endif
                 }
                 g += L;
             }
-#ifdef CDC_TOOLS
-            if (kdbg) p.dbg[505] = clock64();
-#endif
         }
         __syncwarp();
     }
@@ -606,21 +554,8 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                             for (int s8 = 0; s8 < HC / 16; ++s8) st_global_v8(rdst + 2 * s8, xo[2 * s8], xo[2 * s8 + 1]);
                         }
                     }
-                    long long* edbg = (p.dbg != nullptr && blockIdx.x == 0 && warp == 4 && lane == 0 && u == cta && j < 30) ? p.dbg + 256 + j * 8 : nullptr;
-                    if (edbg) edbg[0] = clock64();
                     mbar_wait(bar_tfull + 8 * slot, (gj / NACC) & 1);
                     tc_fence_after();
-                    if (edbg) edbg[1] = clock64();
-                    if (dmode & 1) {  // tools only: MMA phase without epilogue work
-                        if (!(dmode & 4)) {
-                            tmem_zero<HC>(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * BN + half * HC);
-                            if (ALIAS && slot < NALIAS) tmem_zero<HC>(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + (NACC + slot) * BN + half * HC);
-                            tmem_st_wait();
-                        }
-                        tc_fence_before();
-                        mbar_arrive(bar_tempty + 8 * slot);
-                        continue;
-                    }
                     const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + slot * BN + half * HC;
                     uint32_t v[HC];
                     tmem_ld_cols<HC>(taddr, v);
@@ -641,7 +576,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                     tmem_st_wait();
                     tc_fence_before();
                     mbar_arrive(bar_tempty + 8 * slot);
-                    if (edbg) edbg[2] = clock64();
                     float f[HC];
 #pragma unroll
                     for (int c = 0; c < HC; ++c) f[c] = kBiasAcc ? __uint_as_float(v[c]) : __uint_as_float(v[c]) + __uint_as_float(bias_r[c]);
@@ -665,7 +599,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                         o[s4].w = pack_act2(f[s4 * 8 + 6], f[s4 * 8 + 7]);
                         if constexpr (EPI != EPI_STATS) amax2 = act2_absmax(amax2, o[s4]);  // (EPI_STATS: see below)
                     }
-                    if (edbg) edbg[3] = clock64();
                     if constexpr (STAGE) {
                         // 128 pixel rows x 128 B, 128-byte swizzle: 16-byte chunk c of row r sits at chunk c ^ (r & 7)
                         const uint32_t sb = stage + (tile_ctr & 1) * (128 * BN * 2) + row * 128;
@@ -677,10 +610,8 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                                          : "memory");
                         }
                         fence_proxy_async_smem();
-                        if (edbg) edbg[4] = clock64();
                         if (store_leader) bulk_wait_group_read<0>();  // the previous row's store has left its buffer
                         named_bar_sync(1, kEpiThreads);
-                        if (edbg) edbg[5] = clock64();
                         if (store_leader) {
                             tma_store_4d(&p.omap, stage + (tile_ctr & 1) * (128 * BN * 2), cot * BN, seg * 128, h0 + j, b);
                             bulk_commit_group();
@@ -700,7 +631,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                             for (int s4 = 0; s4 < HC / 8; ++s4) dst[s4] = o[s4];
                         }
                     }
-                    if (edbg) edbg[6] = clock64();
                 }
                 g += L;
                 // Saturation diagnostics.  Without statistics: exact, from the packed outputs.  With GroupNorm statistics the
@@ -785,14 +715,7 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                 const uint32_t slot = n % static_cast<uint32_t>(NS), par = (n / static_cast<uint32_t>(NS)) & 1u;
                 const int h = h0 - 1 + i;
                 const bool row_in = h >= 0 && h < p.H;
-#ifdef CDC_TOOLS
-                long long* xdbg = (p.dbg != nullptr && blockIdx.x == 0 && lane == 0 && (warp & 3) == 0 && u == cta && n < 48) ? p.dbg + 1024 + n * 4 : nullptr;
-                if (xdbg) xdbg[0] = clock64();
-#endif
                 mbar_wait(bar_rfull + 8 * slot, par);
-#ifdef CDC_TOOLS
-                if (xdbg) xdbg[1] = clock64();
-#endif
                 if (row_in) {
                     const uint32_t sb = ring + slot * kKfRowBytes + toff;
                     // per half: all loads, all arithmetic, all stores, with distinct registers per vector -- a store that
@@ -822,18 +745,12 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
                         }
                     };
                     part(std::integral_constant<int, 0>{}, std::integral_constant<int, 3>{});
-#ifdef CDC_TOOLS
-                    if (xdbg) xdbg[2] = clock64();
-#endif
                     part(std::integral_constant<int, 3>{}, std::integral_constant<int, 6>{});
                     part(std::integral_constant<int, 6>{}, std::integral_constant<int, 9>{});
                 }
                 fence_proxy_async_smem();  // generic-proxy writes -> visible to the MMA's async-proxy reads
                 __syncwarp();
                 if (lane == 0) mbar_arrive(bar_rready + 8 * slot);
-#ifdef CDC_TOOLS
-                if (xdbg) xdbg[3] = clock64();
-#endif
             }
         }
     }
@@ -841,17 +758,6 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
     tc_fence_before();
     __syncthreads();
     if (threadIdx.x == 0) stamp_end(p.stamp);
-    if (kdbg) {
-        p.dbg[506] = clock64();
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        p.dbg[509] = static_cast<long long>(gt);
-    }
-    if (p.dbg != nullptr && warp == 1 && lane == 0 && blockIdx.x < 160) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        p.dbg[513 + 3 * blockIdx.x] = static_cast<long long>(gt);
-    }
     if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
@@ -886,16 +792,14 @@ int kf_smem_bytes(int bn, int CH, int NS, bool staged, int mode, bool res) {
     return 1024 + NS * kKfRowBytes + ((mode == 1 ? 4 : 9) + (res ? 1 : 0)) * CH * bn * 128 + (staged ? 2 * 128 * bn * 2 : 0) + kKfAux;
 }
 
-bool kf_plan(int bn, int CH, int mode, bool res, int epi, int* NS, bool* staged, int ring_ch1) {
+bool kf_plan(int bn, int CH, int mode, bool res, int* NS, bool* staged) {
     const int limit = 227 * 1024;
-    ring_ch1 = ring_ch1 < 3 ? 3 : ring_ch1 > kKfMaxSlots ? kKfMaxSlots : ring_ch1;
     for (int st = (mode == 1 || res) ? 0 : 1; st >= 0; --st) {  // NS = ring slots of one (row, chunk) each
         if (st && bn != 64) continue;
         // (a single staging buffer + a 3-slot ring for the two-chunk store-only stem was tried: 35 -> 43 us)
-        (void)epi;
         // (stride 2: two slots per (row, chunk); one-chunk convs: a deeper ring where shared memory allows -- the input
         // transform adds a pipeline stage)
-        for (int ns = mode == 2 ? kKfMaxSlots : CH == 1 ? ring_ch1 : 4; ns >= (mode == 2 ? 4 : 3); --ns)
+        for (int ns = mode == 2 ? kKfMaxSlots : CH == 1 ? 6 : 4; ns >= (mode == 2 ? 4 : 3); --ns)
             if (kf_smem_bytes(bn, CH, ns, st != 0, mode, res) <= limit) {
                 *NS = ns;
                 *staged = st != 0;
@@ -905,10 +809,10 @@ bool kf_plan(int bn, int CH, int mode, bool res, int epi, int* NS, bool* staged,
     return false;
 }
 
-bool kf_inst_ok(int bn, int cpg, int epi, int CH, int mode, bool res, bool apply, int ring_ch1) {
+bool kf_inst_ok(int bn, int cpg, int epi, int CH, int mode, bool res, bool apply) {
     int ns;
     bool st;
-    if (!kf_plan(bn, CH, mode, res, epi, &ns, &st, ring_ch1)) return false;
+    if (!kf_plan(bn, CH, mode, res, &ns, &st)) return false;
     // APPLY: transform group g owns the chunks n = g (mod 2) and waits on ring slot n % NS by parity -- sound only when
     // a slot always belongs to the same group, i.e. for an EVEN ring (ADVICE r1)
     if (apply && (ns & 1)) return false;
@@ -938,8 +842,10 @@ cudaError_t launch_conv_kf(const KfParams& p, int bn, int cpg, int epi, int CH, 
     if (smem > 227 * 1024) return cudaErrorInvalidValue;
 #define KF_CASE(BN_, CPG_, EPI_, CH_, ST_, X_, M_, R_, A_)                                                                                \
     if (bn == BN_ && (EPI_ != EPI_STATS || cpg == CPG_) && epi == EPI_ && CH == CH_ && st == ST_ && xk16 == X_ && mode == M_ && res == R_ && \
-        apply == A_)                                                                                                                         \
-        return launch_pdl(conv_kf_kernel<BN_, CPG_, EPI_, CH_, ST_, X_, M_, R_, A_>, grid, block, smem, stream, p);
+        apply == A_) {                                                                                                                       \
+        conv_kf_kernel<BN_, CPG_, EPI_, CH_, ST_, X_, M_, R_, A_><<<grid, block, smem, stream>>>(p);                                         \
+        return cudaGetLastError();                                                                                                           \
+    }
     KF_ALL_CASES()
 #undef KF_CASE
     return cudaErrorInvalidValue;

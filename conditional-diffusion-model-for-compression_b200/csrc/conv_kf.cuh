@@ -41,16 +41,14 @@ struct alignas(64) KfParams {
     int step;
     long long* stamp;     // diagnostics, may be null (see ConvParams)
     unsigned int* sat;
-    long long* dbg;       // optional: issuer / epilogue timeline of CTA 0 (clock64 stamps), tools only
 };
 
 // mode 0: 3x3 conv; mode 1: nearest-x2 upsample + 3x3 conv (four parity 2x2 convs on the low-resolution input);
 // mode 2: 3x3 conv with stride 2 (H, W of KfParams are the OUTPUT grid)
 // res: the ResBlock's 1x1 residual conv rides along (its weights are resident too, its accumulators share TMEM)
 // apply: GroupNorm + SiLU of the input applied in shared memory (see in_acc)
-// ring_ch1: input-ring slots wanted for one-chunk convs (default 6)
-bool kf_inst_ok(int bn, int cpg, int epi, int CH, int mode, bool res, bool apply = false, int ring_ch1 = 6);
-bool kf_plan(int bn, int CH, int mode, bool res, int epi, int* NS, bool* staged, int ring_ch1 = 6);  // shared-memory plan; false if the weights do not fit
+bool kf_inst_ok(int bn, int cpg, int epi, int CH, int mode, bool res, bool apply = false);
+bool kf_plan(int bn, int CH, int mode, bool res, int* NS, bool* staged);  // shared-memory plan; false if the weights do not fit
 int kf_smem_bytes(int bn, int CH, int NS, bool staged, int mode, bool res);
 cudaError_t configure_kf_kernels();
 cudaError_t launch_conv_kf(const KfParams& p, int bn, int cpg, int epi, int CH, bool xk16, int mode, bool res, bool apply,

@@ -17,7 +17,6 @@
 
 #include "conv_epilogue.cuh"
 #include "conv_tc.cuh"
-#include "launch.cuh"
 #include "ptx.cuh"
 
 namespace cdc {
@@ -92,8 +91,6 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_tc_kernel(const __grid_c
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_holder;
-    pdl_wait();  // the prologue above overlapped the preceding kernel's tail
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
 
     auto decode = [&](int tile, int& nt, int& ph, int& b, int& th, int& tw) {
         nt = tile % p.n_tiles;
@@ -214,7 +211,8 @@ static cudaError_t launch_one(const ConvParams& p, int num_sms, cudaStream_t str
     auto kern = conv_tc_kernel<BN, CPG, EPI>;
     const int total = p.n_tiles * p.nphase * p.batch * p.tiles_h * p.tiles_w;
     const int grid = total < num_sms ? total : num_sms;
-    return launch_pdl(kern, dim3(grid), dim3(kConvThreads), Cfg::SMEM_BYTES, stream, p);
+    kern<<<grid, kConvThreads, Cfg::SMEM_BYTES, stream>>>(p);
+    return cudaGetLastError();
 }
 
 #define CDC_ALL_CASES()          \

@@ -4,7 +4,6 @@
 #include "gn_apply.cuh"
 #include "gn_sums.cuh"
 #include "kernels.cuh"
-#include "launch.cuh"
 #include "ptx.cuh"
 
 namespace cdc {
@@ -14,13 +13,9 @@ namespace cdc {
 // One CTA per (image, 64-pixel chunk); fixed-order reductions only.
 constexpr int kStatsPix = 64;
 
-// (tensors written by the preceding kernel are read through plain pointers, not const __restrict__: under PDL the
-// kernel is resident before that data is final, so the non-coherent read-only path must not be used for them)
 __global__ void __launch_bounds__(256) gn_stats_kernel(const act_t* x, gn_sum_t* acc, int HW, int C, long long* stamp) {
     __shared__ float s_sum[8][512], s_sq[8][512];  // [row-in-pass][channel] (C <= 512)
     if (threadIdx.x == 0) stamp_begin(stamp);
-    pdl_wait();
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
     const int b = blockIdx.y, pt = blockIdx.x;
     const int vecs = C / 8;                 // uint4 per pixel
     const int rows = (256 / vecs) < 8 ? (256 / vecs) : 8;  // pixels per pass (smem rows)
@@ -76,7 +71,8 @@ __global__ void __launch_bounds__(256) gn_stats_kernel(const act_t* x, gn_sum_t*
 cudaError_t launch_gn_stats(const act_t* x, gn_sum_t* acc, int B, int HW, int C, cudaStream_t s, long long* stamp) {
     if (C % 32 != 0 || C > 512 || C < 32) return cudaErrorInvalidValue;
     const int PT = (HW + kStatsPix - 1) / kStatsPix;
-    return launch_pdl(gn_stats_kernel, dim3(PT, B), dim3(256), 0, s, x, acc, HW, C, stamp);
+    gn_stats_kernel<<<dim3(PT, B), 256, 0, s>>>(x, acc, HW, C, stamp);
+    return cudaGetLastError();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -149,8 +145,6 @@ __global__ void __launch_bounds__(256, 4) gn_apply_kernel(const uint4* x, const 
                                                           long long vecs_per_img, const GnCoef g, int B) {
     extern __shared__ float2 s_mr[];  // [B][32] (mean, rstd)
     if (threadIdx.x == 0) stamp_begin(g.stamp);
-    pdl_wait();
-    pdl_launch_dependents();  // (after the wait: see launch.cuh)
     const long long stride = gridDim.x * 256LL;
     long long i = blockIdx.x * 256LL + threadIdx.x;
     const int cv = static_cast<int>(i % vecs_per_pix), cpg = g.C / 32;
@@ -222,10 +216,10 @@ cudaError_t launch_gn_apply(const act_t* x, const gn_sum_t* acc, const float* ga
     const GnCoef gc{acc, gamma, beta, film, C, HW, eps, stamp, sat};
     const size_t sm = static_cast<size_t>(B) * 32 * sizeof(float2);
     if (sm > 48 * 1024) return cudaErrorInvalidValue;
-    if (silu && r) return launch_pdl(gn_apply_kernel<true, true>, g, blk, sm, s, xv, rv, yv, nvec, vpp, vpi, gc, B);
-    if (silu) return launch_pdl(gn_apply_kernel<true, false>, g, blk, sm, s, xv, rv, yv, nvec, vpp, vpi, gc, B);
-    if (r) return launch_pdl(gn_apply_kernel<false, true>, g, blk, sm, s, xv, rv, yv, nvec, vpp, vpi, gc, B);
-    return launch_pdl(gn_apply_kernel<false, false>, g, blk, sm, s, xv, rv, yv, nvec, vpp, vpi, gc, B);
+    auto kern = silu ? (r ? gn_apply_kernel<true, true> : gn_apply_kernel<true, false>)
+                     : (r ? gn_apply_kernel<false, true> : gn_apply_kernel<false, false>);
+    kern<<<g, blk, sm, s>>>(xv, rv, yv, nvec, vpp, vpi, gc, B);
+    return cudaGetLastError();
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -7,12 +7,6 @@
 #include "gn_sums.cuh"
 #include "ptx.cuh"
 
-// Packed fp32 pairs (FFMA2) in the per-vector transform: measured SLOWER on B200 (the pairs cost register moves and the
-// packed form is not faster per element on the FMA pipe: APPLY convs 27.7 -> 30.5 us) -- kept for the record, off.
-#ifndef CDC_XF_F32X2
-#define CDC_XF_F32X2 0
-#endif
-
 namespace cdc {
 
 // x * sigmoid(x) = x * (0.5 + 0.5 * tanh(x / 2)): ONE MUFU op (tanh.approx.f32, max relative error 2^-11, below the
@@ -41,28 +35,12 @@ __device__ __forceinline__ uint4 gn_apply_vec(const uint4 u, const uint4 rr, con
     uint32_t o[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-        // the channel pair as ONE packed fp32 FMA (ffma2: both lanes round like fmaf, so the values are those of the
-        // scalar form bit for bit)
-#if CDC_XF_F32X2
-        const float2 v = ffma2(make_float2(c[j].x, c[j].z), make_float2(act_lo(w[j]), act_hi(w[j])), make_float2(c[j].y, c[j].w));
-        float v0 = v.x, v1 = v.y;
-        if (SILU) {
-            const float2 h = SILU_HALF ? v : make_float2(0.5f * v.x, 0.5f * v.y);
-            float2 t;
-            asm("tanh.approx.f32 %0, %1;" : "=f"(t.x) : "f"(h.x));
-            asm("tanh.approx.f32 %0, %1;" : "=f"(t.y) : "f"(h.y));
-            const float2 y = ffma2(h, t, h);  // SiLU(2h) = h + h * tanh(h) (silu_f / silu_h, pairwise)
-            v0 = y.x;
-            v1 = y.y;
-        }
-#else
         float v0 = fmaf(c[j].x, act_lo(w[j]), c[j].y);
         float v1 = fmaf(c[j].z, act_hi(w[j]), c[j].w);
         if (SILU) {
             v0 = SILU_HALF ? silu_h(v0) : silu_f(v0);
             v1 = SILU_HALF ? silu_h(v1) : silu_f(v1);
         }
-#endif
         if (RES) {
             v0 += act_lo(rw[j]);
             v1 += act_hi(rw[j]);

@@ -67,11 +67,7 @@ cudaError_t launch_repack_weight_up2(const float* src, act_t* dst, int O, int I,
 
 // ---- attention (C7; oracle/unet.py Attn) --------------------------------------------------------
 // qkv [B*N][768] act_t (q | k | v, head h = channels 64h..64h+63) -> o [B*N][256] bf16
-#ifdef CDC_TOOLS
-cudaError_t launch_attention(const act_t* qkv, act_t* o, int B, int N, int heads, cudaStream_t s);  // mma.sync A/B reference
-cudaError_t configure_attention();  // dynamic shared-memory limit (call once, outside graph capture)
-#endif
-// tcgen05 version (attention.cu): qkv_map = 3-D tensor map {768 cols, N rows, B} of the qkv tensor, box {64, 128, 1},
+// (attention.cu, tcgen05): qkv_map = 3-D tensor map {768 cols, N rows, B} of the qkv tensor, box {64, 128, 1},
 // 128-byte swizzle (built by the host runtime)
 struct alignas(64) AttnTcParams {
     CUtensorMap qkv_map;

@@ -122,14 +122,6 @@ template <int N>
 __device__ __forceinline__ void bulk_wait_group() {
     asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
 }
-// Programmatic dependent launch: wait for the preceding kernel's memory to be visible / let the next
-// kernel's CTAs start their prologue.  Both are no-ops when the launch carries no PDL attribute.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// Early trigger: only kernels whose dependents are small (GroupNorm apply, or a conv that cannot become
-// resident before this one's CTAs exit anyway) call this.  gn_apply does NOT: its dependent is a conv whose CTAs would
-// claim most of the register file next to the still-running apply CTAs (measured: -1.7 % when every kernel triggered).
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // ---------------------------------------------------------------- tcgen05 / TMEM
 __device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t ncols) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(ncols)
@@ -309,24 +301,6 @@ __device__ __forceinline__ void tmem_st_cols(uint32_t taddr, const uint32_t (&v)
                          : "memory");
         }
     }
-}
-// Packed fp32 pairs (sm_100 FFMA2 / FADD2: two IEEE fp32 operations per instruction, each lane rounded exactly like
-// the scalar form).  The fp32 FMA pipe issues a three-register instruction every other cycle per sub-partition, and the
-// conv epilogue / input transform keep it busy next to the tensor pipe: pairs halve that.
-__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
-    unsigned long long d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;"
-        : "=l"(d)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)),
-          "l"(*reinterpret_cast<const unsigned long long*>(&c)));
-    return *reinterpret_cast<float2*>(&d);
-}
-__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
-    unsigned long long d;
-    asm("add.rn.f32x2 %0, %1, %2;"
-        : "=l"(d)
-        : "l"(*reinterpret_cast<const unsigned long long*>(&a)), "l"(*reinterpret_cast<const unsigned long long*>(&b)));
-    return *reinterpret_cast<float2*>(&d);
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ uint32_t elect_one_sync() {

@@ -28,26 +28,12 @@ namespace cdc {
 
 static std::string g_create_err;
 
-// Planner decisions that tests / tools A/B through cdc_set_plan_option (include/cdc_b200_tools.h).  The product build
-// reads NO environment variables; the tools build (-DCDC_TOOLS) lets the environment override the defaults.
+// Planner decisions that tests / tools A/B through cdc_set_plan_option (include/cdc_b200_tools.h).
 struct PlanOpts {
-    int v[CDC_OPT_COUNT] = {2, 1, 1, 0, 6};
+    int v[CDC_OPT_COUNT] = {2, 1};
     int fuse_apply_max_tiles() const { return v[CDC_OPT_FUSE_APPLY]; }
     bool kf() const { return v[CDC_OPT_KF] != 0; }
-    bool kf_s2() const { return v[CDC_OPT_KF_S2] != 0; }
-    long kf_min_pixels() const { return v[CDC_OPT_KF_MIN_PIXELS]; }
-    int kf_ring() const { return v[CDC_OPT_KF_RING]; }
 };
-static PlanOpts default_plan_opts() {
-    PlanOpts o;
-#ifdef CDC_TOOLS
-    const char* names[CDC_OPT_COUNT] = {"CDC_FUSE_APPLY", "CDC_KF", "CDC_KF_S2", "CDC_KF_MIN_PIXELS", "CDC_KF_RING"};
-    for (int i = 0; i < CDC_OPT_COUNT; ++i)
-        if (const char* e = getenv(names[i])) o.v[i] = atoi(e);
-    if (getenv("CDC_NO_KF")) o.v[CDC_OPT_KF] = 0;
-#endif
-    return o;
-}
 
 // Every entry point that takes a cdc_ctx runs on the context's device and restores the caller's current device on
 // exit (ADVICE r1: a Decoder on cuda:1 must work -- and must not move the process -- while cuda:0 is current).
@@ -164,7 +150,6 @@ struct ConvBuild {
     float* x0_out = nullptr;
     const SamplerTab* samp = nullptr;  // per-step sampler coefficients (host)
     unsigned int* sat = nullptr;       // saturation diagnostics counter (device)
-    long long* dbg = nullptr;  // kf kernel issuer / epilogue timeline (tools)
     // offered: fused 1x1 residual conv of the same input (kf path only; op->desc.res1 says whether it was taken)
     const ConvW* res_w = nullptr;
     Act res_out;
@@ -216,12 +201,6 @@ static int encode_qkv_map(CUtensorMap* m, const act_t* qkv, int cols, int N, int
     const cuuint32_t box[3] = {64, 128, 1};
     return encode_map(m, qkv, 3, dims, strides, box);
 }
-#ifdef CDC_TOOLS
-static bool attention_legacy() {  // A/B switch of the tools build: the mma.sync kernel
-    static const bool v = getenv("CDC_ATTN_LEGACY") != nullptr;
-    return v;
-}
-#endif
 
 // repacked weights as the [n_pad][taps * c_pad] K-major matrix, box {64, BN}
 static int encode_w_map(CUtensorMap* m, const ConvW& w, int BN) {
@@ -245,15 +224,11 @@ static bool conv_uses_kf(const ConvBuild& cb, int B, int num_sms, const PlanOpts
     g->mode = cb.mode == MODE_UP2 ? 1 : cb.mode == MODE_S2 ? 2 : 0;
     if (g->mode == 1 && (!cb.w->up2 || cb.epi != EPI_STORE)) return false;
     if (g->mode == 2 && (cb.epi != EPI_STORE || cb.res_w || cb.in_acc || ((cb.srcs[0].W | cb.srcs[0].H) & 1))) return false;
-    // CDC_KF_S2=0: stride-2 convs through the general kernel (A/B).  Only the 64- and 128-channel downsampling convs have
-    // kf instantiations: with 32-channel N tiles (192 / 256 channels, 64x96 outputs and below) the strip form measured
-    // 3 us per step SLOWER than the general kernel.
-    if (g->mode == 2 && !po.kf_s2()) return false;
+    // (only the 64- and 128-channel downsampling convs have stride-2 kf instantiations: with 32-channel N tiles (192 / 256
+    // channels, 64x96 outputs and below) the strip form measured 3 us per step SLOWER than the general kernel)
     // strip geometry lives on the grid the kernel walks: the input grid (mode 1 writes 2x2 outputs per pixel), for the
     // stride-2 mode the OUTPUT grid
     int gw = cb.srcs[0].W >> (g->mode == 2 ? 1 : 0), gh = cb.srcs[0].H >> (g->mode == 2 ? 1 : 0);
-    // CDC_KF_MIN_PIXELS=n: levels with fewer pixels per image go through the general kernel (A/B of the small levels)
-    if (static_cast<long>(gw) * gh < po.kf_min_pixels()) return false;
     g->tr = false;
     g->nseg = (gw + 127) / 128;
     // segments are 128 pixels wide: too much of the tile would be padding (measured break-even against conv_tc.cu:
@@ -272,10 +247,10 @@ static bool conv_uses_kf(const ConvBuild& cb, int B, int num_sms, const PlanOpts
         if (cb.w->n_pad % bn || (cb.epi == EPI_STATS && bn % cb.cpg)) continue;
         // with the ResBlock's 1x1 residual conv riding along when that fits, else without
         g->res = cb.res_w != nullptr && g->mode == 0 && cb.res_w->n_pad == cb.w->n_pad && cb.res_w->taps == 1 &&
-                 cb.res_w->c_pad == ctot && kf_inst_ok(bn, cb.cpg, cb.epi, g->CH, g->mode, true, false, po.kf_ring()) &&
-                 kf_plan(bn, g->CH, g->mode, true, cb.epi, &g->NS, &g->staged, po.kf_ring());
-        if (!g->res && (!kf_inst_ok(bn, cb.cpg, cb.epi, g->CH, g->mode, false, false, po.kf_ring()) ||
-                        !kf_plan(bn, g->CH, g->mode, false, cb.epi, &g->NS, &g->staged, po.kf_ring())))
+                 cb.res_w->c_pad == ctot && kf_inst_ok(bn, cb.cpg, cb.epi, g->CH, g->mode, true) &&
+                 kf_plan(bn, g->CH, g->mode, true, &g->NS, &g->staged);
+        if (!g->res && (!kf_inst_ok(bn, cb.cpg, cb.epi, g->CH, g->mode, false) ||
+                        !kf_plan(bn, g->CH, g->mode, false, &g->NS, &g->staged)))
             continue;
         g->bn = bn;
         break;
@@ -285,7 +260,7 @@ static bool conv_uses_kf(const ConvBuild& cb, int B, int num_sms, const PlanOpts
     // channels -- gain 2.4 % and 0.8 % images/s; with 3+ tiles the redundant MUFU work costs more than the pass it replaces)
     g->apply = cb.in_acc != nullptr && !g->res && cb.srcs.size() == 1 && cb.cpg == g->CH * 2 &&
                cb.w->n_pad / g->bn <= po.fuse_apply_max_tiles() &&
-               kf_inst_ok(g->bn, cb.cpg, cb.epi, g->CH, g->mode, false, true, po.kf_ring());
+               kf_inst_ok(g->bn, cb.cpg, cb.epi, g->CH, g->mode, false, true);
     g->n_tiles = cb.w->n_pad / g->bn * (g->mode == 1 ? 4 : 1);
     if (cb.epi == EPI_DDIM && g->n_tiles != 1) return false;
     // strip geometry for a walk along image rows (tr = 0) or image columns (tr = 1): relative cost = padding of the
@@ -388,7 +363,6 @@ static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, in
     kp->x = cb.x;
     kp->xpad = cb.xpad;
     kp->x0_out = cb.x0_out;
-    kp->dbg = cb.dbg;
     kp->sat = cb.sat;
     kp->e1 = 1.0f;
     if (kg.apply) op->name += "+gn_in";  // the GroupNorm apply pass no longer touches HBM; its arithmetic rides along
@@ -659,7 +633,7 @@ struct cdc_ctx {
     bool finalized = false, has_ctx = false, has_codec = false;
     int C[4];
 
-    PlanOpts opts = default_plan_opts();
+    PlanOpts opts;
     bool opts_dirty = false;  // an option changed since the plan was built: the next cdc_bind_io re-plans
 
     // schedule
@@ -1068,23 +1042,13 @@ static int build_plans(cdc_ctx* ctx) {
         at.name = "mid.attn.sdpa";
         at.flops = static_cast<double>(B) * ctx->cfg.heads * 4.0 * HW * HW * ctx->cfg.head_dim;
         at.bytes = static_cast<double>(B) * HW * Cm * 2 * 4;
-        const act_t* qp = qkv.p;
-        act_t* op_ = o.p;
-        const int heads = ctx->cfg.heads;
         auto ap = std::shared_ptr<AttnTcParams>(new AttnTcParams());
         memset(ap.get(), 0, sizeof(AttnTcParams));
-        if (encode_qkv_map(&ap->qkv_map, qp, 3 * Cm, HW, B)) return ctx->fail(CDC_ERR_CUDA, "cuTensorMapEncodeTiled (qkv) failed");
-        ap->out = op_;
+        if (encode_qkv_map(&ap->qkv_map, qkv.p, 3 * Cm, HW, B)) return ctx->fail(CDC_ERR_CUDA, "cuTensorMapEncodeTiled (qkv) failed");
+        ap->out = o.p;
         ap->N = HW;
-        ap->heads = heads;
-        at.run = [ap, qp, op_, B, HW, heads](cudaStream_t s, int, long long* stamp) {
-#ifdef CDC_TOOLS
-            if (attention_legacy()) return launch_attention(qp, op_, B, HW, heads, s);
-#endif
-            (void)qp;
-            (void)op_;
-            (void)heads;
-            (void)HW;
+        ap->heads = ctx->cfg.heads;
+        at.run = [ap, B](cudaStream_t s, int, long long* stamp) {
             AttnTcParams q = *ap;
             q.stamp = stamp;
             return launch_attention_tc(q, B, s);
@@ -1337,11 +1301,7 @@ int cdc_create(const cdc_config* cfg, int device, cdc_ctx** out) {
         g_create_err = "cuTensorMapEncodeTiled entry point not found";
         return CDC_ERR_CUDA;
     }
-    if (
-#ifdef CDC_TOOLS
-        (e = configure_attention()) != cudaSuccess ||
-#endif
-        (e = configure_attention_tc()) != cudaSuccess || (e = configure_conv_kernels()) != cudaSuccess ||
+    if ((e = configure_attention_tc()) != cudaSuccess || (e = configure_conv_kernels()) != cudaSuccess ||
         (e = configure_kf_kernels()) != cudaSuccess) {
         g_create_err = std::string("cudaFuncSetAttribute(conv kernels): ") + cudaGetErrorString(e);
         return CDC_ERR_CUDA;
@@ -2085,56 +2045,6 @@ int cdc_test_conv(int device, const void* src0, int c0, const void* src1, int c1
         cb.cpg = cout / 32;
         cb.gn_acc = reinterpret_cast<gn_sum_t*>(gn_sums);
     }
-    void* res_buf = nullptr;
-    void* in_gn = nullptr;
-#ifdef CDC_TOOLS
-    long long* dbg = nullptr;
-    long long* dbg_dev = nullptr;
-    std::vector<long long> dbg_host(2048, 0);
-    ConvW cwr;  // tools (CDC_TEST_CONV_RES=1): time the conv with a 1x1 residual conv of the same input riding along
-    if (getenv("CDC_TEST_CONV_RES") && gn_sums && ksize == 3 && mode == MODE_S1) {
-        // its weights: the centre tap of the 3x3 weights is as good as any for timing -- w_oihw[o][i][1][1]
-        std::vector<float> w33(static_cast<size_t>(cout) * cin * 9), w11(static_cast<size_t>(cout) * cin);
-        CK(cudaMemcpy(w33.data(), w_oihw, w33.size() * 4, cudaMemcpyDeviceToHost));
-        for (size_t i = 0; i < w11.size(); ++i) w11[i] = w33[i * 9 + 4];
-        float* w11d = nullptr;
-        CK(cudaMalloc(&w11d, w11.size() * 4));
-        CK(cudaMemcpy(w11d, w11.data(), w11.size() * 4, cudaMemcpyHostToDevice));
-        int rr = make_conv_w(ctx, ar, w11d, bias, cout, cin, 1, cin, cin, false, &cwr, S(s), false);
-        cudaStreamSynchronize(S(s));
-        cudaFree(w11d);
-        if (rr == 0 && cudaMalloc(&res_buf, static_cast<size_t>(B) * H * W * cwr.n_pad * 2) == cudaSuccess) {
-            cb.res_w = &cwr;
-            cb.res_out.p = static_cast<act_t*>(res_buf);
-            cb.res_out.C = cwr.n_pad;
-            cb.res_out.H = H;
-            cb.res_out.W = W;
-        }
-    }
-    // tools (CDC_TEST_CONV_APPLY=1): time the conv with the input GroupNorm fused -- unit statistics
-    if (getenv("CDC_TEST_CONV_APPLY") && gn_sums && c1 == 0 && cout == cin) {
-        const int cpg_in = cin / 32;
-        std::vector<long long> acc(static_cast<size_t>(B) * kGnImgStride, 0);
-        for (size_t i = 0; i < acc.size(); i += kGnVals)
-            acc[i + 2] = static_cast<long long>(cpg_in) * H * W / 1024;  // mean 0, variance ~1 (squares_hi counts 1024s)
-        std::vector<float> gb(2 * cin, 0.0f);
-        for (int i = 0; i < cin; ++i) gb[i] = 1.0f;
-        CK(cudaMalloc(&in_gn, acc.size() * 8 + gb.size() * 4));
-        CK(cudaMemcpy(in_gn, acc.data(), acc.size() * 8, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(static_cast<char*>(in_gn) + acc.size() * 8, gb.data(), gb.size() * 4, cudaMemcpyHostToDevice));
-        cb.in_acc = static_cast<const gn_sum_t*>(in_gn);
-        cb.in_gamma = reinterpret_cast<const float*>(static_cast<char*>(in_gn) + acc.size() * 8);
-        cb.in_beta = cb.in_gamma + cin;
-    }
-    if (getenv("CDC_STRIP_DEBUG")) {
-        // plain device memory (managed memory would page-fault inside the timed regions)
-        cudaMalloc(&dbg_dev, 2048 * sizeof(long long));
-        std::vector<long long> init(2048, 0);
-        init[511] = atoi(getenv("CDC_STRIP_DEBUG")) / 2;  // 2: no epilogue work; 6 / 10 / 18: + no fences / no re-zero / no ring wait
-        cudaMemcpy(dbg_dev, init.data(), 2048 * sizeof(long long), cudaMemcpyHostToDevice);
-        cb.dbg = dbg_dev;
-    }
-#endif
     Op op;
     std::string e;
     r = build_conv(cb, B, prop.multiProcessorCount, tmp.opts, &op, &e);
@@ -2143,10 +2053,6 @@ int cdc_test_conv(int device, const void* src0, int c0, const void* src1, int c1
         ar.release();
         return r;
     }
-#ifdef CDC_TOOLS
-    if (cb.res_w) printf("test_conv: 1x1 residual conv fused: %s\n", op.desc.res1 ? "yes" : "no");
-    if (cb.in_acc) printf("test_conv: input GroupNorm fused: %s\n", op.desc.apply ? "yes" : "no");
-#endif
     cudaError_t ce = op.run(S(s), 0, nullptr);
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(S(s));
 #ifdef CDC_TOOLS
@@ -2177,55 +2083,8 @@ int cdc_test_conv(int device, const void* src0, int c0, const void* src1, int c1
         cudaEventDestroy(e0);
         cudaEventDestroy(e1);
     }
-    if (dbg_dev) {
-        cudaMemcpy(dbg_host.data(), dbg_dev, 2048 * sizeof(long long), cudaMemcpyDeviceToHost);
-        cudaFree(dbg_dev);
-        dbg = dbg_host.data();
-    }
-    KfGeom kgd;
-    if (dbg && conv_uses_kf(cb, B, prop.multiProcessorCount, tmp.opts, &kgd)) {
-        printf("kf issuer timeline (CTA 0, first strip; S=%d NS=%d staged=%d): row: issue_a wait_next issue_b | since previous row start\n", kgd.S,
-               kgd.NS, kgd.staged ? 1 : 0);
-        for (int i = 0; i < 40 && dbg[i * 4 + 3]; ++i)
-            printf("  %2d: %6lld %6lld %6lld | %6lld\n", i, dbg[i * 4 + 1] - dbg[i * 4 + 0], dbg[i * 4 + 2] - dbg[i * 4 + 1],
-                   dbg[i * 4 + 3] - dbg[i * 4 + 2], i ? dbg[i * 4 + 0] - dbg[(i - 1) * 4 + 0] : 0LL);
-        printf("kf CTA 0 phases (cycles): prologue %lld, to-issuer %lld, weights wait %lld, first row wait %lld, main loop %lld, drain+exit %lld\n",
-               dbg[501] - dbg[500], dbg[502] - dbg[501], dbg[503] - dbg[502], dbg[504] - dbg[503], dbg[505] - dbg[504], dbg[506] - dbg[505]);
-        printf("kf CTA 0: %lld cycles in %lld ns -> SM clock %.0f MHz\n", dbg[506] - dbg[500], dbg[509] - dbg[508],
-               1e3 * static_cast<double>(dbg[506] - dbg[500]) / static_cast<double>(dbg[509] - dbg[508]));
-        if (dbg[1024 + 3] || dbg[1024 + 7]) {
-            printf("kf input-transform timeline (first warp of each group; chunk n belongs to group n %% 2): chunk: wait part1 parts2+3+arrive | total, start since the group's previous chunk\n");
-            for (int n = 0; n < 48 && (dbg[1024 + n * 4 + 3] || n < 2); ++n) {
-                const long long* e = dbg + 1024 + n * 4;
-                if (!e[3]) continue;
-                printf("  %2d: %6lld %6lld %6lld | %6lld %6lld\n", n, e[1] - e[0], e[2] ? e[2] - e[1] : 0LL, e[2] ? e[3] - e[2] : e[3] - e[1], e[3] - e[0],
-                       n >= 2 && (e - 8)[3] ? e[0] - (e - 8)[0] : 0LL);
-            }
-        }
-        printf("kf epilogue warp 4 timeline: tile: wait_tfull ldtm math sts+fence bar tma | total, since previous\n");
-        for (int i = 0; i < 30 && dbg[256 + i * 8 + 1]; ++i) {
-            const long long* e = dbg + 256 + i * 8;
-            printf("  %2d: %6lld %6lld %6lld %6lld %6lld %6lld | %6lld %6lld\n", i, e[1] - e[0], e[2] - e[1], e[3] - e[2], e[4] - e[3],
-                   e[5] - e[4], e[6] - e[5], e[6] - e[0], i ? e[0] - (e - 8)[0] : 0LL);
-        }
-        {  // lifetimes of all CTAs relative to the earliest start
-            long long t0 = 0, t1 = 0;
-            int n = 0;
-            for (int c = 0; c < 160 && dbg[512 + 3 * c]; ++c, ++n) {
-                t0 = n == 0 ? dbg[512 + 3 * c] : std::min(t0, dbg[512 + 3 * c]);
-                t1 = std::max(t1, dbg[513 + 3 * c]);
-            }
-            printf("kf CTAs: %d, first start -> last end %lld ns; per CTA (start, end, SM):", n, t1 - t0);
-            for (int c = 0; c < n; ++c)
-                printf("%s %lld-%lld@%lld", c % 8 == 0 ? "\n " : "", dbg[512 + 3 * c] - t0, dbg[513 + 3 * c] - t0, dbg[514 + 3 * c]);
-            printf("\n");
-        }
-        dbg = nullptr;
-    }
 #endif
     ar.release();
-    if (in_gn) cudaFree(in_gn);
-    if (res_buf) cudaFree(res_buf);
     if (ce != cudaSuccess) {
         g_create_err = std::string("test_conv: ") + cudaGetErrorString(ce);
         return CDC_ERR_CUDA;
@@ -2236,12 +2095,6 @@ int cdc_test_conv(int device, const void* src0, int c0, const void* src1, int c1
 int cdc_test_attention(const void* qkv, void* out, int B, int N, int heads, cdc_stream s) {
     if (!qkv || !out || B < 1 || N < 1 || heads < 1) return CDC_ERR_SHAPE;
     if (configure_attention_tc() != cudaSuccess) return CDC_ERR_CUDA;
-#ifdef CDC_TOOLS
-    if (attention_legacy())
-        return launch_attention(static_cast<const act_t*>(qkv), static_cast<act_t*>(out), B, N, heads, S(s)) == cudaSuccess
-                   ? CDC_OK
-                   : CDC_ERR_CUDA;
-#endif
     AttnTcParams ap;
     memset(&ap, 0, sizeof ap);
     if (encode_qkv_map(&ap.qkv_map, static_cast<const act_t*>(qkv), 3 * heads * 64, N, B)) return CDC_ERR_CUDA;

@@ -2,9 +2,9 @@
  *
  * NOT part of the drop-in boundary (include/cdc_b200.h): nothing here is needed to decode, and nothing here can change
  * what cdc_decode computes.  tests/ and tools/ bind these through ctypes next to the product symbols.
- * (The measurement hooks that DO alter results -- leaving op classes out of the captured graph, environment switches,
- * the mma.sync attention kernel -- exist only in the separate tools build, libcdc_b200_tools.so, compiled with
- * -DCDC_TOOLS by `csrc/build.sh tools`.)
+ * (The measurement hook that DOES alter results -- leaving op classes out of the captured graph -- and the environment
+ * switches exist only in the separate tools build, libcdc_b200_tools.so, compiled with -DCDC_TOOLS by
+ * `csrc/build.sh tools`.)
  */
 #ifndef CDC_B200_TOOLS_H
 #define CDC_B200_TOOLS_H
@@ -19,10 +19,7 @@ extern "C" {
 typedef enum {
     CDC_OPT_FUSE_APPLY = 0,     /* N tiles a conv may have for the input-GroupNorm fusion; 0 = never fuse.  default 2 */
     CDC_OPT_KF = 1,             /* 0: every conv through the general kernel (conv_tc.cu).  default 1 */
-    CDC_OPT_KF_S2 = 2,          /* 0: stride-2 convs through the general kernel.  default 1 */
-    CDC_OPT_KF_MIN_PIXELS = 3,  /* levels with fewer pixels per image use the general kernel.  default 0 */
-    CDC_OPT_KF_RING = 4,        /* input-ring slots of the one-chunk strip convs.  default 6 */
-    CDC_OPT_COUNT = 5
+    CDC_OPT_COUNT = 2
 } cdc_plan_option;
 int cdc_set_plan_option(cdc_ctx* ctx, int option, int value);
 

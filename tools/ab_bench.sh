@@ -7,11 +7,7 @@ for pass in 1 2; do
   for spec in "$@"; do
     name="${spec%%=*}"; rest="${spec#*=}"; path="${rest%%,*}"; envs=""
     [ "${rest}" != "${path}" ] && envs="${rest#*,}"
-    if [ "${path}" = "r1" ]; then
-      (cd tools/bin/r1tree && python bench.py --steps 10 --warmup 3 --no-cpu) > "gpurun_out/ab_${name}_${pass}.json" 2>/dev/null
-    else
-      env ${envs//,/ } CDC_LIB_PATH="${path}" python bench.py --steps 10 --warmup 3 --no-cpu > "gpurun_out/ab_${name}_${pass}.json" 2>/dev/null
-    fi
+    env ${envs//,/ } CDC_LIB_PATH="${path}" python bench.py --steps 10 --warmup 3 --no-cpu > "gpurun_out/ab_${name}_${pass}.json" 2>/dev/null
     python - "$name" "$pass" <<'PY'
 import json, sys
 n, p = sys.argv[1], sys.argv[2]
