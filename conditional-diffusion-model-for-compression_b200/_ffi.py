@@ -11,7 +11,8 @@ SYMBOLS = [
     "cdc_create", "cdc_destroy", "cdc_last_error", "cdc_abi_version", "cdc_act_dtype", "cdc_load_weights", "cdc_finalize_weights",
     "cdc_has_context_net", "cdc_set_schedule", "cdc_schedule_index", "cdc_schedule_coeffs", "cdc_set_sampler",
     "cdc_schedule_coeffs5", "cdc_film_size", "cdc_get_film", "cdc_bind_io", "cdc_set_cond", "cdc_get_cond", "cdc_set_latent",
-    "cdc_set_x", "cdc_get_x", "cdc_get_x0", "cdc_denoise_step", "cdc_decode", "cdc_decode_host", "cdc_launches_per_step",
+    "cdc_set_x", "cdc_get_x", "cdc_get_x0", "cdc_denoise_step", "cdc_decode", "cdc_decode_trajectory", "cdc_trajectory_wait",
+    "cdc_decode_host", "cdc_launches_per_step",
     "cdc_launches_context", "cdc_flops_per_step", "cdc_saturation_count", "cdc_quantize", "cdc_cdf_lookup",
     "cdc_has_codec", "cdc_encode_analysis", "cdc_hyper_encode", "cdc_hyper_decode",
     "cdc_rans_streams_per_channel", "cdc_rans_scratch_bytes", "cdc_rans_max_bytes", "cdc_rans_encode", "cdc_rans_decode",
@@ -94,6 +95,8 @@ def _bind(L):
     L.cdc_get_x0.argtypes = [p, f32p, p]
     L.cdc_denoise_step.argtypes = [p, i32, p]
     L.cdc_decode.argtypes = [p, p]
+    L.cdc_decode_trajectory.argtypes = [p, f32p, f32p, i32, p]
+    L.cdc_trajectory_wait.argtypes = [p, i32]
     L.cdc_decode_host.argtypes = [p, f32p, f32p, f32p, p]
     L.cdc_launches_per_step.argtypes = [p]
     L.cdc_launches_context.argtypes = [p]

@@ -323,21 +323,49 @@ cudaError_t launch_x_in(const float* x_nchw, float* xs, act_t* xpad, int B, int 
     return cudaGetLastError();
 }
 
-__global__ void x_out_kernel(const float* __restrict__ xs, float* __restrict__ x, long long n, int HW, int to_image) {
-    for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += gridDim.x * 256LL) {
-        const long long b = i / HW, p = i % HW;
+// Pixel i of xs (NHWC, 3 fp32 channels) -> its three NCHW planes: consecutive threads store consecutive pixels of a plane.
+__device__ __forceinline__ void x_out_pixel(const float* __restrict__ xs, float* __restrict__ x, long long i, int HW, int to_image) {
+    const long long b = i / HW, p = i % HW;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            float v = xs[i * 3 + c];
-            if (to_image) v = (fminf(fmaxf(v, -1.0f), 1.0f) + 1.0f) / 2.0f;
-            x[(b * 3 + c) * HW + p] = v;
-        }
+    for (int c = 0; c < 3; ++c) {
+        float v = xs[i * 3 + c];
+        if (to_image) v = (fminf(fmaxf(v, -1.0f), 1.0f) + 1.0f) / 2.0f;
+        x[(b * 3 + c) * HW + p] = v;
     }
 }
+__global__ void x_out_kernel(const float* __restrict__ xs, float* __restrict__ x, long long n, int HW, int to_image) {
+    for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += gridDim.x * 256LL) x_out_pixel(xs, x, i, HW, to_image);
+}
+static int x_out_grid(long long n) { return static_cast<int>((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096); }
 cudaError_t launch_x_out(const float* xs, float* x_nchw, int B, int HW, int to_image, cudaStream_t s) {
     const long long n = static_cast<long long>(B) * HW;
-    x_out_kernel<<<static_cast<int>((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096), 256, 0, s>>>(xs, x_nchw, n, HW,
-                                                                                                  to_image);
+    x_out_kernel<<<x_out_grid(n), 256, 0, s>>>(xs, x_nchw, n, HW, to_image);
+    return cudaGetLastError();
+}
+
+// Trajectory store: the slot pointers are read from `dst` when the kernel runs, so a captured graph serves any buffers.
+__global__ void traj_store_kernel(const float* __restrict__ xs, const float* __restrict__ x0s, const TrajPtrs* dst,
+                                  long long slot_x, long long slot_x0, long long n, int HW) {
+    float* x = slot_x >= 0 && dst->x ? dst->x + slot_x * n * 3 : nullptr;
+    float* x0 = slot_x0 >= 0 && dst->x0 ? dst->x0 + slot_x0 * n * 3 : nullptr;
+    for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n; i += gridDim.x * 256LL) {
+        if (x) x_out_pixel(xs, x, i, HW, 0);
+        if (x0) x_out_pixel(x0s, x0, i, HW, 0);
+    }
+}
+cudaError_t launch_traj_store(const float* xs, const float* x0s, const TrajPtrs* dst, int slot_x, int slot_x0, int B, int HW,
+                              cudaStream_t s) {
+    const long long n = static_cast<long long>(B) * HW;
+    traj_store_kernel<<<x_out_grid(n), 256, 0, s>>>(xs, x0s, dst, slot_x, slot_x0, n, HW);
+    return cudaGetLastError();
+}
+
+__global__ void traj_set_ptrs_kernel(TrajPtrs* dst, float* x, float* x0) {
+    dst->x = x;
+    dst->x0 = x0;
+}
+cudaError_t launch_traj_set_ptrs(TrajPtrs* dst, float* x, float* x0, cudaStream_t s) {
+    traj_set_ptrs_kernel<<<1, 1, 0, s>>>(dst, x, x0);
     return cudaGetLastError();
 }
 

@@ -49,6 +49,17 @@ constexpr int kXpadC = 16;
 cudaError_t launch_x_in(const float* x_nchw, float* xs, act_t* xpad, int B, int HW, cudaStream_t s);
 // xs NHWC fp32 -> NCHW fp32, optionally mapped to [0,1]: (clamp(x,-1,1)+1)/2
 cudaError_t launch_x_out(const float* xs, float* x_nchw, int B, int HW, int to_image, cudaStream_t s);
+// Trajectory recording (cdc_decode_trajectory): base pointers of the caller's NCHW fp32 [slots][B][3][H][W] buffers,
+// either may be null.  They live in device memory so that one captured graph serves every call's buffers.
+struct TrajPtrs {
+    float* x;
+    float* x0;
+};
+// xs -> slot slot_x of dst->x and x0s -> slot slot_x0 of dst->x0 (as launch_x_out, to_image = 0); a negative slot skips
+cudaError_t launch_traj_store(const float* xs, const float* x0s, const TrajPtrs* dst, int slot_x, int slot_x0, int B, int HW,
+                              cudaStream_t s);
+// *dst = {x, x0} in stream order
+cudaError_t launch_traj_set_ptrs(TrajPtrs* dst, float* x, float* x0, cudaStream_t s);
 // conv weight repack: OIHW fp32 -> [O_pad][taps][I_pad] act_t with input channels >= split moved to split_pad
 cudaError_t launch_repack_weight(const float* src, act_t* dst, int O, int I, int taps, int O_pad, int I_pad,
                                  int split, int split_pad, cudaStream_t s);

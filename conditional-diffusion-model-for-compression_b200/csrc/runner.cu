@@ -670,6 +670,13 @@ struct cdc_ctx {
     int graph_K = 0;
     int graph_skip = 0;  // tools build only (cdc_debug_graph_skip): class of ops left out of the captured graph
     cudaStream_t cap_stream = nullptr;
+    // cdc_decode_trajectory: a second graph, the K-step loop plus trajectory store nodes and one event-record node per slot
+    cudaGraphExec_t traj_graph = nullptr;
+    int traj_K = 0, traj_every = 0;
+    std::vector<cudaEvent_t> traj_ev;  // [slots]: slot j of the most recent launch is written
+    int traj_issued = 0;               // slots of the most recent launch of traj_graph (0: none since it was built)
+    TrajPtrs* traj_ptrs = nullptr;     // device block the store nodes read the caller's buffers from
+    cudaEvent_t traj_done = nullptr;   // end of the most recent launch: traj_ptrs may be rewritten after it
 
     int fail(int code, const char* fmt, ...) {
         char buf[512];
@@ -1189,15 +1196,28 @@ static int build_plans(cdc_ctx* ctx) {
     return CDC_OK;
 }
 
+static void drop_traj_graph(cdc_ctx* ctx) {
+    if (ctx->traj_graph) cudaGraphExecDestroy(ctx->traj_graph);
+    for (cudaEvent_t ev : ctx->traj_ev)
+        if (ev) cudaEventDestroy(ev);
+    ctx->traj_graph = nullptr;
+    ctx->traj_ev.clear();
+    ctx->traj_K = ctx->traj_every = ctx->traj_issued = 0;
+}
+
 static void drop_graph(cdc_ctx* ctx) {
     if (ctx->graph) cudaGraphExecDestroy(ctx->graph);
     ctx->graph = nullptr;
     ctx->graph_K = 0;
+    drop_traj_graph(ctx);
 }
 
 // Captures the K-step loop into one graph.  stamps != null: the timing variant (cdc_profile_graph) -- every kernel gets
-// its own (start, end) slot [k][op][2].
-static int capture_graph(cdc_ctx* ctx, cudaGraphExec_t* out, long long* stamps) {
+// its own (start, end) slot [k][op][2].  every > 0: the trajectory variant (cdc_decode_trajectory) -- slot j records step
+// k = j * every.  The final conv's epilogue overwrites xs with x_{k+1}, so x_k is stored before step k's ops and x0_hat_k
+// after them: one store node at the top of step k takes x_k and x0_hat_{k-1}, a trailing one x0_hat_{K-1}, and the event of
+// slot j is recorded once both of its planes are stored.
+static int capture_graph(cdc_ctx* ctx, cudaGraphExec_t* out, long long* stamps, int every = 0) {
     if (!ctx->cap_stream) CK(cudaStreamCreateWithFlags(&ctx->cap_stream, cudaStreamNonBlocking));
     cudaGraph_t g = nullptr;
     CK(cudaStreamBeginCapture(ctx->cap_stream, cudaStreamCaptureModeThreadLocal));
@@ -1222,7 +1242,19 @@ static int capture_graph(cdc_ctx* ctx, cudaGraphExec_t* out, long long* stamps) 
     if (!skip.empty() && ctx->graph_skip == 0) ctx->graph_skip = 4;
 #endif
     const size_t nops = ctx->step_seq.ops.size();
-    for (int k = 0; k < ctx->K && e == cudaSuccess; ++k)
+    auto store = [&](int k) {  // trajectory variant, top of step k (k == K: after the last step)
+        const int sx = k < ctx->K && k % every == 0 ? k / every : -1;
+        const int sx0 = k > 0 && (k - 1) % every == 0 ? (k - 1) / every : -1;
+        if (sx < 0 && sx0 < 0) return;
+        e = launch_traj_store(ctx->xs, ctx->x0s, ctx->traj_ptrs, sx, sx0, ctx->B, ctx->H * ctx->W, ctx->cap_stream);
+        if (e == cudaSuccess && sx0 >= 0) e = cudaEventRecordWithFlags(ctx->traj_ev[sx0], ctx->cap_stream, cudaEventRecordExternal);
+        if (e != cudaSuccess) bad = "trajectory store";
+    };
+    for (int k = 0; k < ctx->K && e == cudaSuccess; ++k) {
+        if (every > 0) {
+            store(k);
+            if (e != cudaSuccess) break;
+        }
         for (size_t i = 0; i < nops; ++i) {
             Op& op = ctx->step_seq.ops[i];
 #ifdef CDC_TOOLS
@@ -1239,6 +1271,8 @@ static int capture_graph(cdc_ctx* ctx, cudaGraphExec_t* out, long long* stamps) 
                 break;
             }
         }
+    }
+    if (every > 0 && e == cudaSuccess) store(ctx->K);
     cudaError_t e2 = cudaStreamEndCapture(ctx->cap_stream, &g);
     if (e != cudaSuccess) {
         if (g) cudaGraphDestroy(g);
@@ -1257,6 +1291,22 @@ static int ensure_graph(cdc_ctx* ctx) {
     int r = capture_graph(ctx, &ctx->graph, nullptr);
     if (r) return r;
     ctx->graph_K = ctx->K;
+    return CDC_OK;
+}
+
+static int ensure_traj_graph(cdc_ctx* ctx, int every) {
+    if (ctx->traj_graph && ctx->traj_K == ctx->K && ctx->traj_every == every) return CDC_OK;
+    if (ctx->traj_graph) CK(cudaEventSynchronize(ctx->traj_done));  // its last launch may still be running
+    drop_traj_graph(ctx);
+    ctx->traj_ev.assign((ctx->K + every - 1) / every, nullptr);
+    for (cudaEvent_t& ev : ctx->traj_ev) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    int r = capture_graph(ctx, &ctx->traj_graph, nullptr, every);
+    if (r) {
+        drop_traj_graph(ctx);
+        return r;
+    }
+    ctx->traj_K = ctx->K;
+    ctx->traj_every = every;
     return CDC_OK;
 }
 
@@ -1332,6 +1382,8 @@ void cdc_destroy(cdc_ctx* ctx) {
         if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
         if (ctx->ev_x) cudaEventDestroy(ctx->ev_x);
         if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
+        if (ctx->traj_ptrs) cudaFree(ctx->traj_ptrs);
+        if (ctx->traj_done) cudaEventDestroy(ctx->traj_done);
     }
     delete ctx;
 }
@@ -1714,6 +1766,45 @@ int cdc_decode(cdc_ctx* ctx, cdc_stream s) {
     int r = ensure_graph(ctx);
     if (r) return r;
     CK(cudaGraphLaunch(ctx->graph, S(s)));
+    return CDC_OK;
+}
+
+int cdc_decode_trajectory(cdc_ctx* ctx, float* x_traj, float* x0_traj, int every, cdc_stream s) {
+    NEED_PLAN();
+    if (ctx->K < 1) return ctx->fail(CDC_ERR_STATE, "call cdc_set_schedule first");
+    if (every < 1) return ctx->fail(CDC_ERR_SHAPE, "cdc_decode_trajectory: every must be >= 1, got %d", every);
+    if (!x_traj && !x0_traj) return ctx->fail(CDC_ERR_SHAPE, "cdc_decode_trajectory: both trajectory buffers are null");
+    if (ctx->graph_skip) return ctx->fail(CDC_ERR_STATE, "ops are being left out of the graph (tools build, graph skip): x is garbage");
+    if (!ctx->traj_ptrs) {  // both or neither
+        TrajPtrs* p = nullptr;
+        cudaEvent_t ev = nullptr;
+        CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        const cudaError_t e = cudaMalloc(&p, sizeof(TrajPtrs));
+        if (e != cudaSuccess) {
+            cudaEventDestroy(ev);
+            return ctx->fail(CDC_ERR_CUDA, "cudaMalloc(trajectory pointer block): %s", cudaGetErrorString(e));
+        }
+        ctx->traj_ptrs = p;
+        ctx->traj_done = ev;
+    }
+    int r = ensure_traj_graph(ctx, every);
+    if (r) return r;
+    // the previous launch (possibly on another stream) reads traj_ptrs until its last store node
+    CK(cudaStreamWaitEvent(S(s), ctx->traj_done, 0));
+    CK(launch_traj_set_ptrs(ctx->traj_ptrs, x_traj, x0_traj, S(s)));
+    CK(cudaGraphLaunch(ctx->traj_graph, S(s)));
+    CK(cudaEventRecord(ctx->traj_done, S(s)));
+    ctx->traj_issued = static_cast<int>(ctx->traj_ev.size());
+    return CDC_OK;
+}
+
+int cdc_trajectory_wait(cdc_ctx* ctx, int j) {
+    if (!ctx) return CDC_ERR_STATE;
+    if (!ctx->traj_issued) return ctx->fail(CDC_ERR_STATE, "cdc_trajectory_wait: no cdc_decode_trajectory since the last bind / schedule change");
+    if (j < 0 || j >= ctx->traj_issued)
+        return ctx->fail(CDC_ERR_SHAPE, "cdc_trajectory_wait: slot %d outside the %d slots of the last trajectory decode", j, ctx->traj_issued);
+    GUARD();
+    CK(cudaEventSynchronize(ctx->traj_ev[j]));
     return CDC_OK;
 }
 

@@ -3,7 +3,8 @@
 Same surface as oracle/sampler.py OracleDecoder (the reference ships no code, so the oracle
 *is* the reference interface for this path; SURVEY.md section 8b):
     set_sample_schedule(steps), predict_x0(x_t, t, cond), denoise_step(x_t, t, cond),
-    decode(latent, steps, *, init=None, gamma=0.8, seed=0), quantize_symbols, cdf_lookup.
+    decode(latent, steps, *, init=None, gamma=0.8, seed=0, trajectory=None), quantize_symbols, cdf_lookup;
+plus decode_progressive, a generator of per-step (x_t, x0_hat) previews while the decode runs.
 Tensors at this surface are NCHW fp32 torch tensors; CUDA tensors are used in place, CPU tensors
 are staged through pinned memory by the library (cdc_decode_host).
 """
@@ -58,9 +59,19 @@ class Decoder:
         self.steps = 0
         self.sampler = (0.0, "x", 0)
         self.shape = None
+        self._side = None  # decode_progressive's stream
+        self._side_busy = False  # a decode_progressive generator has not ended: its graph may still run on _side
 
     def _ck(self, rc, what):
         _ffi.check(self.ctx, rc, what, self.L)
+
+    def _stream(self):
+        """The stream handle every call of this decoder enqueues on: the current stream, made to wait for the graph of
+        an unfinished decode_progressive first (it reads and writes the same workspace)."""
+        cur = torch.cuda.current_stream()
+        if self._side_busy and cur != self._side:
+            cur.wait_stream(self._side)
+        return C.c_void_p(cur.cuda_stream)
 
     def __del__(self):
         try:
@@ -101,7 +112,7 @@ class Decoder:
         n = self.L.cdc_film_size(self.ctx)
         out = torch.empty(self.steps, n, device=self.device, dtype=torch.float32)
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_get_film(self.ctx, C.c_void_p(out.data_ptr()), _stream_ptr()), "cdc_get_film")
+            self._ck(self.L.cdc_get_film(self.ctx, C.c_void_p(out.data_ptr()), self._stream()), "cdc_get_film")
         return out
 
     def _k_of(self, t):
@@ -137,7 +148,7 @@ class Decoder:
         with torch.cuda.device(self.device):
             c = [_f32c(t, self.device) for t in cond]
             self.bind(B, H, W)
-            self._ck(self.L.cdc_set_cond(self.ctx, *[C.c_void_p(t.data_ptr()) for t in c], _stream_ptr()), "cdc_set_cond")
+            self._ck(self.L.cdc_set_cond(self.ctx, *[C.c_void_p(t.data_ptr()) for t in c], self._stream()), "cdc_set_cond")
 
     def set_latent(self, latent):
         if latent.dim() != 4 or latent.shape[1] != self.cfg.latent_ch:
@@ -146,7 +157,7 @@ class Decoder:
         with torch.cuda.device(self.device):
             y = _f32c(latent, self.device)
             self.bind(B, h * 16, w * 16)
-            self._ck(self.L.cdc_set_latent(self.ctx, C.c_void_p(y.data_ptr()), _stream_ptr()), "cdc_set_latent")
+            self._ck(self.L.cdc_set_latent(self.ctx, C.c_void_p(y.data_ptr()), self._stream()), "cdc_set_latent")
 
     def get_cond(self):
         """The bound context maps (c0, c1, c2, c3) as NCHW fp32 tensors: what set_latent's context net produced
@@ -155,7 +166,7 @@ class Decoder:
             raise RuntimeError("nothing bound: call set_latent / set_cond first")
         outs = [torch.empty(s, device=self.device, dtype=torch.float32) for s in self.cond_shapes(*self.shape)]
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_get_cond(self.ctx, *[C.c_void_p(t.data_ptr()) for t in outs], _stream_ptr()), "cdc_get_cond")
+            self._ck(self.L.cdc_get_cond(self.ctx, *[C.c_void_p(t.data_ptr()) for t in outs], self._stream()), "cdc_get_cond")
         return tuple(outs)
 
     def _set_x(self, x):
@@ -166,20 +177,20 @@ class Decoder:
             raise ValueError(f"x has shape {tuple(x.shape)}, expected {(B, 3, H, W)} (the bound batch / image size)")
         with torch.cuda.device(self.device):
             xd = _f32c(x, self.device)
-            self._ck(self.L.cdc_set_x(self.ctx, C.c_void_p(xd.data_ptr()), _stream_ptr()), "cdc_set_x")
+            self._ck(self.L.cdc_set_x(self.ctx, C.c_void_p(xd.data_ptr()), self._stream()), "cdc_set_x")
 
     def _get_x(self, to_image=False):
         B, H, W = self.shape
         out = torch.empty(B, 3, H, W, device=self.device, dtype=torch.float32)
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_get_x(self.ctx, C.c_void_p(out.data_ptr()), 1 if to_image else 0, _stream_ptr()), "cdc_get_x")
+            self._ck(self.L.cdc_get_x(self.ctx, C.c_void_p(out.data_ptr()), 1 if to_image else 0, self._stream()), "cdc_get_x")
         return out
 
     def _get_x0(self):
         B, H, W = self.shape
         out = torch.empty(B, 3, H, W, device=self.device, dtype=torch.float32)
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_get_x0(self.ctx, C.c_void_p(out.data_ptr()), _stream_ptr()), "cdc_get_x0")
+            self._ck(self.L.cdc_get_x0(self.ctx, C.c_void_p(out.data_ptr()), self._stream()), "cdc_get_x0")
         return out
 
     # ---- the hot path --------------------------------------------------------------------------
@@ -191,7 +202,7 @@ class Decoder:
             if cond is not None:
                 self.set_cond(cond)
             self._set_x(x_t)
-            self._ck(self.L.cdc_denoise_step(self.ctx, k, _stream_ptr()), "cdc_denoise_step")
+            self._ck(self.L.cdc_denoise_step(self.ctx, k, self._stream()), "cdc_denoise_step")
             return self._get_x()
 
     @torch.no_grad()
@@ -199,11 +210,8 @@ class Decoder:
         self.denoise_step(x_t, t, cond)
         return self._get_x0()
 
-    @torch.no_grad()
-    def decode(self, latent, steps, *, init=None, gamma=0.8, seed=0, cond=None, out=None):
-        """latent y_hat fp32 [B,256,H/16,W/16] -> image fp32 [B,3,H,W] in [0,1] (K steps = one graph launch).
-        Host tensors take the cdc_decode_host path (H2D + decode + D2H inside the library); page-locked inputs and a
-        page-locked `out` (optional, host path only: fp32 [B,3,H,W], returned) are copied from / to directly."""
+    def _decode_inputs(self, latent, steps, init, gamma, seed):
+        """Schedule, shape checks and the default x_T shared by decode and decode_progressive."""
         if steps != self.steps:
             self.set_sample_schedule(steps, *self.sampler)
         if latent.dim() != 4 or latent.shape[1] != self.cfg.latent_ch:
@@ -215,31 +223,130 @@ class Decoder:
             init = gamma * torch.randn(B, 3, H, W, generator=g)
         elif tuple(init.shape) != (B, 3, H, W):
             raise ValueError(f"init has shape {tuple(init.shape)}, expected {(B, 3, H, W)}")
+        return init, (B, H, W)
+
+    @staticmethod
+    def _check_host_out(out, B, H, W):
+        if out is None:
+            return torch.empty(B, 3, H, W, dtype=torch.float32)
+        if out.shape != (B, 3, H, W) or out.dtype != torch.float32 or out.is_cuda or not out.is_contiguous():
+            raise ValueError("out must be a contiguous fp32 host tensor of shape [B,3,H,W]")
+        return out
+
+    @torch.no_grad()
+    def decode(self, latent, steps, *, init=None, gamma=0.8, seed=0, cond=None, out=None, trajectory=None, x0_trajectory=None):
+        """latent y_hat fp32 [B,256,H/16,W/16] -> image fp32 [B,3,H,W] in [0,1] (K steps = one graph launch).
+        Host tensors take the cdc_decode_host path (H2D + decode + D2H inside the library); page-locked inputs and a
+        page-locked `out` (optional, host path only: fp32 [B,3,H,W], returned) are copied from / to directly.
+        trajectory / x0_trajectory (lists, as oracle/sampler.py OracleDecoder.decode(trajectory=...)): K device tensors
+        [B,3,H,W] are appended to each given list, x_t entering step k and the raw x0_hat of step k (views of one
+        allocation, recorded inside the graph by cdc_decode_trajectory).  The image is the same bits either way."""
+        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed)
+        record = trajectory is not None or x0_trajectory is not None
+        host = cond is None and not latent.is_cuda and not init.is_cuda
         with torch.cuda.device(self.device):
             self.bind(B, H, W)
-            if cond is None and not latent.is_cuda and not init.is_cuda:
+            if host and not record:
                 # host buffers: pinned staging + H2D/D2H inside the library
                 lat = latent.float().contiguous()
                 x0 = init.float().contiguous()
-                if out is None:
-                    out = torch.empty(B, 3, H, W, dtype=torch.float32)
-                elif out.shape != (B, 3, H, W) or out.dtype != torch.float32 or out.is_cuda or not out.is_contiguous():
-                    raise ValueError("out must be a contiguous fp32 host tensor of shape [B,3,H,W]")
+                out = self._check_host_out(out, B, H, W)
                 self._ck(self.L.cdc_decode_host(self.ctx, C.c_void_p(lat.data_ptr()), C.c_void_p(x0.data_ptr()),
-                                                C.c_void_p(out.data_ptr()), _stream_ptr()), "cdc_decode_host")
+                                                C.c_void_p(out.data_ptr()), self._stream()), "cdc_decode_host")
                 return out
+            if host:
+                out = self._check_host_out(out, B, H, W)
             if cond is not None:
                 self.set_cond(cond)
             else:
                 self.set_latent(latent)
             self._set_x(init)
-            self._ck(self.L.cdc_decode(self.ctx, _stream_ptr()), "cdc_decode")
-            return self._get_x(to_image=True)
+            if not record:
+                self._ck(self.L.cdc_decode(self.ctx, self._stream()), "cdc_decode")
+                return self._get_x(to_image=True)
+            xt, x0 = self._traj_buffers(trajectory is not None, x0_trajectory is not None, 1)
+            self.decode_trajectory(xt, x0)
+            for lst, buf in ((trajectory, xt), (x0_trajectory, x0)):
+                if lst is not None:
+                    lst.extend(buf.unbind(0))
+            img = self._get_x(to_image=True)
+            return out.copy_(img) if host else img
 
     def decode_resident(self):
         """Replay the K-step graph on whatever x / cond are bound (used by bench.py's device-timed leg)."""
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_decode(self.ctx, _stream_ptr()), "cdc_decode")
+            self._ck(self.L.cdc_decode(self.ctx, self._stream()), "cdc_decode")
+
+    def trajectory_slots(self, every=1):
+        """Slots a trajectory decode with this `every` records: ceil(K / every), slot j = step j * every."""
+        return (self.steps + every - 1) // every
+
+    def _traj_buffers(self, want_x, want_x0, every):
+        B, H, W = self.shape
+        n = self.trajectory_slots(every)
+        buf = torch.empty((int(want_x) + int(want_x0)) * n, B, 3, H, W, device=self.device, dtype=torch.float32)
+        xt = buf[:n] if want_x else None
+        x0 = buf[n * int(want_x):] if want_x0 else None
+        return xt, x0
+
+    def decode_trajectory(self, x_traj=None, x0_traj=None, every=1):
+        """Replay the K-step loop on whatever x / cond are bound (like decode_resident) and record slot j = step
+        j * every into x_traj[j] (x_t entering the step) and x0_traj[j] (its raw x0_hat): contiguous fp32 device
+        tensors [ceil(K / every), B, 3, H, W], either may be None.  Enqueued on the current stream; the image is then
+        what decode_resident leaves (include/cdc_b200.h cdc_decode_trajectory)."""
+        if self.shape is None or not self.steps:
+            raise RuntimeError("bind a shape (set_latent / set_cond) and set a schedule first")
+        if int(every) < 1:
+            raise ValueError(f"every must be >= 1, got {every}")
+        if x_traj is None and x0_traj is None:
+            raise ValueError("give x_traj, x0_traj or both")
+        want = (self.trajectory_slots(int(every)), *self.shape[:1], 3, *self.shape[1:])
+        for name, t in (("x_traj", x_traj), ("x0_traj", x0_traj)):
+            if t is not None and (tuple(t.shape) != want or t.dtype != torch.float32 or t.device != self.device
+                                  or not t.is_contiguous()):
+                raise ValueError(f"{name} must be a contiguous fp32 tensor {want} on {self.device}, got "
+                                 f"{tuple(t.shape)} {t.dtype} on {t.device}")
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)
+        with torch.cuda.device(self.device):
+            self._ck(self.L.cdc_decode_trajectory(self.ctx, ptr(x_traj), ptr(x0_traj), int(every), self._stream()),
+                     "cdc_decode_trajectory")
+
+    @torch.no_grad()
+    def decode_progressive(self, latent, steps, *, every=1, init=None, gamma=0.8, seed=0, cond=None):
+        """Generator: decode as `decode` does and yield (k, x_t, x0_hat) for k = 0, every, 2 * every, ... as soon as
+        the graph has written step k: x_t [B,3,H,W] entering step k and the network's raw x0_hat of that step, device
+        fp32.  (x0_hat.clamp(-1, 1) + 1) / 2 is the preview image.  The graph runs on a stream of its own, so the
+        caller's stream can copy or display a slot while later steps run; stepping the last x_t once more gives decode()'s
+        image.  The buffers live until the graph has passed them, so stopping early is safe.  While the generator is
+        suspended, any call of this decoder first makes the current stream wait for the graph; once it ends (exhausted
+        or closed), the caller's stream waits for the graph."""
+        if int(every) < 1:
+            raise ValueError(f"every must be >= 1, got {every}")
+        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed)
+        with torch.cuda.device(self.device):
+            self.bind(B, H, W)
+            if cond is not None:
+                self.set_cond(cond)
+            else:
+                self.set_latent(latent)
+            self._set_x(init)
+            xt, x0 = self._traj_buffers(True, True, every)
+            cur = torch.cuda.current_stream()
+            if self._side is None:
+                self._side = torch.cuda.Stream(device=self.device)
+            side = self._side
+            side.wait_stream(cur)
+            with torch.cuda.stream(side):
+                self.decode_trajectory(xt, x0, every)
+            xt.record_stream(side)  # (one allocation: the caching allocator keeps it until the graph has passed)
+            self._side_busy = True
+        try:
+            for j in range(xt.shape[0]):
+                self._ck(self.L.cdc_trajectory_wait(self.ctx, j), "cdc_trajectory_wait")
+                yield j * every, xt[j], x0[j]
+        finally:
+            cur.wait_stream(side)
+            self._side_busy = False
 
     # ---- introspection -------------------------------------------------------------------------
     def launches_per_step(self):
@@ -252,7 +359,7 @@ class Decoder:
         """Epilogue passes that stored a value saturated to the fp16 range since creation / the last reset (0 = none)."""
         n = C.c_uint64(0)
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_saturation_count(self.ctx, C.byref(n), 1 if reset else 0, _stream_ptr()), "cdc_saturation_count")
+            self._ck(self.L.cdc_saturation_count(self.ctx, C.byref(n), 1 if reset else 0, self._stream()), "cdc_saturation_count")
         return int(n.value)
 
     def step_ops(self):
@@ -268,14 +375,14 @@ class Decoder:
 
     def run_step_op(self, i, k=0):
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_run_step_op(self.ctx, i, k, _stream_ptr()), "cdc_run_step_op")
+            self._ck(self.L.cdc_run_step_op(self.ctx, i, k, self._stream()), "cdc_run_step_op")
 
     def profile_step(self, k=0, warm=1):
         """In-stream device time (us) of every op of step k (launched back to back, CUDA events in the library)."""
         n = self.L.cdc_num_step_ops(self.ctx)
         buf = (C.c_float * n)()
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_profile_step(self.ctx, k, warm, buf, _stream_ptr()), "cdc_profile_step")
+            self._ck(self.L.cdc_profile_step(self.ctx, k, warm, buf, self._stream()), "cdc_profile_step")
         return list(buf)
 
     def profile_graph(self, reps=5):
@@ -285,7 +392,7 @@ class Decoder:
         st = (C.c_float * (n * self.steps))()
         du = (C.c_float * (n * self.steps))()
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_profile_graph(self.ctx, reps, st, du, _stream_ptr()), "cdc_profile_graph")
+            self._ck(self.L.cdc_profile_graph(self.ctx, reps, st, du, self._stream()), "cdc_profile_graph")
         rs = [[st[k * n + i] for i in range(n)] for k in range(self.steps)]
         rd = [[du[k * n + i] for i in range(n)] for k in range(self.steps)]
         return rs, rd

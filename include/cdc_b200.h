@@ -107,6 +107,16 @@ int cdc_hyper_decode(cdc_ctx* ctx, const float* z_hat, float* mu, float* sigma, 
 /* ---- oracle/sampler.py OracleDecoder.denoise_step / decode ------------------------------------ */
 int cdc_denoise_step(cdc_ctx* ctx, int k, cdc_stream s); /* x <- c0_k*clamp(unet(x, idx_k, cond)) + c1_k*x */
 int cdc_decode(cdc_ctx* ctx, cdc_stream s);              /* all K steps: ONE cudaGraphLaunch */
+/* All K steps like cdc_decode, also recording the trajectory (oracle/sampler.py OracleDecoder.decode(trajectory=...)).
+ * Slot j records step k = j * every, for j < ceil(K / every).
+ * x_traj[j]  = x_t entering step k (x_traj[0] = x_T).
+ * x0_traj[j] = raw x0_hat of step k, as cdc_get_x0 gives it.
+ * Both are NCHW fp32 [slots][B][3][H][W] device buffers. Either may be NULL, but not both.
+ * The final state (cdc_get_x / cdc_get_x0) is bit-identical to cdc_decode's.  A second graph, captured on the first call
+ * for the current (K, every) and dropped with cdc_decode's; the buffer pointers are not baked into it. */
+int cdc_decode_trajectory(cdc_ctx* ctx, float* x_traj, float* x0_traj, int every, cdc_stream s);
+/* Blocks the host until slot j of the most recent cdc_decode_trajectory has been written. */
+int cdc_trajectory_wait(cdc_ctx* ctx, int j);
 /* host-buffer convenience used for end-to-end timing: H2D(latent, x_T) -> context net -> decode ->
  * D2H(image in [0,1]); synchronises the stream before returning. */
 int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host, float* image_host, cdc_stream s);
