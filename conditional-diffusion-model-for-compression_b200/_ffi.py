@@ -12,7 +12,7 @@ SYMBOLS = [
     "cdc_has_context_net", "cdc_set_schedule", "cdc_schedule_index", "cdc_schedule_coeffs", "cdc_set_sampler",
     "cdc_schedule_coeffs5", "cdc_film_size", "cdc_get_film", "cdc_bind_io", "cdc_set_cond", "cdc_get_cond", "cdc_set_latent",
     "cdc_set_x", "cdc_get_x", "cdc_get_x0", "cdc_denoise_step", "cdc_decode", "cdc_decode_trajectory", "cdc_trajectory_wait",
-    "cdc_decode_host", "cdc_launches_per_step",
+    "cdc_decode_host", "cdc_set_image_seeds", "cdc_init_noise", "cdc_decode_host_seeded", "cdc_launches_per_step",
     "cdc_launches_context", "cdc_flops_per_step", "cdc_saturation_count", "cdc_quantize", "cdc_cdf_lookup",
     "cdc_has_codec", "cdc_encode_analysis", "cdc_hyper_encode", "cdc_hyper_decode",
     "cdc_rans_streams_per_channel", "cdc_rans_scratch_bytes", "cdc_rans_max_bytes", "cdc_rans_encode", "cdc_rans_decode",
@@ -98,6 +98,9 @@ def _bind(L):
     L.cdc_decode_trajectory.argtypes = [p, f32p, f32p, i32, p]
     L.cdc_trajectory_wait.argtypes = [p, i32]
     L.cdc_decode_host.argtypes = [p, f32p, f32p, f32p, p]
+    L.cdc_set_image_seeds.argtypes = [p, C.POINTER(C.c_uint64), i32, p]
+    L.cdc_init_noise.argtypes = [p, C.c_float, p]
+    L.cdc_decode_host_seeded.argtypes = [p, f32p, C.c_float, f32p, p]
     L.cdc_launches_per_step.argtypes = [p]
     L.cdc_launches_context.argtypes = [p]
     L.cdc_flops_per_step.argtypes = [p]

@@ -422,7 +422,8 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
         if constexpr (EPI == EPI_DDIM) {
             // 3 real output channels: thread = pixel.  The two warp groups (half 0 / 1) take alternate output rows.
             const float b0 = bias_s[0], b1 = bias_s[1], b2 = bias_s[2];
-            const SamplerCoef sc{p.c0, p.c1, p.e0, p.e1, p.sg, p.seed, p.step};
+            const SamplerCoef sc{p.c0, p.c1, p.e0, p.e1, p.sg, p.seed, p.step, p.img_seeds,
+                                 static_cast<unsigned int>(p.H * p.W)};
             const uint32_t tq = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
             if (half == 0) {
                 // arm every accumulator: zero them all, ONE wait, then the first "drained" arrives

@@ -39,6 +39,7 @@ struct alignas(64) KfParams {
     float e0, e1, sg;     // generalised sampler update (see ConvParams)
     unsigned long long seed;
     int step;
+    const unsigned long long* img_seeds;  // (see ConvParams)
     long long* stamp;     // diagnostics, may be null (see ConvParams)
     unsigned int* sat;
 };

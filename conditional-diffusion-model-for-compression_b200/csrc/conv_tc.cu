@@ -173,7 +173,9 @@ __global__ void __launch_bounds__(kConvThreads, 1) conv_tc_kernel(const __grid_c
         const int half = (warp - 4) >> 2;  // column half of the accumulator
         const int row = q * 32 + lane;
         const int ty = row >> BWl, tx = row & (BW - 1);
-        const EpiArgs ea{p.out, p.residual, p.ldc, p.x, p.xpad, p.x0_out, SamplerCoef{p.c0, p.c1, p.e0, p.e1, p.sg, p.seed, p.step}, p.sat, p.act_slope};
+        const EpiArgs ea{p.out, p.residual, p.ldc, p.x, p.xpad, p.x0_out,
+                         SamplerCoef{p.c0, p.c1, p.e0, p.e1, p.sg, p.seed, p.step, p.img_seeds, static_cast<unsigned int>(p.OH * p.OW)},
+                         p.sat, p.act_slope};
         uint32_t it = 0;
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
             int nt, ph, b, th, tw;

@@ -59,6 +59,7 @@ struct alignas(64) ConvParams {
     float e0, e1, sg;
     unsigned long long seed;
     int step;
+    const unsigned long long* img_seeds;  // per-image seed block (kernels.cuh ImageSeeds), or null: read only when sg != 0
     // diagnostics (either may be null): [0] = earliest CTA start, [1] = latest CTA end (globaltimer ns, atomic min / max);
     // number of (thread, tile) epilogue passes that met a value beyond the fp16 range (stored saturated)
     long long* stamp;

@@ -5,6 +5,7 @@
 #include "gn_sums.cuh"
 #include "kernels.cuh"
 #include "ptx.cuh"
+#include "sampler.cuh"
 
 namespace cdc {
 
@@ -320,6 +321,43 @@ __global__ void x_in_kernel(const float* __restrict__ x, float* __restrict__ xs,
 cudaError_t launch_x_in(const float* x_nchw, float* xs, act_t* xpad, int B, int HW, cudaStream_t s) {
     const long long n = static_cast<long long>(B) * HW;
     x_in_kernel<<<static_cast<int>((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096), 256, 0, s>>>(x_nchw, xs, xpad, n, HW);
+    return cudaGetLastError();
+}
+
+// x_T = gamma * z of every image from its own seed (sampler.cuh, counter (pixel within the image, 0, 1)), written where
+// launch_x_in would put it: xs through shared memory as whole float4s, xpad as one 32-byte sector per pixel (channels
+// 3..15 zero, as the DDIM epilogue stores them).
+constexpr int kInitPix = 256;
+__global__ void __launch_bounds__(kInitPix) init_noise_kernel(const unsigned long long* __restrict__ seeds, float* __restrict__ xs,
+                                                              act_t* __restrict__ xpad, float gamma, long long n, int HW) {
+    __shared__ __align__(16) float tile[kInitPix * 3];
+    for (long long i0 = static_cast<long long>(blockIdx.x) * kInitPix; i0 < n; i0 += static_cast<long long>(gridDim.x) * kInitPix) {
+        const long long i = i0 + threadIdx.x;
+        if (i < n) {
+            const long long b = i / HW;
+            float z[3];
+            philox_normal3(seeds[1 + b], static_cast<unsigned long long>(i - b * HW), 0u, 1u, z);
+            const float v0 = gamma * z[0], v1 = gamma * z[1], v2 = gamma * z[2];
+            tile[threadIdx.x * 3 + 0] = v0;
+            tile[threadIdx.x * 3 + 1] = v1;
+            tile[threadIdx.x * 3 + 2] = v2;
+            st_global_v8(xpad + i * kXpadC, make_uint4(pack_act2(v0, v1), pack_act2(v2, 0.0f), 0u, 0u), make_uint4(0u, 0u, 0u, 0u));
+        }
+        __syncthreads();
+        const long long m = (n - i0 < kInitPix ? n - i0 : kInitPix) * 3;  // floats of this chunk
+        if (m == kInitPix * 3) {
+            if (threadIdx.x < kInitPix * 3 / 4)
+                reinterpret_cast<float4*>(xs + i0 * 3)[threadIdx.x] = reinterpret_cast<const float4*>(tile)[threadIdx.x];
+        } else {
+            for (int j = threadIdx.x; j < m; j += kInitPix) xs[i0 * 3 + j] = tile[j];
+        }
+        __syncthreads();
+    }
+}
+cudaError_t launch_init_noise(const unsigned long long* seeds, float* xs, act_t* xpad, float gamma, int B, int HW, cudaStream_t s) {
+    const long long n = static_cast<long long>(B) * HW;
+    const long long blocks = (n + kInitPix - 1) / kInitPix;
+    init_noise_kernel<<<static_cast<int>(blocks < 8192 ? blocks : 8192), kInitPix, 0, s>>>(seeds, xs, xpad, gamma, n, HW);
     return cudaGetLastError();
 }
 

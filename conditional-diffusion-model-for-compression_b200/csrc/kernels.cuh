@@ -47,6 +47,10 @@ cudaError_t launch_nhwc_act_to_nchw_f32(const act_t* src, float* dst, int B, int
 constexpr int kXpadC = 16;
 // x NCHW fp32 [B,3,H,W] -> xs NHWC fp32 [B*HW][3] and xpad act_t [B*HW][kXpadC] (channels 0..2; rest untouched)
 cudaError_t launch_x_in(const float* x_nchw, float* xs, act_t* xpad, int B, int HW, cudaStream_t s);
+// Per-image seed block of the sampler state (cdc_set_image_seeds): unsigned long long [1 + B], word 0 = 1 while per-image
+// mode is on, words 1 .. B = the seed of image b.  The conv epilogue reads it only when the step adds noise (sg != 0).
+// init_noise: x_T = gamma * z from the seeds (sampler.cuh, x_T plane) -> xs and xpad, as launch_x_in stores them
+cudaError_t launch_init_noise(const unsigned long long* seeds, float* xs, act_t* xpad, float gamma, int B, int HW, cudaStream_t s);
 // xs NHWC fp32 -> NCHW fp32, optionally mapped to [0,1]: (clamp(x,-1,1)+1)/2
 cudaError_t launch_x_out(const float* xs, float* x_nchw, int B, int HW, int to_image, cudaStream_t s);
 // Trajectory recording (cdc_decode_trajectory): base pointers of the caller's NCHW fp32 [slots][B][3][H][W] buffers,

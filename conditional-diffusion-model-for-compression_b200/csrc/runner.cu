@@ -149,6 +149,7 @@ struct ConvBuild {
     act_t* xpad = nullptr;
     float* x0_out = nullptr;
     const SamplerTab* samp = nullptr;  // per-step sampler coefficients (host)
+    const unsigned long long* img_seeds = nullptr;  // per-image seed block (kernels.cuh), or null
     unsigned int* sat = nullptr;       // saturation diagnostics counter (device)
     // offered: fused 1x1 residual conv of the same input (kf path only; op->desc.res1 says whether it was taken)
     const ConvW* res_w = nullptr;
@@ -363,6 +364,7 @@ static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, in
     kp->x = cb.x;
     kp->xpad = cb.xpad;
     kp->x0_out = cb.x0_out;
+    kp->img_seeds = cb.img_seeds;
     kp->sat = cb.sat;
     kp->e1 = 1.0f;
     if (kg.apply) op->name += "+gn_in";  // the GroupNorm apply pass no longer touches HBM; its arithmetic rides along
@@ -527,6 +529,7 @@ static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, int gw,
     cp->x = cb.x;
     cp->xpad = cb.xpad;
     cp->x0_out = cb.x0_out;
+    cp->img_seeds = cb.img_seeds;
     cp->sat = cb.sat;
     cp->e1 = 1.0f;
     cp->act_slope = cb.act_slope;
@@ -658,6 +661,11 @@ struct cdc_ctx {
     Act img64, enc_y, henc_in, henc_z, hdec_in, hdec_out;
     Act cond[4], xpad, latent;
     float *xs = nullptr, *x0s = nullptr;
+    // cdc_set_image_seeds: the seed block the final conv's epilogue and init_noise read ([1 + B], kernels.cuh), whether
+    // per-image mode is on, and the end of the most recent launch that reads the block (it may be rewritten after it)
+    unsigned long long* img_seeds = nullptr;
+    bool seeded = false;
+    cudaEvent_t seeds_done = nullptr;
     gn_sum_t* gn_slots = nullptr;  // [3][kMaxGnSlots][B][32][kGnVals] fixed-point GroupNorm accumulators (gn_sums.cuh)
     unsigned int* sat_dev = nullptr;  // saturation diagnostics counter (cdc_saturation_count)
     float *stage_f32 = nullptr;  // NCHW fp32 staging for host-buffer calls
@@ -968,6 +976,9 @@ static int build_plans(cdc_ctx* ctx) {
     const size_t px = static_cast<size_t>(B) * H * W;
     CK(ar.alloc(reinterpret_cast<void**>(&ctx->xs), px * 3 * 4));
     CK(ar.alloc(reinterpret_cast<void**>(&ctx->x0s), px * 3 * 4));
+    CK(ar.alloc(reinterpret_cast<void**>(&ctx->img_seeds), (static_cast<size_t>(B) + 1) * 8));
+    CK(cudaMemset(ctx->img_seeds, 0, (static_cast<size_t>(B) + 1) * 8));  // per-image mode off
+    ctx->seeded = false;
     CK(ar.alloc(reinterpret_cast<void**>(&ctx->gn_slots), 3 * static_cast<size_t>(kMaxGnSlots) * B * kGnImgStride * sizeof(gn_sum_t)));
     Seq* gn_seqs[3] = {&ctx->step_seq, &ctx->ctx_seq, &ctx->enc_seq};  // the sequences with GroupNorms
     for (int i = 0; i < 3; ++i) gn_seqs[i]->slots = ctx->gn_slots + static_cast<size_t>(i) * kMaxGnSlots * B * kGnImgStride;
@@ -1102,6 +1113,7 @@ static int build_plans(cdc_ctx* ctx) {
         cb.xpad = ctx->xpad.p;
         cb.x0_out = ctx->x0s;
         cb.samp = &ctx->samp;
+        cb.img_seeds = ctx->img_seeds;
         pb.conv(cb);
     }
     if (pb.rc) return pb.rc;
@@ -1310,6 +1322,13 @@ static int ensure_traj_graph(cdc_ctx* ctx, int every) {
     return CDC_OK;
 }
 
+// After a launch that may read the seed block: marks where cdc_set_image_seeds may rewrite it (nothing to mark before the
+// first cdc_set_image_seeds: the block has not been written since the bind zeroed it).
+static int seeds_read(cdc_ctx* ctx, cudaStream_t s) {
+    if (ctx->seeds_done) CK(cudaEventRecord(ctx->seeds_done, s));
+    return CDC_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ C ABI
 #define GUARD() DevGuard dev_guard_(ctx->device)
 
@@ -1384,6 +1403,7 @@ void cdc_destroy(cdc_ctx* ctx) {
         if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
         if (ctx->traj_ptrs) cudaFree(ctx->traj_ptrs);
         if (ctx->traj_done) cudaEventDestroy(ctx->traj_done);
+        if (ctx->seeds_done) cudaEventDestroy(ctx->seeds_done);
     }
     delete ctx;
 }
@@ -1754,10 +1774,39 @@ int cdc_get_x0(cdc_ctx* ctx, float* x0, cdc_stream s) {
     return CDC_OK;
 }
 
+int cdc_set_image_seeds(cdc_ctx* ctx, const uint64_t* seeds_host, int n, cdc_stream s) {
+    NEED_PLAN();
+    if (n != 0 && n != ctx->B) return ctx->fail(CDC_ERR_SHAPE, "cdc_set_image_seeds: %d seeds for a batch of %d (give B, or 0 to turn per-image mode off)", n, ctx->B);
+    if (n != 0 && !seeds_host) return ctx->fail(CDC_ERR_SHAPE, "cdc_set_image_seeds: null seeds");
+    if (n == 0 && !ctx->seeded) return CDC_OK;
+    if (!ctx->seeds_done) CK(cudaEventCreateWithFlags(&ctx->seeds_done, cudaEventDisableTiming));
+    // the previous launch that reads the block (possibly on another stream) must be past it
+    CK(cudaStreamWaitEvent(S(s), ctx->seeds_done, 0));
+    if (n == 0) {
+        CK(cudaMemsetAsync(ctx->img_seeds, 0, 8, S(s)));
+    } else {
+        std::vector<unsigned long long> blk(static_cast<size_t>(n) + 1);
+        blk[0] = 1;
+        for (int b = 0; b < n; ++b) blk[b + 1] = seeds_host[b];
+        // (pageable source: staged by the driver before the call returns, so blk may go out of scope)
+        CK(cudaMemcpyAsync(ctx->img_seeds, blk.data(), blk.size() * 8, cudaMemcpyHostToDevice, S(s)));
+    }
+    ctx->seeded = n != 0;
+    return CDC_OK;
+}
+
+int cdc_init_noise(cdc_ctx* ctx, float gamma, cdc_stream s) {
+    NEED_PLAN();
+    if (!ctx->seeded) return ctx->fail(CDC_ERR_STATE, "cdc_init_noise: no per-image seeds bound (cdc_set_image_seeds)");
+    CK(launch_init_noise(ctx->img_seeds, ctx->xs, ctx->xpad.p, gamma, ctx->B, ctx->H * ctx->W, S(s)));
+    return seeds_read(ctx, S(s));
+}
+
 int cdc_denoise_step(cdc_ctx* ctx, int k, cdc_stream s) {
     NEED_PLAN();
     if (k < 0 || k >= ctx->K) return ctx->fail(CDC_ERR_SHAPE, "step %d outside the %d-step schedule", k, ctx->K);
-    return run_ops(ctx, ctx->step_seq, S(s), k);
+    int r = run_ops(ctx, ctx->step_seq, S(s), k);
+    return r ? r : seeds_read(ctx, S(s));
 }
 
 int cdc_decode(cdc_ctx* ctx, cdc_stream s) {
@@ -1766,7 +1815,7 @@ int cdc_decode(cdc_ctx* ctx, cdc_stream s) {
     int r = ensure_graph(ctx);
     if (r) return r;
     CK(cudaGraphLaunch(ctx->graph, S(s)));
-    return CDC_OK;
+    return seeds_read(ctx, S(s));
 }
 
 int cdc_decode_trajectory(cdc_ctx* ctx, float* x_traj, float* x0_traj, int every, cdc_stream s) {
@@ -1795,7 +1844,7 @@ int cdc_decode_trajectory(cdc_ctx* ctx, float* x_traj, float* x0_traj, int every
     CK(cudaGraphLaunch(ctx->traj_graph, S(s)));
     CK(cudaEventRecord(ctx->traj_done, S(s)));
     ctx->traj_issued = static_cast<int>(ctx->traj_ev.size());
-    return CDC_OK;
+    return seeds_read(ctx, S(s));
 }
 
 int cdc_trajectory_wait(cdc_ctx* ctx, int j) {
@@ -1817,9 +1866,9 @@ static bool host_ptr_is_pinned(const void* p) {
     return at.type == cudaMemoryTypeHost;
 }
 
-int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host, float* image_host, cdc_stream s) {
-    NEED_PLAN();
-    if (!latent_host || !xT_host || !image_host) return ctx->fail(CDC_ERR_SHAPE, "null host buffer");
+// cdc_decode_host (xT_host given) and cdc_decode_host_seeded (xT_host null: x_T drawn on the device from the bound seeds)
+static int decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host, float gamma, float* image_host, cdc_stream s) {
+    if (!latent_host || !image_host) return ctx->fail(CDC_ERR_SHAPE, "null host buffer");
     const size_t nl = static_cast<size_t>(ctx->B) * ctx->cfg.latent_ch * (ctx->H / 16) * (ctx->W / 16);
     const size_t nx = static_cast<size_t>(ctx->B) * 3 * ctx->H * ctx->W;
     if (nl > ctx->pin_nl || nx > ctx->pin_nx) {  // (re)size the pinned staging buffers for this shape
@@ -1847,23 +1896,28 @@ int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host
         memcpy(ctx->pin_in, latent_host, nl * 4);
         lat_src = ctx->pin_in;
     }
-    if (!host_ptr_is_pinned(xT_host)) {
+    if (xT_host && !host_ptr_is_pinned(xT_host)) {
         memcpy(ctx->pin_x, xT_host, nx * 4);
         x_src = ctx->pin_x;
     }
     float* d_lat = ctx->stage_f32;
     float* d_x = ctx->stage_f32 + nl;
     if (nl + nx > ctx->stage_elems) return ctx->fail(CDC_ERR_SHAPE, "staging buffer too small");
-    // x_T (4.7 MB at 768x512) rides a second stream while the context net runs on the latent
-    CK(cudaEventRecord(ctx->ev_fork, S(s)));
-    CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_fork, 0));
-    CK(cudaMemcpyAsync(d_x, x_src, nx * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
-    CK(cudaEventRecord(ctx->ev_x, ctx->copy_stream));
+    if (xT_host) {  // x_T (4.7 MB at 768x512) rides a second stream while the context net runs on the latent
+        CK(cudaEventRecord(ctx->ev_fork, S(s)));
+        CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_fork, 0));
+        CK(cudaMemcpyAsync(d_x, x_src, nx * 4, cudaMemcpyHostToDevice, ctx->copy_stream));
+        CK(cudaEventRecord(ctx->ev_x, ctx->copy_stream));
+    }
     CK(cudaMemcpyAsync(d_lat, lat_src, nl * 4, cudaMemcpyHostToDevice, S(s)));
     int r;
     if ((r = cdc_set_latent(ctx, d_lat, s))) return r;
-    CK(cudaStreamWaitEvent(S(s), ctx->ev_x, 0));
-    if ((r = cdc_set_x(ctx, d_x, s))) return r;
+    if (xT_host) {
+        CK(cudaStreamWaitEvent(S(s), ctx->ev_x, 0));
+        if ((r = cdc_set_x(ctx, d_x, s))) return r;
+    } else if ((r = cdc_init_noise(ctx, gamma, s))) {
+        return r;
+    }
     if ((r = cdc_decode(ctx, s))) return r;
     if ((r = cdc_get_x(ctx, d_x, 1, s))) return r;
     const bool out_pinned = host_ptr_is_pinned(image_host);
@@ -1871,6 +1925,18 @@ int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host
     CK(cudaStreamSynchronize(S(s)));
     if (!out_pinned) memcpy(image_host, ctx->pin_out, nx * 4);
     return CDC_OK;
+}
+
+int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host, float* image_host, cdc_stream s) {
+    NEED_PLAN();
+    if (!xT_host) return ctx->fail(CDC_ERR_SHAPE, "null host buffer");
+    return decode_host(ctx, latent_host, xT_host, 0.0f, image_host, s);
+}
+
+int cdc_decode_host_seeded(cdc_ctx* ctx, const float* latent_host, float gamma, float* image_host, cdc_stream s) {
+    NEED_PLAN();
+    if (!ctx->seeded) return ctx->fail(CDC_ERR_STATE, "cdc_decode_host_seeded: no per-image seeds bound (cdc_set_image_seeds)");
+    return decode_host(ctx, latent_host, nullptr, gamma, image_host, s);
 }
 
 static int count_kernels(const std::vector<Op>& ops) {  // the GroupNorm-slot memset node is not a kernel of ours

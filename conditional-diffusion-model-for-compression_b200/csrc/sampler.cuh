@@ -9,6 +9,9 @@
 // (pixel index, step, 0, 0); words 0/1 -> Box-Muller pair (channels 0, 1), words 2/3 -> channel 2.  The oracle
 // (oracle/sampler.py philox_normal) restates the same function in numpy, so a teacher-forced stochastic step can be
 // compared within the float tolerance.
+// Per-image mode (cdc_set_image_seeds): the key is image b's own seed and the counter's pixel is the index h*W + w
+// WITHIN the image, so image b's noise does not depend on the batch it is decoded in.  Step k's plane uses counter words
+// (k, 0), the x_T plane (init_noise_kernel) (0, 1): the two never share a counter.
 // Oracle counterpart: oracle/sampler.py ddim_update / make_schedule (the reference ships no code).
 #pragma once
 #include <cuda_runtime.h>
@@ -37,11 +40,8 @@ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t
     out[3] = c3;
 }
 
-// three standard normals of pixel `pix` at sampler step `step`
-__device__ __forceinline__ void philox_normal3(unsigned long long seed, int step, unsigned long long pix, float (&z)[3]) {
-    uint32_t w[4];
-    philox4x32_10(static_cast<uint32_t>(pix), static_cast<uint32_t>(pix >> 32), static_cast<uint32_t>(step), 0u,
-                  static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), w);
+// Philox words -> three standard normals (shared by every noise plane)
+__device__ __forceinline__ void philox_words_normal3(const uint32_t (&w)[4], float (&z)[3]) {
     const float u0 = (static_cast<float>(w[0] >> 9) + 0.5f) * (1.0f / 8388608.0f);   // (0, 1): 23 bits + 1/2, exact in fp32
     const float u2 = (static_cast<float>(w[2] >> 9) + 0.5f) * (1.0f / 8388608.0f);
     const float t1 = static_cast<float>(w[1] >> 8) * (1.0f / 16777216.0f);           // [0, 1)
@@ -55,17 +55,35 @@ __device__ __forceinline__ void philox_normal3(unsigned long long seed, int step
     z[2] = r2 * c3;
 }
 
+// three standard normals of counter (pix, c2, c3) under key `seed`
+__device__ __forceinline__ void philox_normal3(unsigned long long seed, unsigned long long pix, uint32_t c2, uint32_t c3,
+                                               float (&z)[3]) {
+    uint32_t w[4];
+    philox4x32_10(static_cast<uint32_t>(pix), static_cast<uint32_t>(pix >> 32), c2, c3, static_cast<uint32_t>(seed),
+                  static_cast<uint32_t>(seed >> 32), w);
+    philox_words_normal3(w, z);
+}
+
 struct SamplerCoef {
     float c0, c1, e0, e1, sg;
     unsigned long long seed;
     int step;
+    const unsigned long long* img_seeds;  // kernels.cuh ImageSeeds block, or null; read only when sg != 0
+    unsigned int hw;                      // pixels per image
 };
 
 // one pixel's three channels: returns x_prev in xn, the (unclamped) x0 estimate in x0
 __device__ __forceinline__ void sampler_update3(const SamplerCoef& s, const float (&outv)[3], const float (&xt)[3],
                                                 unsigned long long pix, float (&x0)[3], float (&xn)[3]) {
     float z[3] = {0.f, 0.f, 0.f};
-    if (s.sg != 0.0f) philox_normal3(s.seed, s.step, pix, z);
+    if (s.sg != 0.0f) {
+        if (s.img_seeds && s.img_seeds[0]) {  // per-image mode: image b's seed, pixel within the image
+            const unsigned long long b = pix / s.hw;
+            philox_normal3(s.img_seeds[1 + b], pix - b * s.hw, static_cast<uint32_t>(s.step), 0u, z);
+        } else {
+            philox_normal3(s.seed, pix, static_cast<uint32_t>(s.step), 0u, z);
+        }
+    }
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
         // (e0 = 0, e1 = 1 reproduces out exactly: 0 * x_t is +-0 for finite x_t and 1 * out + 0 = out)

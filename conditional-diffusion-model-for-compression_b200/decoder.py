@@ -4,7 +4,9 @@ Same surface as oracle/sampler.py OracleDecoder (the reference ships no code, so
 *is* the reference interface for this path; SURVEY.md section 8b):
     set_sample_schedule(steps), predict_x0(x_t, t, cond), denoise_step(x_t, t, cond),
     decode(latent, steps, *, init=None, gamma=0.8, seed=0, trajectory=None), quantize_symbols, cdf_lookup;
-plus decode_progressive, a generator of per-step (x_t, x0_hat) previews while the decode runs.
+plus decode_progressive, a generator of per-step (x_t, x0_hat) previews while the decode runs, and per-image seeds
+(decode(..., seeds=[...]) / set_image_seeds): image b's x_T and sampler noise then depend on seeds[b] alone, so an image
+decodes to the same result in any batch.
 Tensors at this surface are NCHW fp32 torch tensors; CUDA tensors are used in place, CPU tensors
 are staged through pinned memory by the library (cdc_decode_host).
 """
@@ -22,6 +24,24 @@ def _stream_ptr():
 
 def _f32c(t, dev):
     return t.to(device=dev, dtype=torch.float32).contiguous()
+
+
+def _seed_values(seeds, n):
+    """seeds (a sequence of ints, or an int64 / uint64 tensor) -> list of n ints in [0, 2^64); ValueError otherwise."""
+    if isinstance(seeds, torch.Tensor):
+        if seeds.dtype not in (torch.int64, torch.uint64) or seeds.dim() != 1:
+            raise ValueError(f"seeds must be a 1-D int64 / uint64 tensor, got {seeds.dtype} of shape {tuple(seeds.shape)}")
+        vals = seeds.cpu().tolist()
+    else:
+        vals = list(seeds)
+    if len(vals) != n:
+        raise ValueError(f"{len(vals)} seeds for a batch of {n}: give one per image")
+    for v in vals:
+        if isinstance(v, bool) or not hasattr(v, "__index__"):
+            raise ValueError(f"seed {v!r} is not an integer")
+        if not 0 <= int(v) < 1 << 64:
+            raise ValueError(f"seed {int(v)} is outside [0, 2^64)")
+    return [int(v) for v in vals]
 
 
 class Decoder:
@@ -193,6 +213,23 @@ class Decoder:
             self._ck(self.L.cdc_get_x0(self.ctx, C.c_void_p(out.data_ptr()), self._stream()), "cdc_get_x0")
         return out
 
+    def set_image_seeds(self, seeds):
+        """Per-image noise for the bound batch (include/cdc_b200.h cdc_set_image_seeds): seeds[b] keys image b's x_T
+        (init_noise) and its sampler noise at eta > 0, at the pixel's index within the image.  None turns the mode off:
+        the batch-wide seed of set_sample_schedule applies again.  denoise_step / predict_x0 / decode_resident use
+        whatever is bound; a bind to another shape turns the mode off."""
+        if self.shape is None:
+            raise RuntimeError("nothing bound: call set_latent / set_cond first")
+        vals = [] if seeds is None else _seed_values(seeds, self.shape[0])
+        arr = (C.c_uint64 * max(len(vals), 1))(*vals)
+        with torch.cuda.device(self.device):
+            self._ck(self.L.cdc_set_image_seeds(self.ctx, arr, len(vals), self._stream()), "cdc_set_image_seeds")
+
+    def init_noise(self, gamma=0.8):
+        """x_T = gamma * z from the bound per-image seeds, written into the sampler state on the device."""
+        with torch.cuda.device(self.device):
+            self._ck(self.L.cdc_init_noise(self.ctx, float(gamma), self._stream()), "cdc_init_noise")
+
     # ---- the hot path --------------------------------------------------------------------------
     @torch.no_grad()
     def denoise_step(self, x_t, t, cond=None):
@@ -210,15 +247,20 @@ class Decoder:
         self.denoise_step(x_t, t, cond)
         return self._get_x0()
 
-    def _decode_inputs(self, latent, steps, init, gamma, seed):
-        """Schedule, shape checks and the default x_T shared by decode and decode_progressive."""
+    def _decode_inputs(self, latent, steps, init, gamma, seed, seeds=None):
+        """Schedule, shape checks and the default x_T shared by decode and decode_progressive.  With per-image seeds
+        x_T is drawn on the device later (init stays None); the seeds are checked here, before anything is bound."""
         if steps != self.steps:
             self.set_sample_schedule(steps, *self.sampler)
         if latent.dim() != 4 or latent.shape[1] != self.cfg.latent_ch:
             raise ValueError(f"latent must be [B, {self.cfg.latent_ch}, H/16, W/16], got {tuple(latent.shape)}")
         B, _, h, w = latent.shape
         H, W = h * 16, w * 16
-        if init is None:
+        if seeds is not None:
+            if init is not None:
+                raise ValueError("give init or seeds, not both")
+            _seed_values(seeds, B)
+        elif init is None:
             g = torch.Generator().manual_seed(seed)
             init = gamma * torch.randn(B, 3, H, W, generator=g)
         elif tuple(init.shape) != (B, 3, H, W):
@@ -233,19 +275,38 @@ class Decoder:
             raise ValueError("out must be a contiguous fp32 host tensor of shape [B,3,H,W]")
         return out
 
+    def _bind_x(self, init, seeds, gamma):
+        """x_T into the sampler state: init copied in, or drawn on the device from the per-image seeds."""
+        if seeds is None:
+            self._set_x(init)
+        else:
+            self.init_noise(gamma)
+
     @torch.no_grad()
-    def decode(self, latent, steps, *, init=None, gamma=0.8, seed=0, cond=None, out=None, trajectory=None, x0_trajectory=None):
+    def decode(self, latent, steps, *, init=None, gamma=0.8, seed=0, seeds=None, cond=None, out=None, trajectory=None,
+               x0_trajectory=None):
         """latent y_hat fp32 [B,256,H/16,W/16] -> image fp32 [B,3,H,W] in [0,1] (K steps = one graph launch).
         Host tensors take the cdc_decode_host path (H2D + decode + D2H inside the library); page-locked inputs and a
         page-locked `out` (optional, host path only: fp32 [B,3,H,W], returned) are copied from / to directly.
         trajectory / x0_trajectory (lists, as oracle/sampler.py OracleDecoder.decode(trajectory=...)): K device tensors
         [B,3,H,W] are appended to each given list, x_t entering step k and the raw x0_hat of step k (views of one
-        allocation, recorded inside the graph by cdc_decode_trajectory).  The image is the same bits either way."""
-        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed)
+        allocation, recorded inside the graph by cdc_decode_trajectory).  The image is the same bits either way.
+        seeds (one int in [0, 2^64) per image: a sequence, or an int64 / uint64 tensor; not with init): x_T = gamma * z and
+        the eta > 0 sampler noise of image b are keyed by seeds[b] alone (set_image_seeds), so image b decodes the same in
+        any batch.  Without seeds the batch-wide seed applies (x_T from torch.randn with `seed`, as before)."""
+        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed, seeds)
         record = trajectory is not None or x0_trajectory is not None
-        host = cond is None and not latent.is_cuda and not init.is_cuda
+        host = cond is None and not latent.is_cuda and (init is None or not init.is_cuda)
         with torch.cuda.device(self.device):
             self.bind(B, H, W)
+            self.set_image_seeds(seeds)
+            if host and not record and seeds is not None:
+                # host buffers, x_T drawn on the device: no x_T transfer
+                lat = latent.float().contiguous()
+                out = self._check_host_out(out, B, H, W)
+                self._ck(self.L.cdc_decode_host_seeded(self.ctx, C.c_void_p(lat.data_ptr()), float(gamma),
+                                                       C.c_void_p(out.data_ptr()), self._stream()), "cdc_decode_host_seeded")
+                return out
             if host and not record:
                 # host buffers: pinned staging + H2D/D2H inside the library
                 lat = latent.float().contiguous()
@@ -260,7 +321,7 @@ class Decoder:
                 self.set_cond(cond)
             else:
                 self.set_latent(latent)
-            self._set_x(init)
+            self._bind_x(init, seeds, gamma)
             if not record:
                 self._ck(self.L.cdc_decode(self.ctx, self._stream()), "cdc_decode")
                 return self._get_x(to_image=True)
@@ -312,24 +373,25 @@ class Decoder:
                      "cdc_decode_trajectory")
 
     @torch.no_grad()
-    def decode_progressive(self, latent, steps, *, every=1, init=None, gamma=0.8, seed=0, cond=None):
+    def decode_progressive(self, latent, steps, *, every=1, init=None, gamma=0.8, seed=0, seeds=None, cond=None):
         """Generator: decode as `decode` does and yield (k, x_t, x0_hat) for k = 0, every, 2 * every, ... as soon as
         the graph has written step k: x_t [B,3,H,W] entering step k and the network's raw x0_hat of that step, device
         fp32.  (x0_hat.clamp(-1, 1) + 1) / 2 is the preview image.  The graph runs on a stream of its own, so the
         caller's stream can copy or display a slot while later steps run; stepping the last x_t once more gives decode()'s
         image.  The buffers live until the graph has passed them, so stopping early is safe.  While the generator is
         suspended, any call of this decoder first makes the current stream wait for the graph; once it ends (exhausted
-        or closed), the caller's stream waits for the graph."""
+        or closed), the caller's stream waits for the graph.  seeds: as in decode."""
         if int(every) < 1:
             raise ValueError(f"every must be >= 1, got {every}")
-        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed)
+        init, (B, H, W) = self._decode_inputs(latent, steps, init, gamma, seed, seeds)
         with torch.cuda.device(self.device):
             self.bind(B, H, W)
+            self.set_image_seeds(seeds)
             if cond is not None:
                 self.set_cond(cond)
             else:
                 self.set_latent(latent)
-            self._set_x(init)
+            self._bind_x(init, seeds, gamma)
             xt, x0 = self._traj_buffers(True, True, every)
             cur = torch.cuda.current_stream()
             if self._side is None:

@@ -120,6 +120,19 @@ int cdc_trajectory_wait(cdc_ctx* ctx, int j);
 /* host-buffer convenience used for end-to-end timing: H2D(latent, x_T) -> context net -> decode ->
  * D2H(image in [0,1]); synchronises the stream before returning. */
 int cdc_decode_host(cdc_ctx* ctx, const float* latent_host, const float* xT_host, float* image_host, cdc_stream s);
+
+/* ---- per-image seeds: image b's noise depends only on (seeds[b], pixel within the image, plane), not on its batch ----
+ * Philox4x32-10 keyed by seeds[b], counter (p, c2, c3) with p = h*W + w inside the image: x_T uses (c2, c3) = (0, 1),
+ * the sampler noise of step k (eta > 0) (k, 0).  Without seeds bound, the noise is the batch-wide one of cdc_set_sampler.
+ * cdc_set_image_seeds: n == batch turns per-image mode on with these seeds, n == 0 turns it off; any other n is
+ * CDC_ERR_SHAPE.  Written in stream order on `s` (after the last launch that read the previous seeds); the captured graphs
+ * are not re-captured.  A cdc_bind_io to a different shape turns the mode off. */
+int cdc_set_image_seeds(cdc_ctx* ctx, const uint64_t* seeds_host, int n, cdc_stream s);
+/* x_T = gamma * z(seeds[b], pixel) into the sampler state (as cdc_set_x would put it); CDC_ERR_STATE without seeds bound */
+int cdc_init_noise(cdc_ctx* ctx, float gamma, cdc_stream s);
+/* cdc_decode_host with x_T drawn on the device from the bound seeds (cdc_init_noise) instead of copied from the host */
+int cdc_decode_host_seeded(cdc_ctx* ctx, const float* latent_host, float gamma, float* image_host, cdc_stream s);
+
 int cdc_launches_per_step(cdc_ctx* ctx);
 int cdc_launches_context(cdc_ctx* ctx);
 double cdc_flops_per_step(cdc_ctx* ctx); /* algorithmic, SURVEY.md section 8d rule */
