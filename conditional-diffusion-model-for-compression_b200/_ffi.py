@@ -21,9 +21,11 @@ SYMBOLS = [
 TOOLS_SYMBOLS = [
     "cdc_set_plan_option", "cdc_num_step_ops", "cdc_step_op_name", "cdc_step_op_flops", "cdc_step_op_bytes", "cdc_run_step_op",
     "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn", "cdc_step_op_describe",
+    "cdc_seq_num_ops", "cdc_seq_op_name", "cdc_seq_op_flops", "cdc_seq_op_bytes", "cdc_seq_op_describe", "cdc_run_seq_op",
 ]
 OPT_FUSE_APPLY, OPT_KF = range(2)
 OPK_MEMSET, OPK_CONV, OPK_GN_STATS, OPK_GN_APPLY, OPK_ATTENTION = range(5)  # cdc_op_kind
+SEQ_STEP, SEQ_CONTEXT, SEQ_ENCODER, SEQ_HYPER_ENC, SEQ_HYPER_DEC = range(5)  # cdc_seq
 
 
 class CdcConfig(C.Structure):
@@ -44,7 +46,7 @@ class StepOpDesc(C.Structure):
                 ("xk16", C.c_int32), ("tr", C.c_int32), ("res1", C.c_int32), ("apply", C.c_int32),
                 ("src", TensorDesc * 2), ("residual", TensorDesc), ("out", TensorDesc), ("res_out", TensorDesc),
                 ("gn_in_acc", C.c_void_p), ("gn_out_acc", C.c_void_p), ("gn_slots", C.c_int32),
-                ("x", C.c_void_p), ("x0_out", C.c_void_p), ("xpad", C.c_void_p)]
+                ("x", C.c_void_p), ("x0_out", C.c_void_p), ("xpad", C.c_void_p), ("act_slope", C.c_float)]
 
 
 _libs = {}
@@ -127,6 +129,15 @@ def _bind(L):
     L.cdc_step_op_bytes.restype = C.c_double
     L.cdc_run_step_op.argtypes = [p, i32, i32, p]
     L.cdc_step_op_describe.argtypes = [p, i32, C.POINTER(StepOpDesc)]
+    L.cdc_seq_num_ops.argtypes = [p, i32]
+    L.cdc_seq_op_name.argtypes = [p, i32, i32]
+    L.cdc_seq_op_name.restype = C.c_char_p
+    L.cdc_seq_op_flops.argtypes = [p, i32, i32]
+    L.cdc_seq_op_flops.restype = C.c_double
+    L.cdc_seq_op_bytes.argtypes = [p, i32, i32]
+    L.cdc_seq_op_bytes.restype = C.c_double
+    L.cdc_seq_op_describe.argtypes = [p, i32, i32, C.POINTER(StepOpDesc)]
+    L.cdc_run_seq_op.argtypes = [p, i32, i32, i32, p]
     L.cdc_profile_step.argtypes = [p, i32, i32, fp, p]
     L.cdc_profile_graph.argtypes = [p, i32, fp, fp, p]
     L.cdc_test_conv.argtypes = [i32, p, i32, p, i32, i32, i32, i32, f32p, f32p, i32, i32, i32, i32, p, p, p, p]

@@ -22,7 +22,6 @@ typedef __half act_t;
 constexpr uint32_t kUmmaFormat = 0;  // tcgen05 kind::f16 a_format / b_format: 0 = F16
 #define CDC_TMA_DTYPE CU_TENSOR_MAP_DATA_TYPE_FLOAT16
 constexpr float kActMax = 65504.0f;  // values beyond it are stored saturated (and counted: ConvParams::sat)
-__host__ __device__ __forceinline__ float sat_act(float v) { return fminf(fmaxf(v, -65504.0f), 65504.0f); }
 __device__ __forceinline__ uint32_t pack_act2(float lo, float hi) {  // saturating: never stores inf
     uint32_t r;
     asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
@@ -44,7 +43,12 @@ __device__ __forceinline__ uint32_t act2_absmax(uint32_t m, const uint4& v) {
     return act2_absmax(act2_absmax(act2_absmax(act2_absmax(m, v.x), v.y), v.z), v.w);
 }
 __device__ __forceinline__ bool act2_is_sat(uint32_t m) { return (m & 0xFFFFu) == 0x7BFFu || (m >> 16) == 0x7BFFu; }
-__device__ __forceinline__ act_t to_act(float v) { return __float2half_rn(sat_act(v)); }
+// one value, saturating like pack_act2 (+-inf and finite values beyond the range -> +-65504) and keeping NaN a NaN
+__device__ __forceinline__ act_t to_act(float v) {
+    unsigned short r;
+    asm("cvt.rn.satfinite.f16.f32 %0, %1;" : "=h"(r) : "f"(v));
+    return __ushort_as_half(r);
+}
 __device__ __forceinline__ float from_act(act_t v) { return __half2float(v); }
 #else
 typedef __nv_bfloat16 act_t;

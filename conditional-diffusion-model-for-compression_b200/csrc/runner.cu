@@ -594,6 +594,7 @@ static int build_conv(const ConvBuild& cb, int B, int num_sms, const PlanOpts& p
         d.residual.p = const_cast<act_t*>(cb.residual);
     }
     d.gn_out_acc = cb.gn_acc;
+    d.act_slope = cb.act_slope;
     d.x = cb.x;
     d.x0_out = cb.x0_out;
     d.xpad = cb.xpad;
@@ -1979,29 +1980,84 @@ int cdc_set_plan_option(cdc_ctx* ctx, int option, int value) {
     return CDC_OK;
 }
 
-int cdc_num_step_ops(cdc_ctx* ctx) { return ctx ? static_cast<int>(ctx->step_seq.ops.size()) : 0; }
-const char* cdc_step_op_name(cdc_ctx* ctx, int i) {
-    return (ctx && i >= 0 && i < static_cast<int>(ctx->step_seq.ops.size())) ? ctx->step_seq.ops[i].name.c_str() : "";
+// The op sequence `seq` (cdc_seq) of the plan, or null with the error in ctx->err and its code in *rc.
+static Seq* find_seq(cdc_ctx* ctx, int seq, int* rc) {
+    switch (seq) {
+        case CDC_SEQ_STEP: return &ctx->step_seq;
+        case CDC_SEQ_CONTEXT:
+            if (ctx->has_ctx) return &ctx->ctx_seq;
+            *rc = ctx->fail(CDC_ERR_WEIGHT, "op sequence %d: context-net weights (context.*) were not loaded", seq);
+            return nullptr;
+        case CDC_SEQ_ENCODER:
+        case CDC_SEQ_HYPER_ENC:
+        case CDC_SEQ_HYPER_DEC:
+            if (ctx->has_codec) return seq == CDC_SEQ_ENCODER ? &ctx->enc_seq : seq == CDC_SEQ_HYPER_ENC ? &ctx->henc_seq : &ctx->hdec_seq;
+            *rc = ctx->fail(CDC_ERR_WEIGHT, "op sequence %d: codec weights (codec.*) were not loaded", seq);
+            return nullptr;
+        default:
+            *rc = ctx->fail(CDC_ERR_SHAPE, "unknown op sequence %d", seq);
+            return nullptr;
+    }
 }
-double cdc_step_op_flops(cdc_ctx* ctx, int i) {
-    return (ctx && i >= 0 && i < static_cast<int>(ctx->step_seq.ops.size())) ? ctx->step_seq.ops[i].flops : 0;
+// op i of sequence seq, or null (error in ctx->err)
+static const Op* find_op(cdc_ctx* ctx, int seq, int i) {
+    int rc = CDC_OK;
+    const Seq* q = ctx ? find_seq(ctx, seq, &rc) : nullptr;
+    if (!q) return nullptr;
+    if (i < 0 || i >= static_cast<int>(q->ops.size())) {
+        ctx->fail(CDC_ERR_SHAPE, "op %d outside the %zu ops of sequence %d", i, q->ops.size(), seq);
+        return nullptr;
+    }
+    return &q->ops[i];
 }
-double cdc_step_op_bytes(cdc_ctx* ctx, int i) {
-    return (ctx && i >= 0 && i < static_cast<int>(ctx->step_seq.ops.size())) ? ctx->step_seq.ops[i].bytes : 0;
+
+int cdc_seq_num_ops(cdc_ctx* ctx, int seq) {
+    if (!ctx) return 0;
+    int rc = CDC_OK;
+    const Seq* q = find_seq(ctx, seq, &rc);
+    return q ? static_cast<int>(q->ops.size()) : rc;
 }
-int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out) {
+const char* cdc_seq_op_name(cdc_ctx* ctx, int seq, int i) {
+    const Op* op = find_op(ctx, seq, i);
+    return op ? op->name.c_str() : "";
+}
+double cdc_seq_op_flops(cdc_ctx* ctx, int seq, int i) {
+    const Op* op = find_op(ctx, seq, i);
+    return op ? op->flops : 0;
+}
+double cdc_seq_op_bytes(cdc_ctx* ctx, int seq, int i) {
+    const Op* op = find_op(ctx, seq, i);
+    return op ? op->bytes : 0;
+}
+int cdc_seq_op_describe(cdc_ctx* ctx, int seq, int i, cdc_step_op_desc* out) {
     if (!ctx) return CDC_ERR_STATE;
-    if (!out || i < 0 || i >= static_cast<int>(ctx->step_seq.ops.size())) return ctx->fail(CDC_ERR_SHAPE, "bad op index / null output");
-    *out = ctx->step_seq.ops[i].desc;
-    if (out->kind == CDC_OPK_MEMSET) out->gn_slots = ctx->step_seq.gn_used;
+    if (!out) return ctx->fail(CDC_ERR_SHAPE, "null output");
+    int rc = CDC_OK;
+    const Seq* q = find_seq(ctx, seq, &rc);
+    if (!q) return rc;
+    const Op* op = find_op(ctx, seq, i);
+    if (!op) return CDC_ERR_SHAPE;
+    *out = op->desc;
+    if (out->kind == CDC_OPK_MEMSET) out->gn_slots = q->gn_used;
     return CDC_OK;
 }
-int cdc_run_step_op(cdc_ctx* ctx, int i, int k, cdc_stream s) {
+int cdc_run_seq_op(cdc_ctx* ctx, int seq, int i, int k, cdc_stream s) {
     NEED_PLAN();
-    if (i < 0 || i >= static_cast<int>(ctx->step_seq.ops.size()) || k < 0 || k >= ctx->K) return ctx->fail(CDC_ERR_SHAPE, "bad op/step index");
-    CK(ctx->step_seq.ops[i].run(S(s), k, nullptr));
+    int rc = CDC_OK;
+    if (!find_seq(ctx, seq, &rc)) return rc;
+    const Op* op = find_op(ctx, seq, i);
+    if (!op) return CDC_ERR_SHAPE;
+    if (seq == CDC_SEQ_STEP && (k < 0 || k >= ctx->K)) return ctx->fail(CDC_ERR_SHAPE, "step %d outside the %d-step schedule", k, ctx->K);
+    CK(op->run(S(s), seq == CDC_SEQ_STEP ? k : 0, nullptr));  // (the codec sequences run as run_ops runs them: k = 0)
     return CDC_OK;
 }
+
+int cdc_num_step_ops(cdc_ctx* ctx) { return cdc_seq_num_ops(ctx, CDC_SEQ_STEP); }
+const char* cdc_step_op_name(cdc_ctx* ctx, int i) { return cdc_seq_op_name(ctx, CDC_SEQ_STEP, i); }
+double cdc_step_op_flops(cdc_ctx* ctx, int i) { return cdc_seq_op_flops(ctx, CDC_SEQ_STEP, i); }
+double cdc_step_op_bytes(cdc_ctx* ctx, int i) { return cdc_seq_op_bytes(ctx, CDC_SEQ_STEP, i); }
+int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out) { return cdc_seq_op_describe(ctx, CDC_SEQ_STEP, i, out); }
+int cdc_run_step_op(cdc_ctx* ctx, int i, int k, cdc_stream s) { return cdc_run_seq_op(ctx, CDC_SEQ_STEP, i, k, s); }
 
 #ifdef CDC_TOOLS
 // Tools build only: leave a class of ops out of the captured graph (0 = none, 1 = the tcgen05 convs, 2 = the

@@ -424,20 +424,25 @@ class Decoder:
             self._ck(self.L.cdc_saturation_count(self.ctx, C.byref(n), 1 if reset else 0, self._stream()), "cdc_saturation_count")
         return int(n.value)
 
-    def step_ops(self):
-        n = self.L.cdc_num_step_ops(self.ctx)
-        return [(self.L.cdc_step_op_name(self.ctx, i).decode(), self.L.cdc_step_op_flops(self.ctx, i),
-                 self.L.cdc_step_op_bytes(self.ctx, i)) for i in range(n)]
+    def step_ops(self, seq=0):
+        """[(name, flops, bytes)] of the ops of sequence seq of the bound plan (_ffi.SEQ_*: the denoise step, the context
+        net, the analysis encoder, the hyper-encoder, the hyper-decoder; include/cdc_b200_tools.h cdc_seq)."""
+        n = self.L.cdc_seq_num_ops(self.ctx, seq)
+        if n < 0:
+            self._ck(n, "cdc_seq_num_ops")
+        return [(self.L.cdc_seq_op_name(self.ctx, seq, i).decode(), self.L.cdc_seq_op_flops(self.ctx, seq, i),
+                 self.L.cdc_seq_op_bytes(self.ctx, seq, i)) for i in range(n)]
 
-    def step_op_desc(self, i):
-        """_ffi.StepOpDesc of step op i of the bound plan (include/cdc_b200_tools.h cdc_step_op_describe)."""
+    def step_op_desc(self, i, seq=0):
+        """_ffi.StepOpDesc of op i of sequence seq of the bound plan (include/cdc_b200_tools.h cdc_seq_op_describe)."""
         d = _ffi.StepOpDesc()
-        self._ck(self.L.cdc_step_op_describe(self.ctx, i, C.byref(d)), "cdc_step_op_describe")
+        self._ck(self.L.cdc_seq_op_describe(self.ctx, seq, i, C.byref(d)), "cdc_seq_op_describe")
         return d
 
-    def run_step_op(self, i, k=0):
+    def run_step_op(self, i, k=0, seq=0):
+        """Op i of sequence seq alone, on the current stream (k: the sampler step; the codec sequences ignore it)."""
         with torch.cuda.device(self.device):
-            self._ck(self.L.cdc_run_step_op(self.ctx, i, k, self._stream()), "cdc_run_step_op")
+            self._ck(self.L.cdc_run_seq_op(self.ctx, seq, i, k, self._stream()), "cdc_run_seq_op")
 
     def profile_step(self, k=0, warm=1):
         """In-stream device time (us) of every op of step k (launched back to back, CUDA events in the library)."""

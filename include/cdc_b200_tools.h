@@ -5,6 +5,9 @@
  * (The measurement hook that DOES alter results -- leaving op classes out of the captured graph -- and the environment
  * switches exist only in the separate tools build, libcdc_b200_tools.so, compiled with -DCDC_TOOLS by
  * `csrc/build.sh tools`.)
+ * Every op of every sequence the plan builds (the denoise step, the context net, the analysis encoder, the hyper-encoder
+ * and the hyper-decoder) can be described and run alone (cdc_seq_*): tests/test_gpu_step_ops.py and
+ * tests/test_gpu_codec_ops.py check each one against a float64 reference of that one operation.
  */
 #ifndef CDC_B200_TOOLS_H
 #define CDC_B200_TOOLS_H
@@ -24,13 +27,33 @@ typedef enum {
 int cdc_set_plan_option(cdc_ctx* ctx, int option, int value);
 
 /* ---- per-layer access ------------------------------------------------------------------------------------------- */
+/* The op sequences of the bound plan.  The codec sequences exist when their weights were loaded (context.*: CONTEXT;
+ * codec.*: ENCODER, HYPER_ENC, HYPER_DEC); they take no schedule. */
+typedef enum {
+    CDC_SEQ_STEP = 0,       /* one denoise step (cdc_denoise_step) */
+    CDC_SEQ_CONTEXT = 1,    /* the context net (cdc_set_latent) */
+    CDC_SEQ_ENCODER = 2,    /* the analysis encoder (cdc_encode_analysis) */
+    CDC_SEQ_HYPER_ENC = 3,  /* the hyper-encoder (cdc_hyper_encode) */
+    CDC_SEQ_HYPER_DEC = 4,  /* the hyper-decoder (cdc_hyper_decode) */
+    CDC_SEQ_COUNT = 5
+} cdc_seq;
+/* An unknown seq fails with CDC_ERR_SHAPE, a sequence whose weights were not loaded with CDC_ERR_WEIGHT (cdc_last_error
+ * says which): cdc_seq_num_ops returns that code, cdc_seq_op_name "" and the flops / bytes 0. */
+int cdc_seq_num_ops(cdc_ctx* ctx, int seq);
+const char* cdc_seq_op_name(cdc_ctx* ctx, int seq, int i);
+double cdc_seq_op_flops(cdc_ctx* ctx, int seq, int i);
+double cdc_seq_op_bytes(cdc_ctx* ctx, int seq, int i);
+/* runs op i of sequence seq alone on s; k is the sampler step (checked against the schedule for CDC_SEQ_STEP only, the
+ * other sequences ignore it) */
+int cdc_run_seq_op(cdc_ctx* ctx, int seq, int i, int k, cdc_stream s);
+/* the same for CDC_SEQ_STEP */
 int cdc_num_step_ops(cdc_ctx* ctx);
 const char* cdc_step_op_name(cdc_ctx* ctx, int i);
 double cdc_step_op_flops(cdc_ctx* ctx, int i);
 double cdc_step_op_bytes(cdc_ctx* ctx, int i);
 int cdc_run_step_op(cdc_ctx* ctx, int i, int k, cdc_stream s);
 
-/* Read-only description of step op i of the bound plan: what it computes, from which tensors into which, and which
+/* Read-only description of op i of a sequence of the bound plan: what it computes, from which tensors into which, and which
  * kernel instantiation runs it.  Metadata recorded when the plan was built; reading it changes nothing. */
 typedef enum {
     CDC_OPK_MEMSET = 0,     /* clears the step's GroupNorm accumulator slots (gn_out_acc, gn_slots of them) */
@@ -49,8 +72,9 @@ typedef struct {
     char res_weight[64]; /* 1x1 residual conv computed in the same launch ("down.1.rb1.res") or "" */
     char in_gn[64];      /* GroupNorm + SiLU applied to the conv's input rows ("down.0.rb1.gn1") or "" */
     int film_off;        /* offset of the (scale | shift) FiLM pair in a step's FiLM vector (cdc_get_film), -1: none */
-    int mode, ksize, epi, silu;  /* conv: mode 0 stride 1, 1 stride 2, 2 nearest-x2 input; epi 0 store, 1 GroupNorm
-                                    statistics, 2 sampler update (final conv); gn_apply: silu */
+    int mode, ksize, epi, silu;  /* conv: mode 0 stride 1, 1 stride 2, 2 nearest-x2 input, 3 transposed 5x5 stride 2
+                                    (ConvTranspose2d(5, stride 2, padding 2, output_padding 1), weight [in][out][5][5]);
+                                    epi 0 store, 1 GroupNorm statistics, 2 sampler update (final conv); gn_apply: silu */
     int kernel;          /* conv: 1 = conv_tc.cu (general), 2 = conv_kf.cu (strip); 0 otherwise */
     int bn, cpg, ch, staged, xk16, tr, res1, apply;  /* the instantiation / walk that runs (ch: 64-channel input chunks) */
     cdc_tensor_desc src[2], residual, out, res_out;
@@ -60,8 +84,10 @@ typedef struct {
     float* x;            /* final conv: sampler state, NHWC fp32 [B][H][W][3], read as x_t and overwritten with x_prev */
     float* x0_out;       /* final conv: x0 estimate, NHWC fp32 */
     void* xpad;          /* final conv: the stem's 16-bit x_t copy, rewritten with x_prev */
+    float act_slope;     /* conv: LeakyReLU slope applied after the bias (the hyper networks' 0.2), 0: none */
 } cdc_step_op_desc;
-int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out);
+int cdc_seq_op_describe(cdc_ctx* ctx, int seq, int i, cdc_step_op_desc* out);
+int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out);  /* CDC_SEQ_STEP */
 /* in-stream device time (microseconds) of every op of step k, after `warm` untimed steps; us_out[cdc_num_step_ops] */
 int cdc_profile_step(cdc_ctx* ctx, int k, int warm, float* us_out, cdc_stream s);
 /* In-graph timing: captures the same K-step graph with every kernel writing (earliest CTA start, latest CTA end) in
