@@ -16,7 +16,9 @@ SYMBOLS = [
     "cdc_launches_context", "cdc_flops_per_step", "cdc_saturation_count", "cdc_quantize", "cdc_cdf_lookup",
     "cdc_has_codec", "cdc_encode_analysis", "cdc_hyper_encode", "cdc_hyper_decode",
     "cdc_rans_streams_per_channel", "cdc_rans_scratch_bytes", "cdc_rans_max_bytes", "cdc_rans_encode", "cdc_rans_decode",
+    "cdc_set_entropy_tables", "cdc_stream_info", "cdc_compress_max_bytes", "cdc_compress_rgb8", "cdc_decompress_rgb8",
 ]
+ERR_SHAPE, ERR_ARCH, ERR_CUDA, ERR_UNIMPLEMENTED, ERR_STATE, ERR_WEIGHT, ERR_DATA = range(-1, -8, -1)  # cdc_status
 # ... and include/cdc_b200_tools.h (tests / profiling / A-B; same library)
 TOOLS_SYMBOLS = [
     "cdc_set_plan_option", "cdc_num_step_ops", "cdc_step_op_name", "cdc_step_op_flops", "cdc_step_op_bytes", "cdc_run_step_op",
@@ -118,6 +120,12 @@ def _bind(L):
     L.cdc_rans_max_bytes.restype = i64
     L.cdc_rans_encode.argtypes = [p, p, p, p, p, p, i64, i64, i32, p, p, i64, p, p]
     L.cdc_rans_decode.argtypes = [p, i64, p, p, p, p, p, i32, i64, i64, i32, p, p, p, p]
+    L.cdc_set_entropy_tables.argtypes = [p, i32, p, i64, p, p, p, i32, p, p]
+    L.cdc_stream_info.argtypes = [p, i64, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    L.cdc_compress_max_bytes.argtypes = [p]
+    L.cdc_compress_max_bytes.restype = i64
+    L.cdc_compress_rgb8.argtypes = [p, p, p, i64, C.POINTER(i64), p]
+    L.cdc_decompress_rgb8.argtypes = [p, p, i64, C.c_float, p, p]
     # tools header
     L.cdc_set_plan_option.argtypes = [p, i32, i32]
     L.cdc_num_step_ops.argtypes = [p]

@@ -4,6 +4,8 @@ analysis encoder, hyper-encoder / hyper-decoder, latent rounding and CDF lookup,
     codec = Codec(decoder)                  # a Decoder created with the "codec.*" (and "context.*") weights
     enc   = codec.encode(img01)             # dict with the oracle's keys: y, z, qz, z_hat, mu, sigma, q, y_hat, y_sym, z_sym
     img   = codec.decompress(enc["qz"], enc["q"], steps=17)
+    data  = codec.compress_rgb8(rgb8)       # uint8 [B,H,W,3] -> CDC5 bytes, one library call (cdc_compress_rgb8)
+    rgb8  = codec.decompress_rgb8(data, 17, seeds=[7])   # CDC5 bytes -> uint8 [B,H,W,3] (cdc_decompress_rgb8)
 
 Determinism is the contract that matters for a bitstream: encoder and decoder both derive (mu, sigma) from z_hat with
 the same kernels (cdc_hyper_decode), fixed accumulation order, so q / idx / (lo, hi) agree bit for bit between the two
@@ -12,8 +14,8 @@ import ctypes as C
 
 import torch
 
-from . import entropy_tables
-from .decoder import Decoder, DeviceTables, _f32c, _stream_ptr, cdf_lookup, quantize_symbols
+from . import _ffi, entropy_tables
+from .decoder import Decoder, DeviceTables, _f32c, _seed_values, _stream_ptr, cdf_lookup, quantize_symbols
 
 
 class Codec:
@@ -28,6 +30,18 @@ class Codec:
         self.fact = DeviceTables(fact_tables, self.device) if fact_tables is not None else None
         c = decoder.cfg.latent_ch
         self.median = (torch.zeros(c) if median is None else median.detach().float()).to(self.device)
+        # the same tables in the library, for cdc_compress_rgb8 / cdc_decompress_rgb8
+        self._set_tables(0, gauss_tables if gauss_tables is not None else entropy_tables.gaussian_tables())
+        if fact_tables is not None:
+            self._set_tables(1, fact_tables, self.median.cpu().contiguous())
+
+    def _set_tables(self, which, tables, median=None):
+        i32 = [torch.as_tensor(getattr(tables, f)).cpu().to(torch.int32).contiguous() for f in ("cdf", "row_start", "cdf_length", "offset")]
+        scale = torch.as_tensor(tables.scale_table).cpu().to(torch.float32).contiguous() if which == 0 else None
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t is not None else 0)
+        cdf, row_start, cdf_length, offset = i32
+        self._ck(self.L.cdc_set_entropy_tables(self.ctx, which, ptr(cdf), cdf.numel(), ptr(row_start), ptr(cdf_length), ptr(offset),
+                                               row_start.numel(), ptr(scale), ptr(median)), "cdc_set_entropy_tables")
 
     @staticmethod
     def prior_tables(weights, prefix="codec.prior."):
@@ -150,3 +164,59 @@ class Codec:
     def decompress_bytes(self, data: bytes, steps, **kw):
         qz, q = self.decode_symbols(data)
         return self.decompress(qz, q, steps, **kw)
+
+    # ---- the same two directions in one library call each, 8-bit RGB at the boundary ----------------------------------
+    @torch.no_grad()
+    def compress_rgb8(self, img):
+        """uint8 CPU tensor [B,H,W,3] (interleaved RGB, H and W multiples of 64) -> the CDC5 stream as bytes, equal to
+        compress(img.permute(0, 3, 1, 2).float() / 255)[0] (include/cdc_b200.h cdc_compress_rgb8)."""
+        if not isinstance(img, torch.Tensor) or img.dtype != torch.uint8 or img.is_cuda or img.dim() != 4 or img.shape[3] != 3 \
+                or img.shape[0] < 1 or img.shape[1] < 64 or img.shape[2] < 64 or img.shape[1] % 64 or img.shape[2] % 64:
+            raise ValueError("img must be a uint8 CPU tensor [B,H,W,3] with H, W multiples of 64, got "
+                             f"{getattr(img, 'dtype', type(img))} {tuple(getattr(img, 'shape', ()))}")
+        if self.fact is None:
+            raise RuntimeError("compress_rgb8 needs the factorised-prior CDF tables (fact_tables)")
+        B, H, W, _ = img.shape
+        x = img.contiguous()
+        with torch.cuda.device(self.device):
+            self.dec.bind(B, H, W)
+            cap = self.L.cdc_compress_max_bytes(self.ctx)
+            if cap < 0:
+                self._ck(cap, "cdc_compress_max_bytes")
+            out = torch.empty(cap, dtype=torch.uint8)
+            n = C.c_int64(0)
+            self._ck(self.L.cdc_compress_rgb8(self.ctx, C.c_void_p(x.data_ptr()), C.c_void_p(out.data_ptr()), cap, C.byref(n),
+                                              self.dec._stream()), "cdc_compress_rgb8")
+        return out[:n.value].numpy().tobytes()
+
+    @staticmethod
+    def stream_info(data):
+        """(B, H, W) of a CDC5 stream, from the host alone (cdc_stream_info); ValueError if it is malformed."""
+        buf = bytes(data)
+        B, H, W = C.c_int(), C.c_int(), C.c_int()
+        if _ffi.lib().cdc_stream_info(buf, len(buf), C.byref(B), C.byref(H), C.byref(W)) != 0:
+            raise ValueError("not a valid CDC5 stream")
+        return B.value, H.value, W.value
+
+    @torch.no_grad()
+    def decompress_rgb8(self, data, steps, *, seeds, gamma=0.8):
+        """CDC5 bytes -> uint8 CPU tensor [B,H,W,3]: the decode of the stream's latent in `steps` steps with x_T = gamma * z
+        from the per-image seeds, round_half_even(255 * image), in one library call (cdc_decompress_rgb8).  Equal to
+        (decompress_bytes(data, steps, seeds=seeds, gamma=gamma) * 255).round() in uint8 NHWC.  ValueError if the bytes
+        are not a valid stream for this codec."""
+        if self.fact is None:
+            raise RuntimeError("decompress_rgb8 needs the factorised-prior CDF tables (fact_tables)")
+        buf = bytes(data)
+        B, H, W = self.stream_info(buf)
+        _seed_values(seeds, B)
+        with torch.cuda.device(self.device):
+            self.dec.bind(B, H, W)
+            if steps != self.dec.steps:
+                self.dec.set_sample_schedule(steps, *self.dec.sampler)
+            self.dec.set_image_seeds(seeds)
+            out = torch.empty(B, H, W, 3, dtype=torch.uint8)
+            rc = self.L.cdc_decompress_rgb8(self.ctx, buf, len(buf), float(gamma), C.c_void_p(out.data_ptr()), self.dec._stream())
+            if rc == _ffi.ERR_DATA:
+                raise ValueError(f"corrupt CDC5 stream: {self.L.cdc_last_error(self.ctx).decode()}")
+            self._ck(rc, "cdc_decompress_rgb8")
+        return out

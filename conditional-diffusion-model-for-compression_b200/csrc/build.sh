@@ -7,7 +7,7 @@
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
 NVCC="${NVCC:-/usr/local/cuda/bin/nvcc}"
-SRCS=(conv_tc conv_kf elementwise attention entropy rans runner)
+SRCS=(conv_tc conv_kf elementwise attention entropy rans runner bitstream)
 
 build_variant() {  # name, extra flags...
   local name="$1"; shift

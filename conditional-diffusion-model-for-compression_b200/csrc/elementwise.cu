@@ -361,13 +361,16 @@ cudaError_t launch_init_noise(const unsigned long long* seeds, float* xs, act_t*
     return cudaGetLastError();
 }
 
+// The sampler state as an image value in [0, 1]; cdc_get_x(to_image) and the 8-bit output both map through it.
+__device__ __forceinline__ float image01(float v) { return (fminf(fmaxf(v, -1.0f), 1.0f) + 1.0f) / 2.0f; }
+
 // Pixel i of xs (NHWC, 3 fp32 channels) -> its three NCHW planes: consecutive threads store consecutive pixels of a plane.
 __device__ __forceinline__ void x_out_pixel(const float* __restrict__ xs, float* __restrict__ x, long long i, int HW, int to_image) {
     const long long b = i / HW, p = i % HW;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
         float v = xs[i * 3 + c];
-        if (to_image) v = (fminf(fmaxf(v, -1.0f), 1.0f) + 1.0f) / 2.0f;
+        if (to_image) v = image01(v);
         x[(b * 3 + c) * HW + p] = v;
     }
 }
@@ -493,6 +496,90 @@ __global__ void img_in_kernel(const float* __restrict__ img, act_t* __restrict__
 cudaError_t launch_img_in(const float* img_nchw, act_t* dst64, int B, int HW, cudaStream_t s) {
     const long long n = static_cast<long long>(B) * HW;
     img_in_kernel<<<static_cast<int>((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096), 256, 0, s>>>(img_nchw, dst64, n, HW);
+    return cudaGetLastError();
+}
+
+// 8-bit interleaved RGB [n][3] -> img64 channels 0..2 (channel 3 written zero, as it already is), 16 pixels = three 16-byte
+// loads per thread.  2 * (v / 255) - 1 with the division IEEE-rounded as the host's u8 / 255 in fp32 is, so the
+// analysis encoder sees exactly the values launch_img_in makes of that fp32 image.
+__global__ void __launch_bounds__(256) rgb8_in_kernel(const uint8_t* __restrict__ rgb, act_t* __restrict__ dst, long long n16) {
+    for (long long g = blockIdx.x * 256LL + threadIdx.x; g < n16; g += gridDim.x * 256LL) {
+        const uint4* src = reinterpret_cast<const uint4*>(rgb + g * 48);
+        uint4 raw[3] = {src[0], src[1], src[2]};
+        const uint8_t* v = reinterpret_cast<const uint8_t*>(raw);
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+            uint2 w;
+            act_t* px = reinterpret_cast<act_t*>(&w);
+#pragma unroll
+            for (int c = 0; c < 3; ++c) px[c] = to_act(2.0f * (static_cast<float>(v[k * 3 + c]) / 255.0f) - 1.0f);
+            px[3] = to_act(0.0f);
+            *reinterpret_cast<uint2*>(dst + (g * 16 + k) * 64) = w;
+        }
+    }
+}
+cudaError_t launch_rgb8_in(const uint8_t* rgb, act_t* dst64, long long npix, cudaStream_t s) {
+    if (npix % 16 || (reinterpret_cast<uintptr_t>(rgb) & 15u)) return cudaErrorInvalidValue;
+    const long long n16 = npix / 16;
+    rgb8_in_kernel<<<static_cast<int>((n16 + 255) / 256 < 4096 ? (n16 + 255) / 256 : 4096), 256, 0, s>>>(rgb, dst64, n16);
+    return cudaGetLastError();
+}
+
+// xs [n][3] fp32 -> 8-bit interleaved RGB: round_half_even(255 * image01(x)), 16 pixels = twelve 16-byte loads and three
+// 16-byte stores per thread.
+__global__ void __launch_bounds__(256) rgb8_out_kernel(const float* __restrict__ xs, uint8_t* __restrict__ rgb, long long n16) {
+    for (long long g = blockIdx.x * 256LL + threadIdx.x; g < n16; g += gridDim.x * 256LL) {
+        const float4* src = reinterpret_cast<const float4*>(xs + g * 48);
+        uint4 out[3];
+        uint32_t* o = reinterpret_cast<uint32_t*>(out);
+#pragma unroll
+        for (int k = 0; k < 12; ++k) {
+            const float4 f = src[k];
+            const float e[4] = {f.x, f.y, f.z, f.w};
+            uint32_t w = 0;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) w |= static_cast<uint32_t>(static_cast<uint8_t>(rintf(__fmul_rn(image01(e[j]), 255.0f)))) << (8 * j);
+            o[k] = w;
+        }
+        uint4* dst = reinterpret_cast<uint4*>(rgb + g * 48);
+        dst[0] = out[0];
+        dst[1] = out[1];
+        dst[2] = out[2];
+    }
+}
+cudaError_t launch_rgb8_out(const float* xs, uint8_t* rgb, long long npix, cudaStream_t s) {
+    if (npix % 16 || (reinterpret_cast<uintptr_t>(rgb) & 15u) || (reinterpret_cast<uintptr_t>(xs) & 15u)) return cudaErrorInvalidValue;
+    const long long n16 = npix / 16;
+    rgb8_out_kernel<<<static_cast<int>((n16 + 255) / 256 < 4096 ? (n16 + 255) / 256 : 4096), 256, 0, s>>>(xs, rgb, n16);
+    return cudaGetLastError();
+}
+
+// q NCHW int32 [B][C][HW] -> dst NHWC act_t [B][HW][C] = to_act(float(q) + mu), mu = mu_vec[c] or channel c of the NHWC
+// act_t mu_act (ldc channels per pixel).  The same fp32 add and rounding as q.float() + mu on the NCHW fp32 mu, then
+// launch_nchw_f32_to_nhwc_act; the 32 x 32 tile transposes as nchw_to_nhwc_kernel does.
+__global__ void dequant_to_act_kernel(const int32_t* __restrict__ q, const float* __restrict__ mu_vec, const act_t* __restrict__ mu_act,
+                                      int mu_ldc, act_t* __restrict__ dst, int C, int HW) {
+    __shared__ float tile[32][33];
+    const int b = blockIdx.z, c0 = blockIdx.y * 32, p0 = blockIdx.x * 32;
+    for (int j = threadIdx.y; j < 32; j += 8) {
+        const int c = c0 + j, p = p0 + threadIdx.x;
+        tile[j][threadIdx.x] = (c < C && p < HW) ? static_cast<float>(q[(static_cast<size_t>(b) * C + c) * HW + p]) : 0.f;
+    }
+    __syncthreads();
+    for (int j = threadIdx.y; j < 32; j += 8) {
+        const int p = p0 + j, c = c0 + threadIdx.x;
+        if (p < HW && c < C) {
+            const size_t px = static_cast<size_t>(b) * HW + p;
+            const float m = mu_vec ? mu_vec[c] : from_act(mu_act[px * mu_ldc + c]);
+            dst[px * C + c] = to_act(__fadd_rn(tile[threadIdx.x][j], m));
+        }
+    }
+}
+cudaError_t launch_dequant_to_act(const int32_t* q, const float* mu_vec, const act_t* mu_act, int mu_ldc, act_t* dst, int B, int C,
+                                  int HW, cudaStream_t s) {
+    if (!mu_vec == !mu_act) return cudaErrorInvalidValue;
+    dim3 grid((HW + 31) / 32, (C + 31) / 32, B);
+    dequant_to_act_kernel<<<grid, dim3(32, 8), 0, s>>>(q, mu_vec, mu_act, mu_ldc, dst, C, HW);
     return cudaGetLastError();
 }
 

@@ -85,29 +85,40 @@ cudaError_t launch_quantize(const float* y, const float* mu, int32_t* q, float* 
 
 // idx = 63 - #{j in [0,62] : max(sigma, table[0]) <= table[j]}  (or the channel when sigma == null);
 // v = q - offset[idx]; outside [0, max_v) -> escape; (lo, hi) = cdf[idx][v], cdf[idx][v+1].
-struct CdfSmem {
+struct ScaleSmem {
     float tab[64];
     float lg0, inv_step;  // log2(tab[0]), 63 / (log2(tab[63]) - log2(tab[0]))
+};
+struct CdfSmem {
+    ScaleSmem sc;
     int32_t start[256], len[256], off[256];
 };
+
+__device__ __forceinline__ void load_scale_smem(ScaleSmem& sc, const float* __restrict__ scale_table) {  // (the caller syncs)
+    if (threadIdx.x < 64) sc.tab[threadIdx.x] = scale_table[threadIdx.x];
+    if (threadIdx.x == 0) {
+        sc.lg0 = log2f(scale_table[0]);
+        sc.inv_step = 63.0f / (log2f(scale_table[63]) - sc.lg0);
+    }
+}
+
+// The CDF row of a Gaussian symbol: idx = 63 - #{j <= 62 : sg <= tab[j]} = #{j <= 62 : tab[j] < sg} on the ascending
+// table.  The table is log-spaced, so a logarithm lands within one entry of the answer and two exact fix-up loops
+// (comparisons against the table itself) make it exact: 63 compares + 63 adds per symbol had made the lookup ALU-bound
+// (2.6 TB/s).  The encoder's lookup and the decoder's index kernel both call this, so they agree bit for bit.
+__device__ __forceinline__ int scale_index(const ScaleSmem& sc, float sg_in) {
+    const float sg = fmaxf(sg_in, sc.tab[0]);
+    int g = static_cast<int>((__log2f(sg) - sc.lg0) * sc.inv_step) + 1;
+    g = g < 0 ? 0 : (g > 63 ? 63 : g);
+    while (g > 0 && !(sc.tab[g - 1] < sg)) --g;
+    while (g < 63 && sc.tab[g] < sg) ++g;
+    return g;
+}
 
 __device__ __forceinline__ void cdf_one(const CdfSmem& sm, const int32_t* __restrict__ cdf, int rows, bool has_sigma, float sg_in,
                                         int qv, long long i, long long inner, int32_t& idx_o, int32_t& v_o, int32_t& lo_o,
                                         int32_t& hi_o, int32_t& raw_o) {
-    int idx;
-    if (has_sigma) {
-        // idx = 63 - #{j <= 62 : sg <= tab[j]} = #{j <= 62 : tab[j] < sg} on the ascending table.  The table is
-        // log-spaced, so a logarithm lands within one entry of the answer and two exact fix-up loops (comparisons against
-        // the table itself) make it exact: 63 compares + 63 adds per symbol had made this kernel ALU-bound (2.6 TB/s).
-        const float sg = fmaxf(sg_in, sm.tab[0]);
-        int g = static_cast<int>((__log2f(sg) - sm.lg0) * sm.inv_step) + 1;
-        g = g < 0 ? 0 : (g > 63 ? 63 : g);
-        while (g > 0 && !(sm.tab[g - 1] < sg)) --g;
-        while (g < 63 && sm.tab[g] < sg) ++g;
-        idx = g;
-    } else {
-        idx = static_cast<int>((i / inner) % rows);
-    }
+    const int idx = has_sigma ? scale_index(sm.sc, sg_in) : static_cast<int>((i / inner) % rows);
     const int max_v = sm.len[idx] - 2;
     int v = qv - sm.off[idx];
     int raw = 0;
@@ -132,15 +143,11 @@ __global__ void __launch_bounds__(256) cdf_lookup_kernel(const int32_t* __restri
                                                          int32_t* __restrict__ hi_o, int32_t* __restrict__ raw_o,
                                                          long long n, int vec) {
     __shared__ CdfSmem sm;
-    if (t.scale_table && threadIdx.x < 64) sm.tab[threadIdx.x] = t.scale_table[threadIdx.x];
+    if (t.scale_table) load_scale_smem(sm.sc, t.scale_table);
     for (int r = threadIdx.x; r < t.rows && r < 256; r += 256) {
         sm.start[r] = t.row_start[r];
         sm.len[r] = t.cdf_length[r];
         sm.off[r] = t.offset[r];
-    }
-    if (t.scale_table && threadIdx.x == 0) {
-        sm.lg0 = log2f(t.scale_table[0]);
-        sm.inv_step = 63.0f / (log2f(t.scale_table[63]) - sm.lg0);
     }
     __syncthreads();
     const long long tid = blockIdx.x * 256LL + threadIdx.x, nthr = gridDim.x * 256LL;
@@ -188,6 +195,36 @@ cudaError_t launch_cdf_lookup(const int32_t* q, const float* sigma, CdfTables t,
     auto al = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
     const int vec = al(q) && (!sigma || al(sigma)) && al(idx) && al(v) && al(lo) && al(hi) && al(raw) ? 1 : 0;
     cdf_lookup_kernel<<<int_grid(n, vec, num_sms), 256, 0, s>>>(q, sigma, t, inner, idx, v, lo, hi, raw, n, vec);
+    return cudaGetLastError();
+}
+
+// The decoder's CDF rows of y: idx NCHW int32 [B][C][HW] = scale_index(max(sigma, min_sigma)) with sigma channels
+// [c_off, c_off + C) of an NHWC act_t tensor (the hyper-decoder's output), through a 32 x 32 shared tile as
+// nhwc_slice_to_nchw_kernel transposes.  Gives the idx of cdf_lookup on the NCHW fp32 sigma of cdc_hyper_decode without
+// the fp32 round trip.
+__global__ void __launch_bounds__(256) scale_rows_kernel(const act_t* __restrict__ src, const float* __restrict__ scale_table,
+                                                         int32_t* __restrict__ idx, int C, int HW, int ldc, int c_off, float min_sigma) {
+    __shared__ ScaleSmem sc;
+    __shared__ float tile[32][33];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int b = blockIdx.z, c0 = blockIdx.y * 32, p0 = blockIdx.x * 32;
+    load_scale_smem(sc, scale_table);
+    for (int j = ty; j < 32; j += 8) {
+        const int p = p0 + j, c = c0 + tx;
+        tile[j][tx] = (c < C && p < HW) ? from_act(src[(static_cast<size_t>(b) * HW + p) * ldc + c_off + c]) : 0.f;
+    }
+    __syncthreads();
+    for (int j = ty; j < 32; j += 8) {
+        const int c = c0 + j, p = p0 + tx;
+        if (p < HW && c < C) idx[(static_cast<size_t>(b) * C + c) * HW + p] = scale_index(sc, fmaxf(tile[tx][j], min_sigma));
+    }
+}
+
+cudaError_t launch_scale_rows(const act_t* src, int ldc, int c_off, float min_sigma, const float* scale_table, int32_t* idx, int B,
+                              int C, int HW, cudaStream_t s) {
+    if (!scale_table) return cudaErrorInvalidValue;
+    dim3 grid((HW + 31) / 32, (C + 31) / 32, B);
+    scale_rows_kernel<<<grid, 256, 0, s>>>(src, scale_table, idx, C, HW, ldc, c_off, min_sigma);
     return cudaGetLastError();
 }
 

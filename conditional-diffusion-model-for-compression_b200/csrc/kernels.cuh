@@ -73,6 +73,15 @@ cudaError_t launch_repack_weight(const float* src, act_t* dst, int O, int I, int
 cudaError_t launch_repack_weight_convt5(const float* src, act_t* dst, int O, int I, int O_pad, int I_pad, cudaStream_t s);
 // image NCHW fp32 in [0, 1] -> NHWC act_t, 64-channel pixels, channels 0..2 = 2 * img - 1 (channels 3..63 untouched: zero)
 cudaError_t launch_img_in(const float* img_nchw, act_t* dst64, int B, int HW, cudaStream_t s);
+// 8-bit interleaved RGB [npix][3] (16-byte aligned, npix a multiple of 16) -> img64 channels 0..2 = 2 * (v / 255) - 1,
+// the values launch_img_in stores for the fp32 image v / 255
+cudaError_t launch_rgb8_in(const uint8_t* rgb, act_t* dst64, long long npix, cudaStream_t s);
+// xs NHWC fp32 [npix][3] -> 8-bit RGB [npix][3] = round_half_even(255 * (clamp(x,-1,1)+1)/2) (launch_x_out's to_image value)
+cudaError_t launch_rgb8_out(const float* xs, uint8_t* rgb, long long npix, cudaStream_t s);
+// q NCHW int32 [B][C][HW] -> NHWC act_t [B][HW][C] = q + mu in fp32, mu = mu_vec[c] (per channel) or channel c of the NHWC
+// act_t tensor mu_act with mu_ldc channels per pixel (exactly one of the two)
+cudaError_t launch_dequant_to_act(const int32_t* q, const float* mu_vec, const act_t* mu_act, int mu_ldc, act_t* dst, int B, int C,
+                                  int HW, cudaStream_t s);
 // channels [c_off, c_off + C) of an NHWC act_t tensor with ldc channels -> NCHW fp32, optionally clamped from below
 cudaError_t launch_nhwc_slice_to_nchw_f32(const act_t* src, float* dst, int B, int C, int HW, int ldc, int c_off, float min_clamp,
                                           int use_clamp, cudaStream_t s);
@@ -107,6 +116,11 @@ struct CdfTables {
 cudaError_t launch_cdf_lookup(const int32_t* q, const float* sigma, CdfTables t, int64_t inner, int32_t* idx,
                               int32_t* v, int32_t* lo, int32_t* hi, int32_t* raw, int64_t n, int num_sms,
                               cudaStream_t s);
+
+// idx NCHW [B][C][HW] = the Gaussian CDF row (cdf_lookup's scale-table search) of max(sigma, min_sigma), sigma = channels
+// [c_off, c_off + C) of an NHWC act_t tensor with ldc channels per pixel
+cudaError_t launch_scale_rows(const act_t* src, int ldc, int c_off, float min_sigma, const float* scale_table, int32_t* idx, int B,
+                              int C, int HW, cudaStream_t s);
 
 // ---- rANS bitstream (rans.cu; oracle/rans.py pins the format) -------------------------------------------------
 long long rans_scratch_bytes(long long n_chan, long long hw, int spc);

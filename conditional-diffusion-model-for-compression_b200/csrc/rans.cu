@@ -150,6 +150,7 @@ cudaError_t launch_rans_encode(const int32_t* idx, const int32_t* v, const int32
                                unsigned long long* out_bytes, cudaStream_t s) {
     const long long ns = n_chan * spc;
     if (ns <= 0) return cudaErrorInvalidValue;
+    if (reinterpret_cast<uintptr_t>(out) & 3u) return cudaErrorMisalignedAddress;  // the header and size table are u32 stores
     const long long stride = rans_stream_stride(hw, spc);
     uint8_t* sc = static_cast<uint8_t*>(scratch);
     uint32_t* sizes = reinterpret_cast<uint32_t*>(sc + ns * stride);
@@ -242,12 +243,14 @@ cudaError_t launch_rans_decode(const uint8_t* data, long long data_bytes, const 
                                int spc, void* scratch, int32_t* q, int32_t* status, cudaStream_t s) {
     const long long ns = n_chan * spc;
     if (ns <= 0) return cudaErrorInvalidValue;
+    // the size table is read as u32 (a container that starts at an offset of 2 mod 4 in a larger buffer must be copied)
+    if (reinterpret_cast<uintptr_t>(data) & 3u) return cudaErrorMisalignedAddress;
+    if (data_bytes < kRansHeader + 4 * ns) return cudaErrorInvalidValue;  // before any launch reads the size table
     unsigned long long* offs = static_cast<unsigned long long*>(scratch);  // ns entries
     cudaError_t e = cudaMemsetAsync(status, 0, 4, s);
     if (e != cudaSuccess) return e;
     rans_scan_kernel<<<1, 1024, 0, s>>>(reinterpret_cast<const uint32_t*>(data + kRansHeader), offs, ns,
                                         static_cast<unsigned long long>(kRansHeader + 4 * ns), nullptr);
-    if (data_bytes < kRansHeader + 4 * ns) return cudaErrorInvalidValue;
     rans_decode_kernel<<<static_cast<unsigned>((ns + 127) / 128), 128, 0, s>>>(data, offs, idx, t, n_chan, hw, spc, data_bytes, q, status);
     return cudaGetLastError();
 }

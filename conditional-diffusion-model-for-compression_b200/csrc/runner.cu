@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "../../include/cdc_b200_tools.h"
+#include "codec_io.cuh"
 #include "conv_kf.cuh"
 #include "conv_tc.cuh"
 #include "kernels.cuh"
@@ -33,19 +34,6 @@ struct PlanOpts {
     int v[CDC_OPT_COUNT] = {2, 1};
     int fuse_apply_max_tiles() const { return v[CDC_OPT_FUSE_APPLY]; }
     bool kf() const { return v[CDC_OPT_KF] != 0; }
-};
-
-// Every entry point that takes a cdc_ctx runs on the context's device and restores the caller's current device on
-// exit (ADVICE r1: a Decoder on cuda:1 must work -- and must not move the process -- while cuda:0 is current).
-struct DevGuard {
-    int prev = -1, dev;
-    explicit DevGuard(int d) : dev(d) {
-        if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-        if (prev != dev) cudaSetDevice(dev);
-    }
-    ~DevGuard() {
-        if (prev >= 0 && prev != dev) cudaSetDevice(prev);
-    }
 };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -686,6 +674,7 @@ struct cdc_ctx {
     int traj_issued = 0;               // slots of the most recent launch of traj_graph (0: none since it was built)
     TrajPtrs* traj_ptrs = nullptr;     // device block the store nodes read the caller's buffers from
     cudaEvent_t traj_done = nullptr;   // end of the most recent launch: traj_ptrs may be rewritten after it
+    ByteCodec* byte_codec = nullptr;   // cdc_compress_rgb8 / cdc_decompress_rgb8 (bitstream.cu); null until first used
 
     int fail(int code, const char* fmt, ...) {
         char buf[512];
@@ -1405,6 +1394,7 @@ void cdc_destroy(cdc_ctx* ctx) {
         if (ctx->traj_ptrs) cudaFree(ctx->traj_ptrs);
         if (ctx->traj_done) cudaEventDestroy(ctx->traj_done);
         if (ctx->seeds_done) cudaEventDestroy(ctx->seeds_done);
+        byte_codec_destroy(ctx->byte_codec);
     }
     delete ctx;
 }
@@ -1641,6 +1631,7 @@ int cdc_get_film(cdc_ctx* ctx, float* film_dev, cdc_stream s) {
 
 static void release_plan(cdc_ctx* ctx) {  // every op sequence and the workspace they run on
     for (Seq* q : {&ctx->step_seq, &ctx->ctx_seq, &ctx->enc_seq, &ctx->henc_seq, &ctx->hdec_seq}) *q = Seq();
+    byte_codec_release_buffers(ctx->byte_codec);
     ctx->arena.release();
 }
 
@@ -1749,7 +1740,7 @@ int cdc_hyper_decode(cdc_ctx* ctx, const float* z_hat, float* mu, float* sigma, 
     const Act& o = ctx->hdec_out;
     const int Cl = o.C / 2, HW = o.H * o.W;
     CK(launch_nhwc_slice_to_nchw_f32(o.p, mu, ctx->B, Cl, HW, o.C, 0, 0.0f, 0, S(s)));
-    CK(launch_nhwc_slice_to_nchw_f32(o.p, sigma, ctx->B, Cl, HW, o.C, Cl, 0.11f, 1, S(s)));  // sigma = max(sigma_raw, 0.11)
+    CK(launch_nhwc_slice_to_nchw_f32(o.p, sigma, ctx->B, Cl, HW, o.C, Cl, kMinSigma, 1, S(s)));  // sigma = max(sigma_raw, 0.11)
     return CDC_OK;
 }
 
@@ -1939,6 +1930,53 @@ int cdc_decode_host_seeded(cdc_ctx* ctx, const float* latent_host, float gamma, 
     if (!ctx->seeded) return ctx->fail(CDC_ERR_STATE, "cdc_decode_host_seeded: no per-image seeds bound (cdc_set_image_seeds)");
     return decode_host(ctx, latent_host, nullptr, gamma, image_host, s);
 }
+
+}  // extern "C"
+
+// ---- what bitstream.cu (cdc_compress_rgb8 / cdc_decompress_rgb8) sees of a context (codec_io.cuh) ----
+namespace cdc {
+int bound_codec(cdc_ctx* ctx, BoundCodec* out) {
+    NEED_PLAN();
+    NEED_CODEC();
+    BoundCodec v;
+    v.B = ctx->B;
+    v.H = ctx->H;
+    v.W = ctx->W;
+    v.latent_ch = ctx->cfg.latent_ch;
+    v.num_sms = ctx->num_sms;
+    v.device = ctx->device;
+    v.K = ctx->K;
+    v.has_ctx = ctx->has_ctx;
+    v.seeded = ctx->seeded;
+    v.graph_skip = ctx->graph_skip != 0;
+    v.img64 = ctx->img64.p;
+    v.enc_y = ctx->enc_y.p;
+    v.hdec_in = ctx->hdec_in.p;
+    v.hdec_out = ctx->hdec_out.p;
+    v.latent = ctx->latent.p;
+    v.xs = ctx->xs;
+    v.state = &ctx->byte_codec;
+    *out = v;
+    return CDC_OK;
+}
+ByteCodec** byte_codec_slot(cdc_ctx* ctx) { return &ctx->byte_codec; }
+int ctx_device(cdc_ctx* ctx) { return ctx->device; }
+int ctx_latent_ch(cdc_ctx* ctx) { return ctx->cfg.latent_ch; }
+int run_codec_seq(cdc_ctx* ctx, CodecSeq q, cudaStream_t s) {
+    return run_ops(ctx, q == CODEC_SEQ_ENCODER ? ctx->enc_seq : q == CODEC_SEQ_HYPER_DEC ? ctx->hdec_seq : ctx->ctx_seq, s);
+}
+int ctx_fail(cdc_ctx* ctx, int code, const char* fmt, ...) {
+    char buf[512];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    va_end(ap);
+    ctx->err = buf;
+    return code;
+}
+}  // namespace cdc
+
+extern "C" {
 
 static int count_kernels(const std::vector<Op>& ops) {  // the GroupNorm-slot memset node is not a kernel of ours
     int n = 0;

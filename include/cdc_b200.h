@@ -33,7 +33,8 @@ typedef enum {
     CDC_ERR_CUDA = -3,
     CDC_ERR_UNIMPLEMENTED = -4,
     CDC_ERR_STATE = -5,
-    CDC_ERR_WEIGHT = -6
+    CDC_ERR_WEIGHT = -6,
+    CDC_ERR_DATA = -7 /* the bytes are not a valid CDC5 stream for this context */
 } cdc_status;
 
 /* oracle/config.py CDCConfig */
@@ -170,6 +171,35 @@ int cdc_rans_encode(const int32_t* idx, const int32_t* v, const int32_t* lo, con
 int cdc_rans_decode(const uint8_t* data, int64_t data_bytes, const int32_t* idx, const int32_t* cdf, const int32_t* row_start,
                     const int32_t* cdf_length, const int32_t* offset, int rows, int64_t n_chan, int64_t hw, int spc,
                     void* scratch, int32_t* q, int32_t* status_dev, cdc_stream s);
+
+/* ---- the codec at the byte boundary: 8-bit RGB image <-> CDC5 stream, one call each (Codec.compress / decompress_bytes) --
+ * CDC5 = "CDC5" | u32 B, H, W | u64 nz | z container (nz bytes, cdc_rans_*) | y container; seeds and steps are not in it.
+ * Images are host [B][H][W][3] uint8, interleaved RGB.  Host buffers work as in cdc_decode_host: page-locked ones are
+ * copied directly, pageable ones through pinned staging; a device pointer is CDC_ERR_SHAPE.  The work buffers are
+ * allocated on the first compress / decompress for the bound shape and freed with it.  Every byte of a stream is checked
+ * on the host before anything runs on it: a stream that does not parse for this context is CDC_ERR_DATA, as is one whose
+ * rANS payload does not decode (found on the device; the decode then stops before the diffusion steps). */
+/* Entropy tables, host arrays in the layout of entropy_tables.Tables (cdf[n_cdf]; row_start, cdf_length, offset [rows]);
+ * copied to the device and validated (row_start + cdf_length inside n_cdf, cdf_length >= 2).
+ * which = 0: Gaussian, 64 <= rows <= 256 (row = scale-table entry), scale_table[64], median NULL.
+ * which = 1: factorised prior, latent_ch <= rows <= 256 (row = channel), scale_table NULL, median[latent_ch] (NULL: zeros). */
+int cdc_set_entropy_tables(cdc_ctx* ctx, int which, const int32_t* cdf, int64_t n_cdf, const int32_t* row_start,
+                           const int32_t* cdf_length, const int32_t* offset, int rows, const float* scale_table,
+                           const float* median);
+/* Host-only parse of a CDC5 stream (no CUDA call): B, H, W, so the caller can cdc_bind_io.  CDC_ERR_DATA if the header,
+ * either container header or a size table is malformed or points past the end. */
+int cdc_stream_info(const uint8_t* data_host, int64_t nbytes, int* B, int* H, int* W);
+/* Largest stream cdc_compress_rgb8 can write for the bound shape: 24 + both containers' cdc_rans_max_bytes (< 0: error) */
+int64_t cdc_compress_max_bytes(cdc_ctx* ctx);
+/* rgb_host [B][H][W][3] uint8 of the bound shape -> the CDC5 stream in out_host, byte-identical to Codec.compress(rgb / 255),
+ * and its size in *nbytes.  Needs both tables.  CDC_ERR_SHAPE if capacity < *nbytes (which still reports the size needed).
+ * Synchronises s. */
+int cdc_compress_rgb8(cdc_ctx* ctx, const uint8_t* rgb_host, uint8_t* out_host, int64_t capacity, int64_t* nbytes, cdc_stream s);
+/* CDC5 stream -> rgb_host [B][H][W][3] uint8 = round_half_even(255 * (clamp(x,-1,1)+1)/2) of the decode of its latent with
+ * the set schedule and the bound per-image seeds (x_T = gamma * z; CDC_ERR_STATE without seeds, as cdc_decode_host_seeded),
+ * i.e. Decoder.decode(Codec.decompress_bytes(...), seeds=...) in 8 bits.  The stream's B, H, W must be the bound shape
+ * (CDC_ERR_SHAPE).  Needs both tables and the context net.  Synchronises s. */
+int cdc_decompress_rgb8(cdc_ctx* ctx, const uint8_t* data_host, int64_t nbytes, float gamma, uint8_t* rgb_host, cdc_stream s);
 
 #ifdef __cplusplus
 }
