@@ -25,7 +25,7 @@ TOOLS_SYMBOLS = [
     "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn", "cdc_step_op_describe",
     "cdc_seq_num_ops", "cdc_seq_op_name", "cdc_seq_op_flops", "cdc_seq_op_bytes", "cdc_seq_op_describe", "cdc_run_seq_op",
 ]
-OPT_FUSE_APPLY, OPT_KF = range(2)
+OPT_FUSE_APPLY, OPT_KF, OPT_PLAN_SMS = range(3)
 OPK_MEMSET, OPK_CONV, OPK_GN_STATS, OPK_GN_APPLY, OPK_ATTENTION = range(5)  # cdc_op_kind
 SEQ_STEP, SEQ_CONTEXT, SEQ_ENCODER, SEQ_HYPER_ENC, SEQ_HYPER_DEC = range(5)  # cdc_seq
 
@@ -48,7 +48,9 @@ class StepOpDesc(C.Structure):
                 ("xk16", C.c_int32), ("tr", C.c_int32), ("res1", C.c_int32), ("apply", C.c_int32),
                 ("src", TensorDesc * 2), ("residual", TensorDesc), ("out", TensorDesc), ("res_out", TensorDesc),
                 ("gn_in_acc", C.c_void_p), ("gn_out_acc", C.c_void_p), ("gn_slots", C.c_int32),
-                ("x", C.c_void_p), ("x0_out", C.c_void_p), ("xpad", C.c_void_p), ("act_slope", C.c_float)]
+                ("x", C.c_void_p), ("x0_out", C.c_void_p), ("xpad", C.c_void_p), ("act_slope", C.c_float),
+                ("n_tiles", C.c_int32), ("g1", C.c_int32), ("nseg", C.c_int32), ("strips", C.c_int32), ("rows", C.c_int32),
+                ("grid", C.c_int32)]
 
 
 _libs = {}

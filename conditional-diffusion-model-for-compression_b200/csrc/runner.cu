@@ -31,9 +31,11 @@ static std::string g_create_err;
 
 // Planner decisions that tests / tools A/B through cdc_set_plan_option (include/cdc_b200_tools.h).
 struct PlanOpts {
-    int v[CDC_OPT_COUNT] = {2, 1};
+    int v[CDC_OPT_COUNT] = {2, 1, 0};
     int fuse_apply_max_tiles() const { return v[CDC_OPT_FUSE_APPLY]; }
     bool kf() const { return v[CDC_OPT_KF] != 0; }
+    // SMs the plan lays its grids out for: the device's count unless CDC_OPT_PLAN_SMS asks for fewer
+    int plan_sms(int device_sms) const { return v[CDC_OPT_PLAN_SMS] > 0 && v[CDC_OPT_PLAN_SMS] < device_sms ? v[CDC_OPT_PLAN_SMS] : device_sms; }
 };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -373,6 +375,12 @@ static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, in
     d.tr = kg.tr;
     d.res1 = kg.res;
     d.apply = kg.apply;
+    d.n_tiles = kg.n_tiles;
+    d.g1 = kg.G1;
+    d.nseg = kg.nseg;
+    d.strips = kg.S;
+    d.rows = kp->H;
+    d.grid = kg.n_tiles * kg.G1;
     if (kg.res) d.res_out = tensor_desc(cb.res_out);
     if (kg.apply) {
         d.gn_in_acc = const_cast<gn_sum_t*>(cb.in_acc);
@@ -526,6 +534,9 @@ static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, int gw,
     const SamplerTab* samp = cb.samp;
     op->desc.kernel = 1;
     op->desc.bn = bn;
+    const long total = m_tiles * (w.n_pad / bn);  // (launch_conv's grid: conv_tc.cu launch_one)
+    op->desc.n_tiles = static_cast<int>(total);
+    op->desc.grid = static_cast<int>(total < num_sms ? total : num_sms);
     op->run = [cp, bn, cpg, epi, num_sms, samp](cudaStream_t s, int k, long long* stamp) -> cudaError_t {
         ConvParams q = *cp;
         q.stamp = stamp;
@@ -608,6 +619,9 @@ struct WeightT {
 };
 
 constexpr int kMaxGnSlots = 64;  // GroupNorms per sequence (37 in a denoise step, 8 in the context net)
+// Largest batch a plan can run: gn_apply_kernel keeps every image's 32 (mean, rstd) float2 pairs in dynamic shared
+// memory without the opt-in beyond 48 KB (launch_gn_apply refuses more).  Nothing else limits the batch below this.
+constexpr int kMaxBatch = 48 * 1024 / (32 * 8);
 
 struct Seq {  // one op sequence of the plan
     std::vector<Op> ops;
@@ -839,7 +853,7 @@ struct PlanB {
         if (rc) return op;
         std::string e;
         cb.sat = ctx->sat_dev;
-        int r = build_conv(cb, ctx->B, ctx->num_sms, ctx->opts, &op, &e);
+        int r = build_conv(cb, ctx->B, ctx->opts.plan_sms(ctx->num_sms), ctx->opts, &op, &e);
         if (r) {
             rc = ctx->fail(r, "%s", e.c_str());
             return op;
@@ -870,15 +884,16 @@ struct PlanB {
         const float* beta = find_w(c, gnp + ".bias")->p;
         const int Cc = x.C, HW = x.H * x.W, B = c->B;
         const int foff = film_idx >= 0 ? c->film_off[film_idx] : -1;
+        const int sms = c->opts.plan_sms(c->num_sms);
         Op a;
         a.name = name + (silu ? ".apply_silu" : ".apply") + (res ? "_res" : "");
         a.bytes = static_cast<double>(B) * HW * Cc * 2 * (res ? 3 : 2);
         const act_t *xp = x.p, *rp = res;
         act_t* yp = y.p;
         const int si = silu ? 1 : 0;
-        a.run = [c, acc, gamma, beta, foff, xp, rp, yp, B, HW, Cc, si](cudaStream_t s, int k, long long* stamp) {
+        a.run = [c, acc, gamma, beta, foff, xp, rp, yp, B, HW, Cc, si, sms](cudaStream_t s, int k, long long* stamp) {
             const float* film = foff >= 0 ? c->film + static_cast<size_t>(k) * c->film_total + foff : nullptr;
-            return launch_gn_apply(xp, acc, gamma, beta, film, c->cfg.gn_eps, rp, yp, B, HW, Cc, si, c->num_sms, s, stamp, c->sat_dev);
+            return launch_gn_apply(xp, acc, gamma, beta, film, c->cfg.gn_eps, rp, yp, B, HW, Cc, si, sms, s, stamp, c->sat_dev);
         };
         cdc_step_op_desc& d = a.desc;
         d.kind = CDC_OPK_GN_APPLY;
@@ -1638,6 +1653,8 @@ static void release_plan(cdc_ctx* ctx) {  // every op sequence and the workspace
 int cdc_bind_io(cdc_ctx* ctx, int B, int H, int W) {
     if (!ctx || !ctx->finalized) return ctx ? ctx->fail(CDC_ERR_STATE, "finalize weights first") : CDC_ERR_STATE;
     if (B < 1 || H < 64 || W < 64 || (H % 64) || (W % 64)) return ctx->fail(CDC_ERR_SHAPE, "H and W must be multiples of 64, batch >= 1");
+    if (B > kMaxBatch)
+        return ctx->fail(CDC_ERR_SHAPE, "batch %d > %d: the GroupNorm apply kernel holds every image's statistics table in 48 KB of shared memory", B, kMaxBatch);
     if (B == ctx->B && H == ctx->H && W == ctx->W && !ctx->step_seq.ops.empty() && !ctx->opts_dirty) return CDC_OK;
     GUARD();
     CK(cudaDeviceSynchronize());

@@ -150,6 +150,7 @@ class Decoder:
 
     def bind(self, B, H, W):
         if self.shape != (B, H, W):
+            self.shape = None  # (a refused bind leaves nothing bound)
             with torch.cuda.device(self.device):
                 self._ck(self.L.cdc_bind_io(self.ctx, B, H, W), "cdc_bind_io")
             self.shape = (B, H, W)

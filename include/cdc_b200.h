@@ -81,7 +81,9 @@ int cdc_schedule_coeffs5(cdc_ctx* ctx, int k, float* c0, float* c1, float* e0, f
 int cdc_film_size(cdc_ctx* ctx);
 int cdc_get_film(cdc_ctx* ctx, float* film_dev, cdc_stream s);
 
-/* ---- shape binding: allocates the workspace arena, builds tensor maps and the launch plan ------ */
+/* ---- shape binding: allocates the workspace arena, builds tensor maps and the launch plan ------
+ * batch 1 .. 192 (CDC_ERR_SHAPE beyond: the GroupNorm apply kernel holds every image's statistics table in 48 KB of
+ * shared memory); height and width multiples of 64. */
 int cdc_bind_io(cdc_ctx* ctx, int batch, int height, int width);
 int cdc_set_cond(cdc_ctx* ctx, const float* c0, const float* c1, const float* c2, const float* c3, cdc_stream s);
 int cdc_set_latent(cdc_ctx* ctx, const float* y_hat, cdc_stream s); /* runs the context net: cond = context_net(y_hat) */

@@ -22,7 +22,10 @@ extern "C" {
 typedef enum {
     CDC_OPT_FUSE_APPLY = 0,     /* N tiles a conv may have for the input-GroupNorm fusion; 0 = never fuse.  default 2 */
     CDC_OPT_KF = 1,             /* 0: every conv through the general kernel (conv_tc.cu).  default 1 */
-    CDC_OPT_COUNT = 2
+    CDC_OPT_PLAN_SMS = 2,       /* SMs the conv grids and the GroupNorm apply grid are laid out for; 0 (default) or more
+                                   than the device has: the device's count.  A test lever: a few SMs put several strips
+                                   (and images) on one strip-conv CTA at small shapes */
+    CDC_OPT_COUNT = 3
 } cdc_plan_option;
 int cdc_set_plan_option(cdc_ctx* ctx, int option, int value);
 
@@ -85,6 +88,12 @@ typedef struct {
     float* x0_out;       /* final conv: x0 estimate, NHWC fp32 */
     void* xpad;          /* final conv: the stem's 16-bit x_t copy, rewritten with x_prev */
     float act_slope;     /* conv: LeakyReLU slope applied after the bias (the hyper networks' 0.2), 0: none */
+    /* conv launch geometry.  conv_kf.cu: n_tiles N tiles (output-parity tiles included) of g1 CTAs each; the kernel-space
+     * grid (image rows, or image columns for the transposed walk) has `rows` rows, split into nseg 128-pixel segment
+     * columns per image and `strips` strips per column; CTA c of a tile runs the units (image, segment, strip)
+     * u = c, c + g1, ... < B * nseg * strips.  conv_tc.cu: n_tiles output tiles (N tiles x phases x images x pixel
+     * tiles) over `grid` persistent CTAs (g1, nseg, strips, rows 0).  grid: CTAs launched (both kernels). */
+    int n_tiles, g1, nseg, strips, rows, grid;
 } cdc_step_op_desc;
 int cdc_seq_op_describe(cdc_ctx* ctx, int seq, int i, cdc_step_op_desc* out);
 int cdc_step_op_describe(cdc_ctx* ctx, int i, cdc_step_op_desc* out);  /* CDC_SEQ_STEP */

@@ -61,6 +61,73 @@ def _inst(d):
             f"res1{d.res1} apply{d.apply} tr{d.tr}")
 
 
+def image_scale(B):
+    """Per-image input scale 2^((b mod 4) - 1), [B, 1, 1, 1]: every image of a batch gets its own GroupNorm statistics (a
+    kernel that used another image's would be off by a factor, not by sampling noise), and a power of two keeps the
+    synthetic inputs exact."""
+    return (2.0 ** (torch.arange(B, dtype=torch.float64) % 4 - 1)).float().reshape(B, 1, 1, 1)
+
+
+def kf_acc_ring(key):
+    """Accumulator-ring length (logical slots) of the conv_kf.cu instantiation key (_kf_key): 6 with the fused residual
+    conv or the aliased ring of the 64-column tiles (BN = 32 with the residual conv likewise), else min(16, 512 / BN)."""
+    bn, _, epi, _, _, _, mode, res1, _ = key
+    alias = mode == 0 and epi != 2 and ((bn == 64 and not res1) or (bn == 32 and res1))
+    return 6 if res1 or alias else min(16, 512 // bn)
+
+
+def kf_geometry(d, B):
+    """Which parts of the strip kernel's unit loop a conv_kf.cu op (description d, batch B) runs: a set of
+    "several_units" (a CTA runs more than one unit), "two_images" (one CTA's units belong to two images), "one_row"
+    (strips of one row), "uneven" (strips of unequal length), "ragged" (the last 128-pixel segment is partly outside the
+    image) and "ring_wrap" (a strip is longer than the accumulator ring).  From the launch geometry of the description."""
+    units, per_img = B * d.nseg * d.strips, d.nseg * d.strips
+    f = set()
+    if units > d.g1:
+        f.add("several_units")
+        if any(len({u // per_img for u in range(c, units, d.g1)}) > 1 for c in range(d.g1)):
+            f.add("two_images")
+    if d.strips == d.rows:
+        f.add("one_row")
+    if d.rows % d.strips:
+        f.add("uneven")
+    s2 = d.mode == 1  # stride 2: the kernel walks the output grid
+    cols = (d.src[0].H if d.tr else d.src[0].W) >> (1 if s2 else 0)
+    if cols % 128:
+        f.add("ragged")
+    if -(-d.rows // d.strips) > kf_acc_ring(_kf_key(d)):
+        f.add("ring_wrap")
+    return f
+
+
+class GeometrySeen:
+    """The launch geometry of the checked conv ops: kf_geometry per conv_kf.cu instantiation and per (walk, MODE), and the
+    conv_tc.cu instantiations that ran more tiles than CTAs."""
+
+    def __init__(self):
+        self.kf, self.cls, self.tc_waves = {}, set(), set()
+
+    def add(self, d, B):
+        if d.kind != 1:
+            return
+        if d.kernel == 2:
+            geo = kf_geometry(d, B)
+            self.kf.setdefault(_kf_key(d), set()).update(geo)
+            self.cls.update(((d.tr, _kf_key(d)[6]), g) for g in geo)
+        elif d.n_tiles > d.grid:
+            self.tc_waves.add((d.bn, d.cpg, d.epi))
+
+
+def _geom(d, B):
+    """The launch geometry of conv op d, for the per-op listings."""
+    if d.kind != 1:
+        return ""
+    if d.kernel == 1:
+        return f"{d.n_tiles} tiles / {d.grid} CTAs"
+    return (f"{B * d.nseg * d.strips} units / {d.g1} CTAs x {d.n_tiles} tiles, {d.nseg} seg, {d.strips} strips of "
+            f"{d.rows} rows")
+
+
 def fixed_point_(module):
     """Every conv (and transposed-conv) weight of module on a per-layer grid 2^-m, m the largest with
     4 * max|w| * 2^m < 2^11: the weights and every sum of four of them (the nearest-x2 parity weights) are exact in fp16."""
@@ -266,8 +333,13 @@ def _check_conv(st, d, snap, k):
         xp = c0 * x0.clamp(-1.0, 1.0) + c1 * xt
         tol = abs(c0) * tol_x0 + 2 * U32 * (abs(c0) * x0.abs().clamp(max=1.0) + abs(c1) * xt.abs()) + 1e-30
         if sg != 0.0:
-            from oracle.sampler import philox_normal
-            z = _nhwc(philox_normal(st.seed, k, st.B, st.H, st.W_).double().to(DEV))
+            if getattr(st, "image_seeds", None):  # per-image seeds bound (cdc_set_image_seeds)
+                from tests.seeded_reference import philox_normal_images, step_plane
+                z = philox_normal_images(st.image_seeds, *step_plane(k), st.H, st.W_)
+            else:
+                from oracle.sampler import philox_normal
+                z = philox_normal(st.seed, k, st.B, st.H, st.W_)
+            z = _nhwc(z.double().to(DEV))
             xp = xp + sg * z
             tol = tol + sg * 2.0 ** -18 * (z.abs() + 1.0)  # fp32 logf / sqrtf / sincospif of the Box-Muller pair
         got_x = st.views[d.x].double()

@@ -12,15 +12,18 @@ with the same bits in every buffer as the entry left: the entry runs exactly the
 The sequences decide the bitstream (y, z, and from z_hat the mu / sigma of every y symbol, on both sides of the stream),
 and they run code the denoise step never takes: the 5x5 stride-2 convs, the 5x5 transposed convs, the LeakyReLU epilogue,
 the 256 -> 512 output conv, the encoder's strip-kernel instantiations, and the input GroupNorm without FiLM.
+
+With B > 1, image b's input is scaled by 2^((b mod 4) - 1) (per-image GroupNorm statistics), and the coverage test
+requires the strip kernel's unit-loop regimes of tests/test_gpu_step_ops.py check_geometry_coverage here too.
 """
 import time
 
 import pytest
 import torch
 
-from tests.op_reference import (DEV, SeqBuffers, _bits, _check_conv, _check_gn_apply, _check_gn_stats, _fixed_point_unet,
-                                _inst, _kf_key, _nhwc, _view, fixed_point_)
-from tests.test_gpu_step_ops import KF_NOT_IN_STEP
+from tests.op_reference import (DEV, GeometrySeen, SeqBuffers, _bits, _check_conv, _check_gn_apply, _check_gn_stats,
+                                _fixed_point_unet, _geom, _inst, _kf_key, _nhwc, _view, fixed_point_, image_scale)
+from tests.test_gpu_step_ops import KF_NOT_IN_STEP, check_geometry_coverage
 
 pytestmark = pytest.mark.gpu
 
@@ -36,12 +39,19 @@ CONFIGS = [
     ("context_three_images_64x128", CONTEXT, (3, 64, 128), {}),
     ("context_tall_64x1024", CONTEXT, (1, 1024, 64), {}),  # the strip kernel's transposed walk
     ("context_general_kernel_768x512", CONTEXT, (1, 512, 768), {"OPT_KF": 0}),
+    ("context_2048x2048", CONTEXT, (1, 2048, 2048), {}),
+    ("context_16x256x256", CONTEXT, (16, 256, 256), {}),
+    ("context_one_row_64x1024", CONTEXT, (1, 64, 1024), {}),
+    # planned for a few SMs: several units per CTA, of two images, for every strip instantiation
+    ("context_plan_sms4_2x64x1024", CONTEXT, (2, 64, 1024), {"OPT_PLAN_SMS": 4}),
+    ("context_plan_sms4_2x384x128", CONTEXT, (2, 384, 128), {"OPT_PLAN_SMS": 4}),  # the transposed walk
     ("encoder_64x64", ENCODER, (1, 64, 64), {}),
     ("encoder_three_images_64x128", ENCODER, (3, 64, 128), {}),
     ("encoder_two_images_192x256", ENCODER, (2, 192, 256), {}),
     ("encoder_tall_64x1024", ENCODER, (1, 1024, 64), {}),
     ("encoder_768x512", ENCODER, (1, 512, 768), {}),
     ("encoder_2048x2048", ENCODER, (1, 2048, 2048), {}),
+    ("encoder_plan_sms4_2x64x1024", ENCODER, (2, 64, 1024), {"OPT_PLAN_SMS": 4}),  # the encoder's own instantiations
     ("hyper_enc_64x64", HYPER_ENC, (1, 64, 64), {}),  # z is 1 x 1: every tap reads padding or sits at an edge
     ("hyper_enc_two_images_192x256", HYPER_ENC, (2, 192, 256), {}),
     ("hyper_enc_1024x64", HYPER_ENC, (1, 64, 1024), {}),  # z 1 x 16
@@ -54,6 +64,7 @@ CONFIGS = [
 
 _cache = {}
 _seen, _done = set(), set()
+_geo = GeometrySeen()
 
 
 def _setup():
@@ -93,16 +104,18 @@ class _Seq(SeqBuffers):
 
 
 def _driven_input(seq, B, H, W):
-    """The caller's input of the sequence's public entry (NCHW fp32, host)."""
+    """The caller's input of the sequence's public entry (NCHW fp32, host); image b scaled by image_scale when B > 1."""
     from oracle.weights import synthetic_image, synthetic_latent
     g = torch.Generator().manual_seed(17)
     if seq == CONTEXT:
-        return synthetic_latent(B, H, W)
-    if seq == ENCODER:
-        return synthetic_image(B, H, W, index=3)
-    if seq == HYPER_ENC:  # y of realistic magnitude, bf16-exact
-        return (8.0 * torch.randn(B, 256, H // 16, W // 16, generator=g)).bfloat16().float()
-    return torch.round(4.0 * torch.randn(B, 256, H // 64, W // 64, generator=g))  # z_hat
+        x = synthetic_latent(B, H, W)
+    elif seq == ENCODER:
+        x = synthetic_image(B, H, W, index=3)
+    elif seq == HYPER_ENC:  # y of realistic magnitude, bf16-exact
+        x = (8.0 * torch.randn(B, 256, H // 16, W // 16, generator=g)).bfloat16().float()
+    else:
+        x = torch.round(4.0 * torch.randn(B, 256, H // 64, W // 64, generator=g))  # z_hat
+    return x * image_scale(B) if B > 1 else x
 
 
 def _entry(dec, codec, seq, x):
@@ -180,6 +193,7 @@ def test_codec_ops_match_float64(cfg):
     t0 = time.perf_counter()
     ocfg, dec, codec, W = _setup()
     dec.set_plan_option(_ffi.OPT_KF, opts.get("OPT_KF", 1))
+    dec.set_plan_option(_ffi.OPT_PLAN_SMS, opts.get("OPT_PLAN_SMS", 0))
     B, H, Wd = shape
     x = _driven_input(seq, B, H, Wd)
     dec.bind(B, H, Wd)
@@ -211,7 +225,7 @@ def test_codec_ops_match_float64(cfg):
         else:
             pytest.fail(f"{op}: op kind {d.kind} has no float64 reference here")
         shown = " ".join(f"{key}={val:.3g}" for key, val in worst.items())
-        print(f"[{name}] {i:3d} {op:32s} {_inst(d):84s} {shown}")
+        print(f"[{name}] {i:3d} {op:32s} {_inst(d):84s} {shown}  [{_geom(d, B)}]")
         for key, val in worst.items():
             if key == "err/S":
                 worst_s = max(worst_s, (val, op))
@@ -220,6 +234,7 @@ def test_codec_ops_match_float64(cfg):
                 if not val <= 1.0:
                     bad.append(f"op {i} {op} ({_inst(d)}): {key} err/tol = {val:.3g}")
         _seen.update(_features(d))
+        _geo.add(d, B)
         st.advance(d, snap)
     for p, v in st.views.items():
         assert _same_bits(v, entry[p]), f"{name}: the op-by-op replay left other bits than the public entry"
@@ -281,3 +296,5 @@ def test_codec_op_coverage():
     assert len(want) == 2, "KF_NOT_IN_STEP names the encoder's two strip instantiations"
     want |= {"kf apply without FiLM", "gn_apply without FiLM", ("tc", 1, 5), ("tc", 3, 5), ("slope", 0.2)}
     assert want <= _seen, f"never checked: {sorted(map(str, want - _seen))}"
+    # every strip instantiation the codec sequences ran, in the unit-loop regimes the step's coverage test requires
+    check_geometry_coverage(set(_geo.kf), _geo)

@@ -164,6 +164,21 @@ def test_wrong_shapes_fail_loudly():
         dec.bind(1, 100, 256)
 
 
+def test_batch_beyond_the_groupnorm_table_is_refused_at_bind():
+    """193 images need a 49 KB GroupNorm statistics table: cdc_bind_io refuses the batch (instead of a later CUDA error
+    from the first step), and the context then binds and decodes a valid shape as a fresh one does."""
+    from cdc_b200 import CDCConfig, Decoder
+    from cdc_b200.synthetic import init_noise, latent, random_weights
+    w = random_weights(CDCConfig(), seed=0, with_context=True)
+    a = Decoder(CDCConfig(), w, device=DEV)
+    a.bind(2, 64, 128)
+    with pytest.raises(RuntimeError, match="GroupNorm"):
+        a.bind(193, 64, 64)
+    out = a.decode(latent(2, 64, 128, index=1), 3, init=init_noise(2, 64, 128, index=1))
+    ref = Decoder(CDCConfig(), w, device=DEV).decode(latent(2, 64, 128, index=1), 3, init=init_noise(2, 64, 128, index=1))
+    assert torch.isfinite(ref).all() and torch.equal(out, ref)
+
+
 def test_rebinding_shapes_and_schedules_is_stateless():
     """One context decodes different shapes / step counts back to back (workspace, tensor maps, pinned staging and the
     graph are rebuilt); every result equals the one a fresh context produces."""
