@@ -10,8 +10,9 @@ LIB_PATH = os.environ.get("CDC_LIB_PATH") or os.path.join(_HERE, "libcdc_b200.so
 SYMBOLS = [
     "cdc_create", "cdc_destroy", "cdc_last_error", "cdc_abi_version", "cdc_act_dtype", "cdc_load_weights", "cdc_finalize_weights",
     "cdc_has_context_net", "cdc_set_schedule", "cdc_schedule_index", "cdc_schedule_coeffs", "cdc_set_sampler",
-    "cdc_schedule_coeffs5", "cdc_film_size", "cdc_get_film", "cdc_bind_io", "cdc_set_cond", "cdc_get_cond", "cdc_set_latent",
-    "cdc_set_x", "cdc_get_x", "cdc_get_x0", "cdc_denoise_step", "cdc_decode", "cdc_decode_trajectory", "cdc_trajectory_wait",
+    "cdc_schedule_coeffs5", "cdc_film_size", "cdc_get_film", "cdc_bind_io", "cdc_set_batch_invariant", "cdc_set_cond",
+    "cdc_get_cond", "cdc_set_latent", "cdc_set_x", "cdc_get_x", "cdc_get_x0", "cdc_denoise_step", "cdc_decode",
+    "cdc_decode_trajectory", "cdc_trajectory_wait",
     "cdc_decode_host", "cdc_set_image_seeds", "cdc_init_noise", "cdc_decode_host_seeded", "cdc_launches_per_step",
     "cdc_launches_context", "cdc_flops_per_step", "cdc_saturation_count", "cdc_quantize", "cdc_cdf_lookup",
     "cdc_has_codec", "cdc_encode_analysis", "cdc_hyper_encode", "cdc_hyper_decode",
@@ -89,6 +90,7 @@ def _bind(L):
     L.cdc_film_size.argtypes = [p]
     L.cdc_get_film.argtypes = [p, f32p, p]
     L.cdc_bind_io.argtypes = [p, i32, i32, i32]
+    L.cdc_set_batch_invariant.argtypes = [p, i32]
     L.cdc_set_cond.argtypes = [p, f32p, f32p, f32p, f32p, p]
     L.cdc_get_cond.argtypes = [p, f32p, f32p, f32p, f32p, p]
     L.cdc_set_latent.argtypes = [p, f32p, p]

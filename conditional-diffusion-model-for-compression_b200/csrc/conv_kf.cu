@@ -84,6 +84,15 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
     // its epilogue, already at the register limit, spills on the second load: 47.6 -> 49.7 us; it keeps 6 + 2 residual slots.
     constexpr bool ALIAS = MODE == 0 && EPI != EPI_DDIM && ((BN == 64 && !RES1) || (BN == 32 && RES1));
     constexpr uint32_t NALIAS = ALIAS ? 2 : 0;
+    // With ALIAS the logical slot of an output row is numerics, not just storage: rows in logical slots 0 and 1 receive
+    // some taps in their second home, and the two partial sums are added in the epilogue.  So a strip's results depend on
+    // (g mod NACC) at its start, i.e. on how many rows its CTA ran before it.  p.slot0 makes every strip start at slot 0:
+    // between strips all three roles advance g to the next multiple of NACC through PHANTOM rows -- no MMA, no TMEM access,
+    // but every barrier phase of a real row (the issuer waits "drained" and arrives "complete", the epilogue waits
+    // "complete" and arrives "drained"; the producer, which waits "drained" only to reuse TMEM, just counts them), so
+    // every (g / NACC) & 1 parity stays right.  Elsewhere the slot is storage only: a window that wraps is split along N,
+    // and every output element still sums the same products in the same order.
+    const bool slot0 = ALIAS && p.slot0 != 0;
     constexpr uint32_t NACC = RES1 ? 6 : ALIAS ? 6 : (512 / BN < kKfAccMax ? 512 / BN : kKfAccMax);
     constexpr int TMEM_COLS = (NACC + NALIAS + NRES) * BN <= 128 ? 128 : (NACC + NALIAS + NRES) * BN <= 256 ? 256 : 512;  // power of two
     static_assert(!RES1 || (MODE == 0 && !STAGE && EPI != EPI_DDIM && (BN == 64 || BN == 32)), "fused residual conv: 3x3 stats/store convs");
@@ -222,6 +231,7 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
             uint32_t slot = 0, par = 0;  // ring position / fill parity (continues across strips)
             uint32_t g = 0;
             for (int u = cta; u < units; u += p.G1) {
+                if (slot0) g = (g + NACC - 1) / NACC * NACC;  // phantom rows (see ALIAS): counted, not waited for
                 int b, seg, si, h0, L;
                 decode(u, b, seg, si, h0, L);
                 const int w0 = seg * 128 - 1;
@@ -322,6 +332,19 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
             const uint32_t pin_word = aux + 460;
             auto pin = [&](uint32_t v) { asm volatile("st.shared.b32 [%0], %1;" ::"r"(pin_word), "r"(v) : "memory"); };
             for (int u = cta; u < units; u += p.G1) {
+                // phantom rows up to the next multiple of NACC (see ALIAS).  "Drained" is waited for before "complete" is
+                // arrived at, as for a real row, whose MMAs the producer only feeds after that wait: the epilogue has then
+                // consumed the slot's previous "complete" phase.  (The first strip starts at g = 0: nothing to do.)
+                if (slot0) {
+                    for (; g % NACC != 0; ++g) {
+                        mbar_wait(bar_tempty + 8 * (g % NACC), (g / NACC) & 1);
+                        mbar_arrive(bar_tfull + 8 * (g % NACC));
+                        if constexpr (RES1) {  // the fused 1x1 conv's ring is indexed by the same counter: its phases advance too
+                            mbar_wait(bar_xempty + 8 * (g % NRESD), (g / NRESD) & 1);
+                            mbar_arrive(bar_xfull + 8 * (g % NRESD));
+                        }
+                    }
+                }
                 int b, seg, si, h0, L;
                 decode(u, b, seg, si, h0, L);
                 const int nrows = MODE == 2 ? 2 * L + 1 : L + 2;
@@ -516,6 +539,16 @@ __global__ void __launch_bounds__(128 + kEpiThreads + (APPLY ? kKfXfExtra : 0), 
             for (int s_ = 0; s_ < static_cast<int>(NACC + NRES); ++s_)
                 mbar_arrive(s_ < static_cast<int>(NACC) ? bar_tempty + 8 * s_ : bar_xempty + 8 * (s_ - NACC));  // (barrier indices, not slots)
             for (int u = cta; u < units; u += p.G1, ++unit_ctr) {
+                if (slot0) {  // phantom rows (see ALIAS and the issuer): the slot keeps its armed bias, its second home its zeros
+                    for (; g % NACC != 0; ++g) {
+                        if constexpr (RES1) {
+                            mbar_wait(bar_xfull + 8 * (g % NRES), (g / NRES) & 1);
+                            mbar_arrive(bar_xempty + 8 * (g % NRES));
+                        }
+                        mbar_wait(bar_tfull + 8 * (g % NACC), (g / NACC) & 1);
+                        mbar_arrive(bar_tempty + 8 * (g % NACC));
+                    }
+                }
                 int b, seg, si, h0, L;
                 decode(u, b, seg, si, h0, L);
                 const int gx = seg * 128 + row;

@@ -15,6 +15,8 @@ struct alignas(64) KfParams {
     int H, W, batch;      // INPUT grid (mode 1: the low-resolution tensor; the output is 2H x 2W)
     int nseg;             // ceil(W / 128) column segments
     int S;                // strips per column (rows are spread evenly over them)
+    int slot0;            // 1: every strip starts at logical accumulator slot 0, however many strips its CTA ran before
+                          // (the aliased rings' sums then do not depend on the grid: batch-invariant plans)
     int NS;               // input-row ring slots
     int n_tiles;          // N tiles (mode 1: channel tiles x 4 parities); every CTA keeps ONE tile's weights resident
     int G1;               // CTAs per N tile (grid = n_tiles * G1)

@@ -36,6 +36,11 @@ struct PlanOpts {
     bool kf() const { return v[CDC_OPT_KF] != 0; }
     // SMs the plan lays its grids out for: the device's count unless CDC_OPT_PLAN_SMS asks for fewer
     int plan_sms(int device_sms) const { return v[CDC_OPT_PLAN_SMS] > 0 && v[CDC_OPT_PLAN_SMS] < device_sms ? v[CDC_OPT_PLAN_SMS] : device_sms; }
+    // cdc_set_batch_invariant: every op is laid out per image as for a batch of 1 (strip lengths, walk direction, N tiles),
+    // and the strip conv starts every strip at accumulator slot 0, so an image's bits do not depend on its batch
+    bool batch_invariant = false;
+    // the batch the geometry decisions are made for (the launch still covers all B images)
+    int plan_batch(int B) const { return batch_invariant ? 1 : B; }
 };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -256,16 +261,18 @@ static bool conv_uses_kf(const ConvBuild& cb, int B, int num_sms, const PlanOpts
     if (cb.epi == EPI_DDIM && g->n_tiles != 1) return false;
     // strip geometry for a walk along image rows (tr = 0) or image columns (tr = 1): relative cost = padding of the
     // 128-pixel segments x halo rows per strip; the transposed walk is used for unstaged kernels when it is >10 % cheaper
+    // (S is chosen for the plan batch; with a plan batch of 1 and B > 1 a CTA runs several strips, of any images)
     auto plan = [&](int w_, int h_, int* nseg, int* S, int* G1) {
         *nseg = (w_ + 127) / 128;
-        const int cols = B * *nseg;  // independent strip columns per N tile
+        const int cols = po.plan_batch(B) * *nseg;  // independent strip columns per N tile
         int g1 = num_sms / g->n_tiles;
         if (g1 < 1) g1 = 1;
         int s_ = g1 / cols;
         if (s_ < 1) s_ = 1;
         if (s_ > h_) s_ = h_;
         *S = s_;
-        *G1 = cols * s_ < g1 ? cols * s_ : g1;
+        const int units = B * *nseg * s_;
+        *G1 = units < g1 ? units : g1;
         const double L = static_cast<double>(h_) / s_;
         return (*nseg * 128.0 / w_) * (L + 2.0) / L;
     };
@@ -309,7 +316,7 @@ struct KfLaunch {
 };
 
 // The kh-fused strip kernel (conv_kf.cu) in geometry kg.  Returns an error message, or null.
-static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, int gw, int gh, Op* op) {
+static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, const PlanOpts& po, int gw, int gh, Op* op) {
     const ConvW& w = *cb.w;
     auto kp = std::shared_ptr<KfParams>(new KfParams());
     memset(kp.get(), 0, sizeof(KfParams));
@@ -338,6 +345,7 @@ static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, in
     kp->batch = B;
     kp->nseg = kg.nseg;
     kp->S = kg.S;
+    kp->slot0 = po.batch_invariant ? 1 : 0;
     kp->NS = kg.NS;
     kp->n_tiles = kg.n_tiles;
     kp->G1 = kg.G1;
@@ -399,7 +407,7 @@ static const char* plan_conv_kf(const ConvBuild& cb, const KfGeom& kg, int B, in
 }
 
 // The general implicit-GEMM kernel (conv_tc.cu).  Returns an error message, or null.
-static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, int gw, int gh, Op* op) {
+static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, const PlanOpts& po, int gw, int gh, Op* op) {
     const ConvW& w = *cb.w;
     const int ctot = w.c_pad;
     const bool x2 = cb.mode == MODE_UP2 || cb.mode == MODE_CONVT;  // four output phases, each on the input grid
@@ -418,8 +426,9 @@ static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, int gw,
     const int BW = 1 << bwl, BH = 128 >> bwl;
     const int tiles_w = (gw + BW - 1) / BW, tiles_h = (gh + BH - 1) / BH;
 
-    // N tile
+    // N tile (chosen for the plan batch; the grid covers all B images)
     const long m_tiles = static_cast<long>(nphase) * B * tiles_w * tiles_h;
+    const long m_tiles_plan = static_cast<long>(nphase) * po.plan_batch(B) * tiles_w * tiles_h;
     int bn = 0;
     if (cb.epi == EPI_DDIM) {
         bn = 16;
@@ -433,7 +442,7 @@ static const char* plan_conv_tc(const ConvBuild& cb, int B, int num_sms, int gw,
         for (int c : cands) {
             if (w.n_pad % c) continue;
             if (cb.epi == EPI_STATS && !stats_inst_ok(c, cb.cpg)) continue;
-            const long tiles = m_tiles * (w.n_pad / c);
+            const long tiles = m_tiles_plan * (w.n_pad / c);
             const long waves = (tiles + num_sms - 1) / num_sms;
             const double mma = 4.0 * (c / 2.0), mem = (16384.0 + c * 128.0) / 33.0;
             const double cost = static_cast<double>(waves) * (mma > mem ? mma : mem);
@@ -603,8 +612,8 @@ static int build_conv(const ConvBuild& cb, int B, int num_sms, const PlanOpts& p
                         : 2.0 * M * w.n_true * (static_cast<double>(taps) * w.c_true);
     op->bytes = 2.0 * (m_in * w.c_true + M * w.n_true + static_cast<double>(taps) * w.c_true * w.n_true);
     KfGeom kg;
-    const char* m = conv_uses_kf(cb, B, num_sms, po, &kg) ? plan_conv_kf(cb, kg, B, gw, gh, op)
-                                                          : plan_conv_tc(cb, B, num_sms, gw, gh, op);
+    const char* m = conv_uses_kf(cb, B, num_sms, po, &kg) ? plan_conv_kf(cb, kg, B, po, gw, gh, op)
+                                                          : plan_conv_tc(cb, B, num_sms, po, gw, gh, op);
     return m ? fail(m) : CDC_OK;
 }
 
@@ -1671,6 +1680,16 @@ int cdc_bind_io(cdc_ctx* ctx, int B, int H, int W) {
         return r;
     }
     CK(cudaDeviceSynchronize());
+    return CDC_OK;
+}
+
+int cdc_set_batch_invariant(cdc_ctx* ctx, int on) {
+    if (!ctx) return CDC_ERR_STATE;
+    if (on != 0 && on != 1) return ctx->fail(CDC_ERR_SHAPE, "cdc_set_batch_invariant: %d is neither 0 nor 1", on);
+    if (ctx->opts.batch_invariant != (on == 1)) {
+        ctx->opts.batch_invariant = on == 1;
+        ctx->opts_dirty = true;  // the next cdc_bind_io re-plans, also for the bound shape
+    }
     return CDC_OK;
 }
 

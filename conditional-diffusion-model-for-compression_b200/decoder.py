@@ -6,7 +6,7 @@ Same surface as oracle/sampler.py OracleDecoder (the reference ships no code, so
     decode(latent, steps, *, init=None, gamma=0.8, seed=0, trajectory=None), quantize_symbols, cdf_lookup;
 plus decode_progressive, a generator of per-step (x_t, x0_hat) previews while the decode runs, and per-image seeds
 (decode(..., seeds=[...]) / set_image_seeds): image b's x_T and sampler noise then depend on seeds[b] alone, so an image
-decodes to the same result in any batch.
+decodes to the same result in any batch -- bit for bit with Decoder(..., batch_invariant=True).
 Tensors at this surface are NCHW fp32 torch tensors; CUDA tensors are used in place, CPU tensors
 are staged through pinned memory by the library (cdc_decode_host).
 """
@@ -45,10 +45,13 @@ def _seed_values(seeds, n):
 
 
 class Decoder:
-    def __init__(self, cfg: CDCConfig, weights, device="cuda:0", tables=None, variant="product"):
+    def __init__(self, cfg: CDCConfig, weights, device="cuda:0", tables=None, variant="product", batch_invariant=False):
         """weights: dict name -> tensor (oracle UNet.state_dict(); optional 'context.*' entries from
         oracle ContextNet.state_dict()) or a path to a safetensors file holding the same.
-        variant: which build of the library to bind ("product"; "bf16" / "tools" exist for tests and tools)."""
+        variant: which build of the library to bind ("product"; "bf16" / "tools" exist for tests and tools).
+        batch_invariant: plan every batch per image as for a batch of 1 (include/cdc_b200.h cdc_set_batch_invariant), so
+        that with per-image seeds an image decodes -- and, through a Codec on this decoder, encodes -- to the same bits
+        alone, in any batch and in any shard of a multi-GPU run; at batch 1 the plan is the default one."""
         if not torch.cuda.is_available():
             raise RuntimeError("cdc_b200.Decoder needs a CUDA device (sm_100a); there is no CPU fallback")
         self.cfg = cfg
@@ -74,6 +77,8 @@ class Decoder:
                 self._ck(self.L.cdc_load_weights(self.ctx, name.encode(), C.c_void_p(d.data_ptr()), shape, d.dim()),
                          f"cdc_load_weights({name})")
             self._ck(self.L.cdc_finalize_weights(self.ctx), "cdc_finalize_weights")
+        self.batch_invariant = bool(batch_invariant)
+        self._ck(self.L.cdc_set_batch_invariant(self.ctx, 1 if self.batch_invariant else 0), "cdc_set_batch_invariant")
         self.has_context_net = bool(self.L.cdc_has_context_net(self.ctx))
         self.tables = tables
         self.steps = 0

@@ -85,6 +85,17 @@ int cdc_get_film(cdc_ctx* ctx, float* film_dev, cdc_stream s);
  * batch 1 .. 192 (CDC_ERR_SHAPE beyond: the GroupNorm apply kernel holds every image's statistics table in 48 KB of
  * shared memory); height and width multiples of 64. */
 int cdc_bind_io(cdc_ctx* ctx, int batch, int height, int width);
+/* Batch-invariant plans: on = 1 lays every op sequence (denoise step, context net, analysis encoder, hyper-encoder,
+ * hyper-decoder) out per image exactly as for a batch of 1; the launches still cover the whole batch.  on = 0 (the
+ * default) plans for the bound batch; any other value is CDC_ERR_SHAPE.  Takes effect at the next cdc_bind_io, which
+ * re-plans when the mode changed, also for the bound shape.
+ * The guarantee, for any batch 1 .. 192 and any position b: everything computed for image b -- the context maps, x_t and
+ * raw x0_hat of every step, the final image, y, z, mu, sigma and the quantised symbols of the codec side, the pixels of
+ * cdc_decompress_rgb8 -- is bit for bit what the same call gives for that image bound alone, and what the default mode
+ * gives at batch 1.  Conditions: the noise is per image (seeds bound with cdc_set_image_seeds, or a caller-supplied x_T with
+ * eta = 0), and both runs use the same SM count (a device of the same model) and the same build (fp16 or bf16).  The cost
+ * is throughput at large batches: shorter strips mean more halo rows per image (DESIGN.md). */
+int cdc_set_batch_invariant(cdc_ctx* ctx, int on);
 int cdc_set_cond(cdc_ctx* ctx, const float* c0, const float* c1, const float* c2, const float* c3, cdc_stream s);
 int cdc_set_latent(cdc_ctx* ctx, const float* y_hat, cdc_stream s); /* runs the context net: cond = context_net(y_hat) */
 int cdc_set_x(cdc_ctx* ctx, const float* x_nchw, cdc_stream s);
