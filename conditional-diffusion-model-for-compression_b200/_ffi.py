@@ -25,6 +25,7 @@ TOOLS_SYMBOLS = [
     "cdc_set_plan_option", "cdc_num_step_ops", "cdc_step_op_name", "cdc_step_op_flops", "cdc_step_op_bytes", "cdc_run_step_op",
     "cdc_profile_step", "cdc_profile_graph", "cdc_test_conv", "cdc_test_attention", "cdc_test_gn", "cdc_step_op_describe",
     "cdc_seq_num_ops", "cdc_seq_op_name", "cdc_seq_op_flops", "cdc_seq_op_bytes", "cdc_seq_op_describe", "cdc_run_seq_op",
+    "cdc_test_scale_rows", "cdc_test_dequant", "cdc_test_rgb8_in", "cdc_test_rgb8_out",
 ]
 OPT_FUSE_APPLY, OPT_KF, OPT_PLAN_SMS = range(3)
 OPK_MEMSET, OPK_CONV, OPK_GN_STATS, OPK_GN_APPLY, OPK_ATTENTION = range(5)  # cdc_op_kind
@@ -155,6 +156,10 @@ def _bind(L):
     L.cdc_test_conv.argtypes = [i32, p, i32, p, i32, i32, i32, i32, f32p, f32p, i32, i32, i32, i32, p, p, p, p]
     L.cdc_test_attention.argtypes = [p, p, i32, i32, i32, p]
     L.cdc_test_gn.argtypes = [p, p, p, f32p, f32p, f32p, i32, i32, i32, i32, C.c_float, p]
+    L.cdc_test_scale_rows.argtypes = [p, i32, i32, C.c_float, f32p, i32p, i32, i32, i32, p]
+    L.cdc_test_dequant.argtypes = [i32p, f32p, p, i32, p, i32, i32, i32, p]
+    L.cdc_test_rgb8_in.argtypes = [p, p, i64, p]
+    L.cdc_test_rgb8_out.argtypes = [f32p, p, i64, p]
     for s in SYMBOLS + TOOLS_SYMBOLS:
         getattr(L, s)  # raises AttributeError if the headers and the library disagree
     if hasattr(L, "cdc_debug_graph_skip"):  # tools build only

@@ -2405,4 +2405,33 @@ int cdc_test_gn(const void* x, const void* r, void* y, const float* gamma, const
     return e == cudaSuccess ? CDC_OK : CDC_ERR_CUDA;
 }
 
+// ---- the byte-boundary kernels of cdc_compress_rgb8 / cdc_decompress_rgb8, alone ----
+int cdc_test_scale_rows(const void* sigma_act, int ldc, int c_off, float min_sigma, const float* scale_table, int32_t* idx, int B,
+                        int C, int HW, cdc_stream s) {
+    if (!sigma_act || !scale_table || !idx || B < 1 || C < 1 || HW < 1 || c_off < 0 || ldc < c_off + C) return CDC_ERR_SHAPE;
+    return launch_scale_rows(static_cast<const act_t*>(sigma_act), ldc, c_off, min_sigma, scale_table, idx, B, C, HW, S(s)) == cudaSuccess
+               ? CDC_OK
+               : CDC_ERR_CUDA;
+}
+
+int cdc_test_dequant(const int32_t* q, const float* mu_vec, const void* mu_act, int mu_ldc, void* dst, int B, int C, int HW,
+                     cdc_stream s) {
+    if (!q || !dst || !mu_vec == !mu_act || B < 1 || C < 1 || HW < 1 || (mu_act && mu_ldc < C)) return CDC_ERR_SHAPE;
+    return launch_dequant_to_act(q, mu_vec, static_cast<const act_t*>(mu_act), mu_ldc, static_cast<act_t*>(dst), B, C, HW, S(s)) ==
+                   cudaSuccess
+               ? CDC_OK
+               : CDC_ERR_CUDA;
+}
+
+int cdc_test_rgb8_in(const uint8_t* rgb, void* dst64, int64_t npix, cdc_stream s) {
+    if (!rgb || !dst64 || npix < 16 || npix % 16 || (reinterpret_cast<uintptr_t>(rgb) & 15u)) return CDC_ERR_SHAPE;
+    return launch_rgb8_in(rgb, static_cast<act_t*>(dst64), npix, S(s)) == cudaSuccess ? CDC_OK : CDC_ERR_CUDA;
+}
+
+int cdc_test_rgb8_out(const float* xs, uint8_t* rgb, int64_t npix, cdc_stream s) {
+    if (!xs || !rgb || npix < 16 || npix % 16 || ((reinterpret_cast<uintptr_t>(xs) | reinterpret_cast<uintptr_t>(rgb)) & 15u))
+        return CDC_ERR_SHAPE;
+    return launch_rgb8_out(xs, rgb, npix, S(s)) == cudaSuccess ? CDC_OK : CDC_ERR_CUDA;
+}
+
 }  // extern "C"

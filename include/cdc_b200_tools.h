@@ -116,6 +116,22 @@ int cdc_test_conv(int device, const void* src0, int c0, const void* src1, int c1
 int cdc_test_attention(const void* qkv, void* out, int B, int N, int heads, cdc_stream s);
 int cdc_test_gn(const void* x, const void* r, void* y, const float* gamma, const float* beta, const float* film,
                 int B, int HW, int C, int silu, float eps, cdc_stream s);
+/* The byte-boundary kernels of cdc_compress_rgb8 / cdc_decompress_rgb8, each alone on device buffers (no context;
+ * CDC_ERR_SHAPE on bad arguments):
+ *   scale_rows: idx NCHW int32 [B][C][HW] = the CDF row of max(sigma, min_sigma), sigma = channels [c_off, c_off + C) of
+ *               the NHWC 16-bit sigma_act (ldc channels per pixel); scale_table fp32 [64]
+ *   dequant:    dst NHWC 16-bit [B][HW][C] = 16-bit of float(q) + mu, q NCHW int32; mu = mu_vec[c] (fp32 [C]) or channel c of
+ *               the NHWC 16-bit mu_act (mu_ldc channels per pixel): exactly one of the two
+ *   rgb8_in:    8-bit interleaved RGB [npix][3] (16-byte aligned) -> channels 0..2 of dst64 (64 channels per pixel) =
+ *               16-bit of 2 * (v / 255) - 1, channel 3 = 0, channels 4..63 untouched; npix a multiple of 16
+ *   rgb8_out:   xs fp32 [npix][3] -> rgb [npix][3] = round_half_even(255 * (clamp(x, -1, 1) + 1) / 2); both 16-byte
+ *               aligned, npix a multiple of 16 */
+int cdc_test_scale_rows(const void* sigma_act, int ldc, int c_off, float min_sigma, const float* scale_table, int32_t* idx, int B,
+                        int C, int HW, cdc_stream s);
+int cdc_test_dequant(const int32_t* q, const float* mu_vec, const void* mu_act, int mu_ldc, void* dst, int B, int C, int HW,
+                     cdc_stream s);
+int cdc_test_rgb8_in(const uint8_t* rgb, void* dst64, int64_t npix, cdc_stream s);
+int cdc_test_rgb8_out(const float* xs, uint8_t* rgb, int64_t npix, cdc_stream s);
 
 #ifdef CDC_TOOLS
 /* tools build only: leave a class of ops out of the captured graph (0 none, 1 tcgen05 convs, 2 elementwise/GroupNorm,
